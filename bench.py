@@ -6,7 +6,7 @@ points resident in HBM (a contiguous range of one N*2^LOG2N-point MSM, SURVEY.md
 rotating set of scalar vectors.  Each step: the Pippenger pipeline on each rank -> one 128-byte
 XYZZ partial per rank -> NCCL all-gather (the only exchange step) -> final add + normalisation.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--log2n 20] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--log2n 20] [--impl ours|reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  `value` = device-timed throughput with inputs resident in HBM;
 `e2e` = the same metric through the legacy C-ABI call `compute_multi_exp` with HOST buffers
@@ -48,7 +48,23 @@ def parse():
                     help="extra sizes (log2) timed at N=1 and reported under 'sweep'")
     ap.add_argument("--strong", default=os.environ.get("PORLA_BENCH_STRONG", "20,24,26"),
                     help="sizes (log2) of the ONE MSM sharded over all GPUs, reported under 'strong' (N > 1)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (float64), to compare two builds")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return a
+
+
+def dump_outputs(path, arrays):
+    """Writes each array as path/<name>.npy in float64; the inputs depend only on the arguments, so two builds run with
+    the same arguments must write the same files."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def workload_name(log2n, world):
@@ -732,6 +748,10 @@ def run_ours(args):
         sampler.stop_flag = True
         sampler.join(timeout=2)
     value = world * n / (ms_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # the affine result of the last timed step as the caller receives it: X and Y, 32 big-endian bytes each
+        last = bytes(out_host)
+        dump_outputs(args.dump_outputs, {"msm_result": [list(last[:32]), list(last[32:])]})
 
     # ---- roofline of the dominant kernel, measured live with CUDA events on the launch stream
     p_int = lib.porla_measure_pint(1, 1.0) if rank == 0 else 0.0

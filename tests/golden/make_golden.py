@@ -63,6 +63,27 @@ def secp_vectors():
     return out
 
 
+def secp_config4_vector():
+    """BASELINE config 4 (2^18 terms, the inputs of bench.py's secp256k1 block), computed with the big-int oracle, which
+    reproduces the reference's ecmult_multi_var outputs of secp256k1_ref.json.  Takes about a minute."""
+    c = O.SECP256K1
+    n = 1 << 18
+    q = int.from_bytes(hashlib.sha256(b"porla-seed").digest(), "big")
+    Q = O.mul(c, q, (c.gx, c.gy))
+    pts, cur = [], (c.gx, c.gy)
+    for _ in range(n):
+        pts.append(cur)
+        cur = O.add(c, cur, Q)
+    sc = [int.from_bytes(hashlib.sha256(b"cfg4" + i.to_bytes(4, "little")).digest(), "little") for i in range(n)]
+    r = O.msm(c, sc, pts, window=12)
+    be = lambda v: v.to_bytes(32, "big")
+    return {"source": "oracle/curves_py.py msm (big-int oracle; pinned to the reference's ecmult_multi_var by secp256k1_ref.json)",
+            "inputs": "points: P0 = G, P(i+1) = P(i) + q*G with q = sha256('porla-seed'); scalars: sha256('cfg4' || LE32(i)) "
+                      "as 32 little-endian bytes, NOT reduced",
+            "n": n, "chain_sha256": hashlib.sha256(b"".join(be(x) + be(y) for x, y in pts)).hexdigest(),
+            "xy": (be(r[0]) + be(r[1])).hex(), "sec1": O.secp_sec1_compressed(r).hex()}
+
+
 def bn254_vectors():
     c = O.BN254
     G = (1, 2)
@@ -96,9 +117,10 @@ def bn254_vectors():
     return out
 
 
+MAKERS = {"secp256k1_ref": secp_vectors, "bn254": bn254_vectors, "secp256k1_config4": secp_config4_vector}
+
 if __name__ == "__main__":
-    with open(os.path.join(HERE, "secp256k1_ref.json"), "w") as f:
-        json.dump(secp_vectors(), f, indent=1)
-    with open(os.path.join(HERE, "bn254.json"), "w") as f:
-        json.dump(bn254_vectors(), f, indent=1)
+    for name in sys.argv[1:] or MAKERS:        # e.g. `make_golden.py secp256k1_config4` needs no reference build
+        with open(os.path.join(HERE, name + ".json"), "w") as f:
+            json.dump(MAKERS[name](), f, indent=1)
     print("wrote golden vectors")
