@@ -150,20 +150,6 @@ void porla_msm_window_sums_device(const porla_table* t, const void* d_scalars, i
                                   int window_bits, void* d_window_sums, void* cuda_stream);
 void porla_msm_finalize_host(int curve, const void* h_window_sums, int64_t nparts, int nwin, int c,
                              int out_fmt, void* out64);
-/* Bucket-slice form of the sharded MSM (round 2): every rank holds the WHOLE table (an SRS is replicated once) and sees
- * ALL n scalars, but keeps only the (term, window) pairs whose bucket index is congruent to `slice_index` modulo
- * `slice_count` (a power of two, at most porla_msm_max_slices): 1 / slice_count of the bucket updates and of the buckets
- * to reduce, at the window size planned for the WHOLE MSM (plan_code = porla_msm_plan(curve, n_total, ...)).  The window
- * sums of the slice_count ranks add up window by window exactly like those of range shards (porla_msm_finalize_host).
- * The scalars may arrive in parts (the rank's own range first, the ranges gathered from the other ranks after it):
- * part_mode 0 = the whole MSM in one call, 1 / 2 / 3 = first / middle / last part, which accumulate table[first .. first+n)
- * x d_scalars[0 .. n) into ONE bucket array d_buckets (porla_msm_slice_bucket_bytes, caller-allocated; only the last
- * part reduces it and writes d_window_sums). */
-int porla_msm_max_slices(int curve, int plan_code, int want);
-uint64_t porla_msm_slice_bucket_bytes(int curve, int plan_code, int slice_count);
-void porla_msm_slice_window_sums_device(const porla_table* t, int64_t first, const void* d_scalars, int64_t n, int scalar_fmt,
-                                        int plan_code, int slice_index, int slice_count, int part_mode, void* d_buckets,
-                                        void* d_window_sums, void* cuda_stream);
 /* Multi-GPU combine: parts[k*nbatch + m] (k < count) are XYZZ partials gathered from the ranks. */
 void porla_msm_combine_device(int curve, const void* d_parts, int64_t count, int64_t nbatch,
                               int out_fmt, void* d_out, void* cuda_stream);
@@ -177,18 +163,10 @@ void porla_msm_combine_device(int curve, const void* d_parts, int64_t count, int
  *     device below which fewer devices are used (default 2^16).
  *   - porla_mtable: a point table resident in HBM, range-sharded over `ndev` devices (0 = all visible) at creation;
  *     an MSM over it moves only the scalars (host form) or nothing (resident form: d_scalars_per_part[p] is a device
- *     pointer ON the device of part p holding that part's scalars).
- *   - porla_mtable_create_replicated: the table is resident IN FULL on every device (an SRS: n * 96 B each) and an MSM
- *     is partitioned by bucket slice instead of by point range (see porla_msm_slice_window_sums_device): device p still
- *     owns the scalars of range p before the call (resident pointer, or its share of the host array over its own PCIe
- *     link), gathers the other ranges over NVLink while it accumulates its own, and reduces 1 / ndev of the buckets.
- *     porla_mtable_slices() = ndev when that route is taken (ndev a power of two, enough buckets per slice), else 1:
- *     the call then falls back to the point-range partition over views of the replicated table. */
+ *     pointer ON the device of part p holding that part's scalars). */
 int porla_device_count(void);
 typedef struct porla_mtable porla_mtable;
 porla_mtable* porla_mtable_create(int curve, const void* h_points, int64_t n, int point_fmt, int ndev);
-porla_mtable* porla_mtable_create_replicated(int curve, const void* h_points, int64_t n, int point_fmt, int ndev);
-int porla_mtable_slices(const porla_mtable* mt);
 int porla_mtable_devices(const porla_mtable* mt);
 int64_t porla_mtable_len(const porla_mtable* mt);
 void porla_mtable_range(const porla_mtable* mt, int part, int* device, int64_t* first, int64_t* count);

@@ -748,53 +748,6 @@ void porla_msm_window_sums_device(const porla_table* t, const void* d_scalars, i
     msm_device(t->t.curve, t->t, (const uint8_t*)d_scalars, (uint32_t)n, 1, opt, nullptr, nullptr, (cudaStream_t)cuda_stream);
 }
 
-static MsmPlan plan_of_code(int curve, int plan_code) {
-    MsmPlan p;
-    p.c = PORLA_PLAN_WINDOW(plan_code);
-    p.glv = (plan_code & PORLA_PLAN_GLV_ON) ? 1 : 0;
-    p.mode = kPlanPipeline;
-    p.nwin = msm_plan(curve, 1u << 20, 1, p.c, p.glv).nwin;     // windows for this window size (independent of n once forced)
-    return p;
-}
-
-int porla_msm_max_slices(int curve, int plan_code, int want) { return msm_max_slices(plan_of_code(curve, plan_code), want); }
-
-uint64_t porla_msm_slice_bucket_bytes(int curve, int plan_code, int slice_count) {
-    return msm_bucket_bytes(plan_of_code(curve, plan_code)) / (uint64_t)(slice_count > 0 ? slice_count : 1);
-}
-
-void porla_msm_slice_window_sums_device(const porla_table* t, int64_t first, const void* d_scalars, int64_t n, int scalar_fmt,
-                                        int plan_code, int slice_index, int slice_count, int part_mode, void* d_buckets,
-                                        void* d_window_sums, void* cuda_stream) {
-    check_shape(n, 1, "porla_msm_slice_window_sums_device");
-    if (first < 0 || first + n > (int64_t)t->t.n) die("porla_msm_slice_window_sums_device: range outside the table");
-    if (!(plan_code & (PORLA_PLAN_GLV_ON | PORLA_PLAN_GLV_OFF))) die("porla_msm_slice_window_sums_device: needs a plan code of porla_msm_plan");
-    if (part_mode != kPartWhole && !d_buckets) die("porla_msm_slice_window_sums_device: a streamed part needs the shared bucket array");
-    MsmOptions opt;
-    decode_plan(plan_code, &opt);
-    opt.scalar_be = scalar_fmt == PORLA_SCALAR_BE32;
-    opt.shared_points = 1;
-    opt.no_fixed_base = 1;
-    opt.no_small = 1;
-    opt.d_window_sums = d_window_sums;
-    opt.slice_index = slice_index;
-    opt.slice_count = slice_count;
-    opt.part_mode = part_mode;
-    opt.d_buckets = d_buckets;
-    PointTable view = t->t;
-    view.d_points = (uint8_t*)t->t.d_points + (size_t)first * 64;
-    view.d_flags = t->t.d_flags ? t->t.d_flags + first : nullptr;
-    view.n = (uint32_t)n;
-    view.d_fb_points = nullptr;
-    view.d_lut = nullptr;
-    view.fb_c = view.fb_nwin = 0;
-    if (t->t.d_phi_x) {
-        view.d_phi_x = (uint8_t*)t->t.d_phi_x + (size_t)first * 32;
-        view.phi_off = (uint32_t)n;
-    }
-    msm_device(t->t.curve, view, (const uint8_t*)d_scalars, (uint32_t)n, 1, opt, nullptr, nullptr, (cudaStream_t)cuda_stream);
-}
-
 void porla_msm_finalize_host(int curve, const void* h_window_sums, int64_t nparts, int nwin, int c, int out_fmt, void* out64) {
     finalize_host_parts(curve, h_window_sums, (int)nparts, nwin, PORLA_PLAN_WINDOW(c), out_fmt, (uint8_t*)out64);
 }

@@ -350,13 +350,6 @@ MsmPlan msm_plan(int curve, uint32_t n, uint32_t nbatch, int window_bits, int gl
 
 size_t msm_bucket_bytes(const MsmPlan& plan) { return ((size_t)plan.nwin << (plan.c - 1)) * 128; }
 
-int msm_max_slices(const MsmPlan& plan, int want) {
-    if (plan.mode != kPlanPipeline) return 1;
-    int s = 1;
-    while (s * 2 <= want && ((1u << (plan.c - 1)) / (uint32_t)(s * 2)) >= (4u << (plan.c / 2))) s *= 2;
-    return s;
-}
-
 // ---------------------------------------------------------------------------- host finaliser
 template <class F64>
 static void finalize_host_impl(const void* h_window_sums, int nparts, int nwin, int c, int out_fmt, uint8_t* out64) {

@@ -106,12 +106,6 @@ struct MsmOptions {
     // array, msm_bucket_bytes() bytes; every part must use the same window layout (window_bits and glv forced).
     int part_mode = 0;
     void* d_buckets = nullptr;
-    // Bucket slice (multi.cu, sharding.py: ONE MSM over several devices that all see every term): this call keeps only the
-    // (term, window) pairs whose bucket index is congruent to slice_index modulo slice_count (a power of two) -- 1 / slice_count
-    // of the bucket updates and of the buckets to reduce -- and weights the buckets accordingly, so that the window sums of
-    // the slice_count calls add up to the window sums of the whole MSM.  All slices must share one forced window layout.
-    int slice_index = 0;
-    int slice_count = 1;
 };
 enum : int { kPartWhole = 0, kPartFirst = 1, kPartMiddle = 2, kPartLast = 3 };
 
@@ -126,9 +120,6 @@ struct MsmPlan {
 MsmPlan msm_plan(int curve, uint32_t n, uint32_t nbatch, int window_bits, int glv = -1);
 // Bytes of the bucket array of ONE MSM under a pipeline plan (nwin bucket sets of 2^(c-1) XYZZ records).
 size_t msm_bucket_bytes(const MsmPlan& plan);
-// Largest slice_count (a power of two <= want) a pipeline plan can be cut into: every slice keeps at least 2^(c/2) * 4 buckets
-// per window so that the sort's coarse bins and the reduction's chunks stay whole.
-int msm_max_slices(const MsmPlan& plan, int want);
 // Plan for a specific call.  Fixed-base expansion applicable: nwin = 1 (a single shared bucket set or the
 // look-up table, one "window sum" per MSM, no doublings), c = the expansion's window size.  Few terms in
 // total and no explicit window size: one window per scalar bit (k_small_bits), c = 1.

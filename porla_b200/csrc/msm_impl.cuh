@@ -197,22 +197,7 @@ void msm_impl(const PointTable& table, const uint8_t* d_scalars, uint32_t n, uin
     }
     sh.c = wplan.c;
     sh.nwin = glv ? 2 * wplan.nwin : (C::kScalarBits + 1 + sh.c - 1) / sh.c;
-    // bucket slice: this call owns every slice_count-th bucket of every window (MsmOptions::slice_index / slice_count)
-    int slice_shift = 0;
-    while ((1 << slice_shift) < opt.slice_count) slice_shift++;
-    if (opt.slice_count > 1) {
-        const bool ok = (1 << slice_shift) == opt.slice_count && opt.slice_index >= 0 && opt.slice_index < opt.slice_count &&
-                        !fixed && nbatch == 1 && opt.window_bits > 0 && opt.glv >= 0 && opt.no_fixed_base &&
-                        msm_max_slices(wplan, opt.slice_count) == opt.slice_count;
-        if (!ok) {
-            fprintf(stderr, "[libmultiexp/porla_b200] FATAL: bucket slice %d of %d: needs one MSM, a forced window layout and a power-of-two "
-                            "slice count that leaves whole coarse bins (c = %d)\n", opt.slice_index, opt.slice_count, wplan.c);
-            abort();
-        }
-    }
-    sh.slice_shift = (uint32_t)slice_shift;
-    sh.slice_r = opt.slice_count > 1 ? (uint32_t)opt.slice_index : 0u;
-    sh.nbuckets = (1u << (sh.c - 1)) >> slice_shift;
+    sh.nbuckets = 1u << (sh.c - 1);
     sh.fixed_n = fixed ? table.fb_n : 0u;
     sh.glv_wh = glv ? wplan.nwin : 0;
     sh.phi_off = glv ? table.phi_off : 0u;
@@ -261,22 +246,20 @@ void msm_impl(const PointTable& table, const uint8_t* d_scalars, uint32_t n, uin
     if (!reduce_v1) blocks_per_slot = 2 * scan_bps;                                        // partials: out_w then out_s
 
     // accumulation geometry: slice length L (pairs per thread)
-    const uint64_t pairs_cap = pairs64 ? pairs64 : 1;   // capacity: a skewed input may put every pair into one slice
-    // geometry (slice length, waves) is planned for the EXPECTED number of pairs: 1 / slice_count of them
-    const uint64_t pairs_geo = (pairs_cap >> slice_shift) ? (pairs_cap >> slice_shift) : 1;
+    const uint64_t pairs_cap = pairs64 ? pairs64 : 1;
     // One "wave" = the threads of k_accumulate resident at once (4 blocks x 128 threads per SM at 106
     // registers).  L is the slice length that fills a whole number of waves with slices of at most 64
     // pairs; small MSMs get one wave of short slices, never slices so short that stitching the cut
     // buckets costs more than the additions (L = 4 made a 2^16-point MSM spend 6x longer in k_stitch
     // than in k_accumulate).
     const uint64_t wave = 148ull * 4ull * kAccThreads;
-    const uint64_t waves = (pairs_geo + wave * 64 - 1) / (wave * 64);
-    uint32_t L = (uint32_t)((pairs_geo + waves * wave - 1) / (waves * wave));
+    const uint64_t waves = (pairs_cap + wave * 64 - 1) / (wave * 64);
+    uint32_t L = (uint32_t)((pairs_cap + waves * wave - 1) / (waves * wave));
     if (waves == 1) {
         // A single wave does better three quarters full with longer slices: 12 warps per SM already saturate the
         // multiplier pipe and every slice boundary saved is a partial sum less to stitch (measured: 2^16 terms,
         // 0.96 wave of 18-pair slices 0.353 ms, 0.72 wave of 24-pair slices 0.301 ms; 2^17: 0.560 -> 0.519 ms).
-        const uint64_t l2 = pairs_geo / (wave * 18 / 25);
+        const uint64_t l2 = pairs_cap / (wave * 18 / 25);
         if (l2 >= 16 && l2 <= 64) L = (uint32_t)l2;
     }
     if (L < 16) L = 16;
@@ -289,7 +272,7 @@ void msm_impl(const PointTable& table, const uint8_t* d_scalars, uint32_t n, uin
         const char* e = getenv("PORLA_ACC_AFFINE");
         const bool big = pairs_cap >= (uint64_t)148 * PORLA_AFF_MIN_BLOCKS * kAffThreads * kAffL * 2;
         const int want = e ? atoi(e) : (big ? kAffDefaultRounds : 0);
-        if (want > 0 && !streamed && slice_shift == 0) {
+        if (want > 0 && !streamed) {
             aff_rounds = want > 2 ? 2 : want;
             L = kAffL;
         }
@@ -298,7 +281,7 @@ void msm_impl(const PointTable& table, const uint8_t* d_scalars, uint32_t n, uin
     // One serial XYZZ addition is ~7 us of latency: with few slices in flight (small MSMs) a bucket cut into
     // dozens of slices is better finished by a cooperating block; with the machine full, the serial loop in
     // every owner thread has the higher throughput (2^24, c = 20: 16 k top-window buckets of 17 slices).
-    const uint32_t serial_limit = (nslices_cap >> slice_shift) < 200000u ? kStitchSerialSmall : kStitchSerial;
+    const uint32_t serial_limit = nslices_cap < 200000u ? kStitchSerialSmall : kStitchSerial;
     const uint32_t long_cap = (uint32_t)(pairs_cap / ((uint64_t)L * serial_limit)) + 2;
 
     // sort path: shared-memory radix partition (two MSD passes) for large single MSMs, else one returning
@@ -348,7 +331,7 @@ void msm_impl(const PointTable& table, const uint8_t* d_scalars, uint32_t n, uin
     // 2.07 -> see profiles/r02b_sort_without_exact_histogram.txt.
     const char* sv2 = getenv("PORLA_SORT_V2");
     const bool v2_fits = ncoarse > 0 && pairs_cap / ncoarse <= (uint64_t)(kBigBin * 0.95);
-    const bool sort_v2 = radix && slice_shift == 0 && lb <= 10 && (size_t)ncoarse * 4 <= (160u << 10) && (sv2 ? sv2[0] == '1' : v2_fits);
+    const bool sort_v2 = radix && lb <= 10 && (size_t)ncoarse * 4 <= (160u << 10) && (sv2 ? sv2[0] == '1' : v2_fits);
     PORLA_CUDA(cudaMemsetAsync(counters, 0, (size_t)nbt * 4, stream));
     PORLA_CUDA(cudaMemsetAsync(grand, 0, 4, stream));
     PORLA_CUDA(cudaMemsetAsync(long_count, 0, 4, stream));
@@ -529,7 +512,7 @@ void msm_impl(const PointTable& table, const uint8_t* d_scalars, uint32_t n, uin
                                    ? (uint32_t)(slots * blocks_per_slot)
                                    : (uint32_t)((slots + kRedThreads / threads_per_slot - 1) / (kRedThreads / threads_per_slot));
         k_reduce<C><<<rgrid, kRedThreads, 0, stream>>>((const XC*)buckets, sh.nbuckets, chunk, threads_per_slot, (uint32_t)slots,
-                                                       (XC*)partials, sh.slice_shift, sh.slice_r);
+                                                       (XC*)partials);
         LAUNCHED();
         if (blocks_per_slot > 1) {
             k_window_sums<C><<<(uint32_t)slots, kRedThreads, 0, stream>>>((const XC*)partials, blocks_per_slot, (XC*)wsum);
@@ -544,10 +527,10 @@ void msm_impl(const PointTable& table, const uint8_t* d_scalars, uint32_t n, uin
                                    : (uint32_t)((slots + kQuadsPerBlock / scan_group - 1) / (kQuadsPerBlock / scan_group));
         k_reduce_scan<C><<<sgrid, kQuadThreads, 0, stream>>>(buckets, sh.nbuckets, log_m, scan_group, (uint32_t)slots, out_w, out_s);
         LAUNCHED();
-        if (scan_bps > 1 || sh.slice_shift != 0) {
+        if (scan_bps > 1) {
             uint32_t log_u = log_m;                      // weight of one block: m * kQuadsPerBlock buckets
             while ((1u << log_u) < ((uint32_t)kQuadsPerBlock << log_m)) log_u++;
-            k_reduce_top<C><<<(uint32_t)slots, kQuadThreads, 0, stream>>>(out_w, out_s, scan_bps, log_u, sh.slice_shift, sh.slice_r, wsum);
+            k_reduce_top<C><<<(uint32_t)slots, kQuadThreads, 0, stream>>>(out_w, out_s, scan_bps, log_u, wsum);
             LAUNCHED();
             window_sums = wsum;
         }

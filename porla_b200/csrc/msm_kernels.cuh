@@ -40,20 +40,7 @@ struct MsmShape {
     uint32_t fixed_n;    // 0: general.  > 0: fixed-base table of stride fixed_n (windows share buckets)
     int glv_wh;          // 0: off.  > 0: GLV, windows per half; nwin = 2 * glv_wh, window w and w + glv_wh share buckets
     uint32_t phi_off;    // GLV: phi(P_i) is the table entry phi_off + i
-    // Bucket slice (one MSM over several devices, every device sees ALL terms): this launch keeps only the digits whose
-    // bucket (|d| - 1) is congruent to slice_r modulo 2^slice_shift and files them under the local bucket (|d| - 1) >>
-    // slice_shift; nbuckets is then the LOCAL count 2^(c-1) >> slice_shift.  The interleaving spreads every window --
-    // also the short top one and short (31-bit) scalars -- evenly over the slices.  slice_shift = 0: everything.
-    uint32_t slice_shift;
-    uint32_t slice_r;
 };
-
-// local bucket of digit magnitude `mag` (0xffffffff: not in this launch's slice, or mag == 0)
-PORLA_D uint32_t slice_bucket(const MsmShape& sh, uint32_t mag) {
-    const uint32_t b = mag - 1u;
-    if (mag == 0u || (b & ((1u << sh.slice_shift) - 1u)) != sh.slice_r) return 0xffffffffu;
-    return b >> sh.slice_shift;
-}
 
 // ---------------------------------------------------------------------------- small helpers
 template <class T>
@@ -396,13 +383,12 @@ k_digits(const uint8_t* __restrict__ scalars, int big_endian,
                     carry = dneg;
                     uint32_t mag = dneg ? ((1u << sh.c) - d) : d;
                     uint32_t neg = dneg ^ flip[h];
-                    const uint32_t lbk = slice_bucket(sh, mag);
-                    if (lbk != 0xffffffffu && w >= w_begin && w < w_end) {
+                    if (mag != 0 && w >= w_begin && w < w_end) {
                         if (sh.fixed_n) {
-                            bucket[k] = slot_base + lbk;
+                            bucket[k] = slot_base + (mag - 1);
                             val[k] = ((uint32_t)w * sh.fixed_n + pidx) | (neg << 31);
                         } else {
-                            bucket[k] = slot_base + (uint32_t)wl * sh.nbuckets + lbk;
+                            bucket[k] = slot_base + (uint32_t)wl * sh.nbuckets + (mag - 1);
                             val[k] = (pidx + (h ? sh.phi_off : 0u)) | (neg << 31);
                         }
                     }
@@ -637,10 +623,9 @@ k_partition_coarse(const uint8_t* __restrict__ scalars, int big_endian, const ui
                 uint32_t dneg = d > half;
                 carry[q] = dneg;
                 uint32_t mag = dneg ? ((1u << sh.c) - d) : d;
-                const uint32_t lbk = slice_bucket(sh, mag);
-                if (lbk != 0xffffffffu) {
-                    uint32_t r = atomicAdd(&cnt[lbk >> lb], 1u);     // r < kPartTile = 2^11
-                    item[q] = lbk | (r << 20) | ((dneg ^ ((m >> flip_bit) & 1u)) << 31);
+                if (mag != 0) {
+                    uint32_t r = atomicAdd(&cnt[(mag - 1) >> lb], 1u);     // r < kPartTile = 2^11
+                    item[q] = (mag - 1) | (r << 20) | ((dneg ^ ((m >> flip_bit) & 1u)) << 31);
                 }
             }
         }
@@ -1248,8 +1233,7 @@ constexpr int kRedThreads = 64;
 template <class C>
 __global__ void __launch_bounds__(kRedThreads)
 k_reduce(const XYZZ<typename C::FC>* __restrict__ buckets, uint32_t nb, uint32_t chunk,
-         uint32_t threads_per_slot, uint32_t total_slots, XYZZ<typename C::FC>* __restrict__ partials,
-         uint32_t slice_shift, uint32_t slice_r) {
+         uint32_t threads_per_slot, uint32_t total_slots, XYZZ<typename C::FC>* __restrict__ partials) {
     using F = typename C::FC;
     __shared__ XYZZ<F> sh[kRedThreads];
     // Geometry (1-D grid; gridDim.y would cap the number of window slots at 65535):
@@ -1283,18 +1267,8 @@ k_reduce(const XYZZ<typename C::FC>* __restrict__ buckets, uint32_t nb, uint32_t
             run.add(bk);
             acc.add(run);
         }
-        if (slice_shift == 0) {
-            if (lo != 0) {
-                XYZZ<F> w = mul_small(run, lo);
-                acc.add(w);
-            }
-        } else {
-            // bucket slice: local bucket k stands for the digit magnitude (k << slice_shift) + slice_r + 1, so the chunk is
-            // 2^shift * sum (k - lo + 1) B_k + ((lo - 1) * 2^shift + slice_r + 1) * S; written with non-negative weights as
-            // 2^shift * (acc - S) + ((lo << shift) + slice_r + 1) * S
-            acc.add(run.neg());
-            for (uint32_t d = 0; d < slice_shift; d++) acc = acc.dbl();
-            XYZZ<F> w = mul_small(run, (lo << slice_shift) + slice_r + 1u);
+        if (lo != 0) {
+            XYZZ<F> w = mul_small(run, lo);
             acc.add(w);
         }
     }
@@ -1436,12 +1410,10 @@ k_reduce_scan(XYZZ<typename C::F>* buckets, uint32_t nb, uint32_t log_m, uint32_
 // up to 64 blocks) and folds them with running sums -- S' = sum S_j, W' = sum W_j + 2^log_u * sum_j j S_j -- after which the
 // quads are combined like the blocks themselves: window sum = sum_b W'_b + 2^(log_u + log2 per) * sum_b b S'_b, the second
 // term as the sum of the suffix sums RS_b, b >= 1.
-// Bucket slice (MsmShape::slice_shift / slice_r): local bucket k stands for the digit magnitude (k << shift) + r + 1, so the
-// slot's sum is 2^shift * (Z1 - G) + (r + 1) G = 2^shift * Z1 - (2^shift - 1 - r) G with Z1 the 1-based sum and G = RS_0.
 template <class C>
 __global__ void __launch_bounds__(kQuadThreads)
 k_reduce_top(const XYZZ<typename C::F>* __restrict__ in_w, const XYZZ<typename C::F>* __restrict__ in_s, uint32_t nblk_in,
-             uint32_t log_u, uint32_t slice_shift, uint32_t slice_r, XYZZ<typename C::F>* __restrict__ wsum) {
+             uint32_t log_u, XYZZ<typename C::F>* __restrict__ wsum) {
     using F = typename C::F;
     using Q = QuadPoint<F>;
     __shared__ XYZZ<F> sh[kQuadsPerBlock];
@@ -1474,7 +1446,6 @@ k_reduce_top(const XYZZ<typename C::F>* __restrict__ in_w, const XYZZ<typename C
         for (uint32_t q = per; q > 1; q >>= 1) log_u++;      // a quad now stands for `per` blocks
     }
     a = quad_suffix_scan(sh, b, b, nblk, a);                // quads >= nblk hold infinity and stay out of it
-    const Q g = quad_from_shared(&sh[0]);                   // RS_0: the plain sum of the slot's buckets
     Q v = (b != 0 && live) ? a : Q::inf();
     for (uint32_t d = 0; d < log_u; d++) v = quad_dbl_nl(v);
     v = quad_add_nl(v, wq);
@@ -1482,21 +1453,7 @@ k_reduce_top(const XYZZ<typename C::F>* __restrict__ in_w, const XYZZ<typename C
     quad_to_shared(&sh[b], v);
     __syncthreads();
     quad_tree_sum(sh, b, b, nblk);
-    if (threadIdx.x < 32) {                                  // quad 0 finishes (its warp keeps it company)
-        Q z = quad_from_shared(&sh[0]);
-        if (slice_shift != 0) {
-            for (uint32_t d = 0; d < slice_shift; d++) z = quad_dbl_nl(z);
-            const uint32_t k = (1u << slice_shift) - 1u - slice_r;       // < 2^slice_shift <= 8
-            Q t = Q::inf();
-            for (int bit = 3; bit >= 0; bit--) {
-                t = quad_dbl_nl(t);
-                t = quad_add_nl(t, ((k >> bit) & 1u) ? g : Q::inf());
-            }
-            if ((threadIdx.x & 3) == 1) t.c = t.c.neg();
-            z = quad_add_nl(z, t);
-        }
-        if (b == 0) z.store(wsum + blockIdx.x);
-    }
+    if (b == 0) quad_from_shared(&sh[0]).store(wsum + blockIdx.x);
 }
 
 // ---------------------------------------------------------------------------- window sums

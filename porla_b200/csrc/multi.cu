@@ -382,14 +382,6 @@ struct porla_mtable {
     PointTable part[kMaxDevices];
     uint8_t* d_scalars[kMaxDevices] = {};     // per-device scratch for host-scalar calls (count * 32 B)
     uint8_t* d_ws[kMaxDevices] = {};          // per-device window sums
-    // Replicated form (porla_mtable_create_replicated): every device holds ALL n points (part[p].n == n) and owns a bucket
-    // slice instead of a point range; first[] / count[] then say which range of the SCALARS lives on which device before
-    // a call.  d_all[p]: n * 32 B on device p, the scalars of the other devices' ranges as gathered over NVLink on every
-    // call; the device's own range inside it stays zero (written once at creation) when the call runs in two parts.
-    int replicated = 0;
-    int two_part = 0;
-    uint8_t* d_all[kMaxDevices] = {};
-    cudaEvent_t ev_own[kMaxDevices] = {};     // device p's own scalar range has arrived in d_scalars[p]
 };
 
 // entries [a, a + len) of a resident table (no fixed-base expansion: the parts of a sharded MSM exchange nwin window sums)
@@ -412,12 +404,12 @@ extern "C" {
 
 int porla_device_count(void) { return device_count(); }
 
-static porla_mtable* mtable_create(int curve, const void* h_points, int64_t n, int point_fmt, int ndev, int replicated) {
+porla_mtable* porla_mtable_create(int curve, const void* h_points, int64_t n, int point_fmt, int ndev) {
     device_init();
     const int visible = device_count() > kMaxDevices ? kMaxDevices : device_count();
     if (ndev <= 0) ndev = visible;
     const bool oversubscribe = getenv("PORLA_OVERSUBSCRIBE_DEVICES") != nullptr;   // tests on a box with fewer GPUs
-    if ((ndev > visible && !oversubscribe) || ndev > kMaxDevices || n < 0 || n >= ((int64_t)1 << 31) * (replicated ? 1 : ndev)) {
+    if ((ndev > visible && !oversubscribe) || ndev > kMaxDevices || n < 0 || n >= ((int64_t)1 << 31) * ndev) {
         fprintf(stderr, "[libmultiexp/porla_b200] FATAL: porla_mtable_create: %d devices requested, %d visible (n = %lld)\n", ndev,
                 visible, (long long)n);
         abort();
@@ -429,50 +421,18 @@ static porla_mtable* mtable_create(int curve, const void* h_points, int64_t n, i
     device_ranges(n, ndev, mt->first, mt->count);
     for (int p = 0; p < ndev; p++) mt->devices[p] = part_device(p);
     const uint8_t* pts = (const uint8_t*)h_points;
-    mt->replicated = replicated;
-    // two parts (own range under the gather, then the rest) pay one more addition per bucket: worth it from 2^22 terms
-    mt->two_part = replicated && (n >= ((int64_t)1 << 22) || getenv("PORLA_SLICE_TWO_PART")) && !getenv("PORLA_SLICE_ONE_PART");
     run_on_devices(ndev, [&](int p) {
         Staging& sg = worker_staging();
         const size_t m = (size_t)mt->count[p];
-        const size_t tab_first = replicated ? 0 : (size_t)mt->first[p], tab_n = replicated ? (size_t)n : m;
         uint8_t* d_tmp = nullptr;
-        PORLA_CUDA(cudaMalloc(&d_tmp, (tab_n ? tab_n : 1) * 64));
-        h2d_copy(d_tmp, pts + tab_first * 64, tab_n * 64, sg.stream);
-        table_import_device(curve, d_tmp, point_fmt, (uint32_t)tab_n, &mt->part[p], sg.stream);
+        PORLA_CUDA(cudaMalloc(&d_tmp, (m ? m : 1) * 64));
+        h2d_copy(d_tmp, pts + (size_t)mt->first[p] * 64, m * 64, sg.stream);
+        table_import_device(curve, d_tmp, point_fmt, (uint32_t)m, &mt->part[p], sg.stream);
         PORLA_CUDA(cudaFree(d_tmp));
         PORLA_CUDA(cudaMalloc(&mt->d_scalars[p], (m ? m : 1) * 32));
         PORLA_CUDA(cudaMalloc(&mt->d_ws[p], 256 * 128));
-        if (replicated) {
-            PORLA_CUDA(cudaMalloc(&mt->d_all[p], (size_t)(n ? n : 1) * 32));
-            PORLA_CUDA(cudaMemsetAsync(mt->d_all[p], 0, (size_t)(n ? n : 1) * 32, sg.stream));
-            PORLA_CUDA(cudaEventCreateWithFlags(&mt->ev_own[p], cudaEventDisableTiming));
-            for (int q = 0; q < ndev; q++) {      // direct NVLink copies between the devices of the table
-                if (mt->devices[q] == mt->devices[p]) continue;
-                int can = 0;
-                if (cudaDeviceCanAccessPeer(&can, mt->devices[p], mt->devices[q]) == cudaSuccess && can) {
-                    cudaError_t e = cudaDeviceEnablePeerAccess(mt->devices[q], 0);
-                    if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) PORLA_CUDA(e);
-                }
-                cudaGetLastError();
-            }
-            PORLA_CUDA(cudaStreamSynchronize(sg.stream));
-        }
     });
     return mt;
-}
-
-porla_mtable* porla_mtable_create(int curve, const void* h_points, int64_t n, int point_fmt, int ndev) {
-    return mtable_create(curve, h_points, n, point_fmt, ndev, 0);
-}
-
-porla_mtable* porla_mtable_create_replicated(int curve, const void* h_points, int64_t n, int point_fmt, int ndev) {
-    return mtable_create(curve, h_points, n, point_fmt, ndev, 1);
-}
-
-int porla_mtable_slices(const porla_mtable* mt) {
-    if (!mt->replicated || mt->n == 0) return 1;
-    return msm_max_slices(msm_plan(mt->curve, (uint32_t)mt->n, 1, 0), mt->ndev);
 }
 
 int porla_mtable_devices(const porla_mtable* mt) { return mt->ndev; }
@@ -488,87 +448,12 @@ void porla_mtable_range(const porla_mtable* mt, int part, int* device, int64_t* 
     *count = mt->count[part];
 }
 
-// Replicated table: ONE MSM over all n terms, device p accumulating and reducing bucket slice p of ndev.  Before a call the
-// scalars are range-sharded (device p holds [first[p], first[p] + count[p]): resident, or uploaded over its own PCIe link);
-// every device gathers the other ranges over NVLink (cudaMemcpyPeerAsync on its copy stream) -- the one real exchange step
-// of the sharded MSM -- while it already accumulates the terms of its own range (part 1); part 2 adds the gathered terms
-// into the same buckets, which are reduced once.  Compared with the point-range partition no device repeats the fixed costs
-// of a whole (smaller) MSM: the bucket updates and the buckets to reduce are both divided by ndev at the window size of the
-// WHOLE MSM (2^24 terms: 13 windows of 20 bits on every device instead of 15 of 17 bits per 2^21-term shard).
-static void mtable_msm_sliced(const porla_mtable* mt, const uint8_t* h_scalars, void* const* d_scalars_per_part, int scalar_fmt,
-                              int out_fmt, uint8_t* out64) {
-    const MsmPlan plan = msm_plan(mt->curve, (uint32_t)mt->n, 1, 0);
-    const size_t ws_bytes = (size_t)plan.nwin * 128;
-    const int P = mt->ndev;
-    std::vector<uint8_t> ws((size_t)P * ws_bytes);
-    std::atomic<int> arrived{0};
-    run_on_devices(P, [&](int p) {
-        Staging& sg = worker_staging();
-        const size_t m = (size_t)mt->count[p];
-        const uint8_t* d_own = d_scalars_per_part ? (const uint8_t*)d_scalars_per_part[p] : mt->d_scalars[p];
-        if (!d_scalars_per_part) {
-            h2d_copy(mt->d_scalars[p], h_scalars + (size_t)mt->first[p] * 32, m * 32, sg.stream);
-            PORLA_CUDA(cudaEventRecord(mt->ev_own[p], sg.stream));
-            arrived.fetch_add(1);
-            while (arrived.load() < P) std::this_thread::yield();      // every device's upload has been issued
-        }
-        // gather the other devices' ranges (start with the right-hand neighbour so that the sources are spread)
-        for (int k = 1; k < P; k++) {
-            const int q = (p + k) % P;
-            if (!mt->count[q]) continue;
-            const uint8_t* src = d_scalars_per_part ? (const uint8_t*)d_scalars_per_part[q] : mt->d_scalars[q];
-            uint8_t* dst = mt->d_all[p] + (size_t)mt->first[q] * 32;
-            const size_t bytes = (size_t)mt->count[q] * 32;
-            if (!d_scalars_per_part) PORLA_CUDA(cudaStreamWaitEvent(sg.copy_stream, mt->ev_own[q], 0));
-            if (mt->devices[q] == mt->devices[p]) PORLA_CUDA(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, sg.copy_stream));
-            else PORLA_CUDA(cudaMemcpyPeerAsync(dst, mt->devices[p], src, mt->devices[q], bytes, sg.copy_stream));
-        }
-        if (!mt->two_part && m)     // one part: the own range joins the gathered array
-            PORLA_CUDA(cudaMemcpyAsync(mt->d_all[p] + (size_t)mt->first[p] * 32, d_own, m * 32, cudaMemcpyDeviceToDevice, sg.stream));
-        PORLA_CUDA(cudaEventRecord(sg.ev[0], sg.copy_stream));
-        MsmOptions opt;
-        opt.scalar_be = scalar_fmt == PORLA_SCALAR_BE32;
-        opt.out_fmt = out_fmt;
-        opt.shared_points = 1;
-        opt.window_bits = plan.c;
-        opt.glv = plan.glv;
-        opt.no_fixed_base = 1;
-        opt.no_small = 1;
-        opt.d_window_sums = mt->d_ws[p];
-        opt.slice_index = p;
-        opt.slice_count = P;
-        if (mt->two_part) {
-            opt.d_buckets = sg.dev(msm_bucket_bytes(plan) / (size_t)P);
-            if (m) {
-                opt.part_mode = kPartFirst;
-                msm_device(mt->curve, table_view(mt->part[p], (size_t)mt->first[p], m), d_own, (uint32_t)m, 1, opt, nullptr, nullptr,
-                           sg.stream);
-            }
-            opt.part_mode = m ? kPartLast : kPartWhole;
-        }
-        PORLA_CUDA(cudaStreamWaitEvent(sg.stream, sg.ev[0], 0));
-        msm_device(mt->curve, mt->part[p], mt->d_all[p], (uint32_t)mt->n, 1, opt, nullptr, nullptr, sg.stream);
-        uint8_t* h = sg.pinned(ws_bytes);
-        PORLA_CUDA(cudaMemcpyAsync(h, mt->d_ws[p], ws_bytes, cudaMemcpyDeviceToHost, sg.stream));
-        PORLA_CUDA(cudaStreamSynchronize(sg.stream));
-        memcpy(ws.data() + (size_t)p * ws_bytes, h, ws_bytes);
-    });
-    finalize_host_parts(mt->curve, ws.data(), P, plan.nwin, plan.c, out_fmt, out64);
-}
-
 // Shared body: scalars either in host memory (one array of n, copied range by range) or already resident
 // (d_scalars_per_part[p] on device p).
 static void mtable_msm(const porla_mtable* mt, const uint8_t* h_scalars, void* const* d_scalars_per_part, int scalar_fmt,
                        int out_fmt, uint8_t* out64) {
     if (mt->n == 0) {
         memset(out64, 0, 64);
-        return;
-    }
-    // Measured on 8 B200s (profiles/r02c_bucket_slices_and_scan_reduce.md): a slice of 8 of a 2^24-term MSM takes 7.6 ms on its
-    // device against 6.4 ms for a 2^21-term range shard (every device recodes and filters all 2^24 scalars), so the bucket-slice
-    // route is opt-in (PORLA_SLICES=1) and a replicated table is cut by point range otherwise.
-    if (mt->replicated && porla_mtable_slices(mt) == mt->ndev && mt->ndev > 1 && getenv("PORLA_SLICES")) {
-        mtable_msm_sliced(mt, h_scalars, d_scalars_per_part, scalar_fmt, out_fmt, out64);
         return;
     }
     int64_t largest = 0;
@@ -598,7 +483,6 @@ static void mtable_msm(const porla_mtable* mt, const uint8_t* h_scalars, void* c
             so.no_small = 1;
             so.d_window_sums = mt->d_ws[p];
             so.d_buckets = d_bk;
-            const PointTable full = mt->replicated ? table_view(mt->part[p], (size_t)mt->first[p], m) : mt->part[p];
             size_t a = 0;
             for (int h = 0; h < nparts; h++) {
                 const size_t last = h == nparts - 1 ? m : (m * (2 * (size_t)h + 1)) / (2 * (size_t)nparts);
@@ -606,7 +490,7 @@ static void mtable_msm(const porla_mtable* mt, const uint8_t* h_scalars, void* c
                 h2d_copy(mt->d_scalars[p] + a * 32, h_scalars + ((size_t)mt->first[p] + a) * 32, len * 32, sg.copy_stream);
                 PORLA_CUDA(cudaEventRecord(sg.ev[h], sg.copy_stream));
                 PORLA_CUDA(cudaStreamWaitEvent(sg.stream, sg.ev[h], 0));
-                const PointTable view = table_view(full, a, len);          // entries [a, a + len) of this device's range
+                const PointTable view = table_view(mt->part[p], a, len);   // entries [a, a + len) of this device's range
                 so.part_mode = h == 0 ? kPartFirst : (h == nparts - 1 ? kPartLast : kPartMiddle);
                 msm_device(mt->curve, view, mt->d_scalars[p] + a * 32, (uint32_t)len, 1, so, nullptr, nullptr, sg.stream);
                 a = last;
@@ -626,8 +510,7 @@ static void mtable_msm(const porla_mtable* mt, const uint8_t* h_scalars, void* c
         opt.no_small = 1;
         opt.d_window_sums = mt->d_ws[p];
         if (m && d_sc)
-            msm_device(mt->curve, mt->replicated ? table_view(mt->part[p], (size_t)mt->first[p], m) : mt->part[p], d_sc, (uint32_t)m, 1,
-                       opt, nullptr, nullptr, sg.stream);
+            msm_device(mt->curve, mt->part[p], d_sc, (uint32_t)m, 1, opt, nullptr, nullptr, sg.stream);
         else if (!m) PORLA_CUDA(cudaMemsetAsync(mt->d_ws[p], 0, ws_bytes, sg.stream));
         uint8_t* h = sg.pinned(ws_bytes);
         PORLA_CUDA(cudaMemcpyAsync(h, mt->d_ws[p], ws_bytes, cudaMemcpyDeviceToHost, sg.stream));
@@ -665,8 +548,6 @@ void porla_mtable_destroy(porla_mtable* mt) {
     if (!mt) return;
     run_on_devices(mt->ndev, [&](int p) {
         table_free(&mt->part[p]);
-        if (mt->d_all[p]) PORLA_CUDA(cudaFree(mt->d_all[p]));
-        if (mt->ev_own[p]) PORLA_CUDA(cudaEventDestroy(mt->ev_own[p]));
         if (mt->d_scalars[p]) PORLA_CUDA(cudaFree(mt->d_scalars[p]));
         if (mt->d_ws[p]) PORLA_CUDA(cudaFree(mt->d_ws[p]));
     });

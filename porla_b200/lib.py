@@ -38,8 +38,7 @@ NEW_SYMBOLS = [
     "porla_device_count", "porla_mtable_create", "porla_mtable_devices", "porla_mtable_len", "porla_mtable_range",
     "porla_mtable_msm_host_scalars", "porla_mtable_msm_resident", "porla_mtable_scalars_upload", "porla_mtable_scalars_free",
     "porla_mtable_destroy", "porla_debug_copy_ring_bytes", "porla_msm_host_devices", "porla_debug_h2d_rate",
-    "porla_mtable_create_replicated", "porla_mtable_slices", "porla_msm_max_slices", "porla_msm_slice_bucket_bytes",
-    "porla_msm_slice_window_sums_device", "porla_debug_quad_op",
+    "porla_debug_quad_op",
 ]
 
 
@@ -141,11 +140,6 @@ def load() -> C.CDLL:
         "porla_debug_point_add_host": (None, [I, P, P, C.c_int64, I, P]),
         "porla_device_count": (I, []),
         "porla_mtable_create": (P, [I, P, C.c_int64, I, I]),
-        "porla_mtable_create_replicated": (P, [I, P, C.c_int64, I, I]),
-        "porla_mtable_slices": (I, [P]),
-        "porla_msm_max_slices": (I, [I, I, I]),
-        "porla_msm_slice_bucket_bytes": (C.c_uint64, [I, I, I]),
-        "porla_msm_slice_window_sums_device": (None, [P, C.c_int64, P, C.c_int64, I, I, I, I, I, P, P, P]),
         "porla_mtable_devices": (I, [P]),
         "porla_mtable_len": (C.c_int64, [P]),
         "porla_mtable_range": (None, [P, I, C.POINTER(I), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
@@ -389,16 +383,11 @@ class MultiTable:
     """A point table resident in HBM and range-sharded over the GPUs of the box inside ONE process (the in-call
     partition of Client.hpp:747-787 with devices in place of host threads)."""
 
-    def __init__(self, curve: int, points, n: int, point_fmt: int = POINT_BE64, ndev: int = 0, replicated: bool = False):
-        """replicated=True: every device holds the whole table and an MSM is partitioned by bucket slice (device p keeps
-        the bucket indices congruent to p modulo ndev) instead of by point range; the scalar ranges are gathered over
-        NVLink inside the call (porla_mtable_create_replicated)."""
+    def __init__(self, curve: int, points, n: int, point_fmt: int = POINT_BE64, ndev: int = 0):
         self.curve, self.n = curve, n
         self._keep = points
-        create = load().porla_mtable_create_replicated if replicated else load().porla_mtable_create
-        self.handle = create(curve, _as_void_p(points), n, point_fmt, ndev)
+        self.handle = load().porla_mtable_create(curve, _as_void_p(points), n, point_fmt, ndev)
         self.ndev = int(load().porla_mtable_devices(C.c_void_p(self.handle)))
-        self.slices = int(load().porla_mtable_slices(C.c_void_p(self.handle)))
 
     def part_range(self, part: int):
         d, f, c = C.c_int(0), C.c_int64(0), C.c_int64(0)

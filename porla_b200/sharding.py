@@ -78,74 +78,3 @@ class ShardedMsm:
                                          C.cast(self.out, C.c_void_p))
         return bytes(self.out)
 
-
-class SlicedMsm:
-    """One MSM of `n_total` terms over `world` processes by BUCKET SLICE (round 2): every rank holds the whole table resident
-    (an SRS is replicated once, n_total * 96 bytes) and owns the scalars of shard_range(n_total, world, rank) before a call.
-    A call all-gathers the scalars over NVLink (NCCL, the one real exchange step of this path) while the rank already
-    accumulates the terms of its own range into its buckets; the gathered terms follow into the same buckets, which are
-    reduced once.  Rank r keeps only the (term, window) pairs whose bucket index is congruent to r modulo world: 1 / world of
-    the bucket updates AND of the buckets to reduce, at the window size of the WHOLE MSM -- no rank repeats the fixed costs
-    of a smaller MSM, which is what caps the point-range partition (ShardedMsm) at ~6.5x on 8 GPUs.  The per-window sums
-    meet in one small all-gather and rank 0 combines them as for range shards.
-
-    `world` must be a power of two not larger than porla_msm_max_slices (else use ShardedMsm)."""
-
-    def __init__(self, curve: int, n_total: int, world: int, rank: int, dist, device, two_part=None):
-        import ctypes as C
-        import torch
-        from . import lib as L
-        self.C, self.torch, self.L = C, torch, L
-        self.lib = L.load()
-        self.curve, self.world, self.rank, self.dist, self.n = curve, world, rank, dist, n_total
-        c_, w_ = C.c_int(0), C.c_int(0)
-        self.lib.porla_msm_plan(curve, n_total, 1, 0, C.byref(c_), C.byref(w_))
-        self.plan_code, self.nwin = c_.value, w_.value
-        if self.lib.porla_msm_max_slices(curve, self.plan_code, world) != world:
-            raise ValueError("an MSM of %d terms cannot be cut into %d bucket slices" % (n_total, world))
-        self.lo, self.hi = shard_range(n_total, world, rank)
-        if n_total % world:
-            raise ValueError("SlicedMsm needs equal scalar ranges (n_total divisible by world) for the all-gather")
-        self.two_part = (n_total >= (1 << 22)) if two_part is None else bool(two_part)
-        self.wsum = torch.zeros(self.nwin * 128, dtype=torch.uint8, device=device)
-        self.all_scalars = torch.zeros(n_total * 32, dtype=torch.uint8, device=device)
-        nbytes = int(self.lib.porla_msm_slice_bucket_bytes(curve, self.plan_code, world))
-        self.buckets = torch.empty(nbytes, dtype=torch.uint8, device=device) if self.two_part else None
-        self.host = torch.zeros(world * self.nwin * 128, dtype=torch.uint8).pin_memory()
-        self.out = (C.c_ubyte * 64)()
-
-    def msm(self, table, own_scalars, scalar_fmt: int, out_fmt: int = 0):
-        """`table`: the WHOLE table (porla_b200.Table of n_total points); own_scalars: torch.uint8 tensor holding the
-        (hi - lo) * 32 bytes of this rank's scalar range.  Returns the 64-byte result on rank 0, None elsewhere."""
-        C, torch = self.C, self.torch
-        stream = torch.cuda.current_stream().cuda_stream
-        own = own_scalars.view(torch.uint8).reshape(-1)
-        n_own = self.hi - self.lo
-        work = None
-        if self.world > 1:
-            work = self.dist.all_gather_into_tensor(self.all_scalars, own, async_op=True)
-        else:
-            self.all_scalars.copy_(own)
-        args = (scalar_fmt, self.plan_code, self.rank, self.world)
-        bk = C.c_void_p(self.buckets.data_ptr()) if self.two_part else None
-        if self.two_part and self.world > 1:
-            # part 1: the own range, straight from the caller's buffer, while the all-gather is in flight
-            self.lib.porla_msm_slice_window_sums_device(C.c_void_p(table.handle), self.lo, C.c_void_p(own.data_ptr()), n_own, *args, 1,
-                                                        bk, C.c_void_p(self.wsum.data_ptr()), C.c_void_p(stream))
-            work.wait()
-            self.all_scalars[self.lo * 32:self.hi * 32].zero_()      # the own terms are in the buckets already
-            self.lib.porla_msm_slice_window_sums_device(C.c_void_p(table.handle), 0, C.c_void_p(self.all_scalars.data_ptr()), self.n,
-                                                        *args, 3, bk, C.c_void_p(self.wsum.data_ptr()), C.c_void_p(stream))
-        else:
-            if work is not None:
-                work.wait()
-            self.lib.porla_msm_slice_window_sums_device(C.c_void_p(table.handle), 0, C.c_void_p(self.all_scalars.data_ptr()), self.n,
-                                                        *args, 0, None, C.c_void_p(self.wsum.data_ptr()), C.c_void_p(stream))
-        allw = gather_window_sums(self.wsum, self.world, self.dist)
-        if self.rank != 0:
-            return None
-        self.host.copy_(allw, non_blocking=True)
-        torch.cuda.current_stream().synchronize()
-        self.lib.porla_msm_finalize_host(self.curve, C.c_void_p(self.host.data_ptr()), self.world, self.nwin, self.plan_code, out_fmt,
-                                         C.cast(self.out, C.c_void_p))
-        return bytes(self.out)

@@ -84,18 +84,24 @@ def test_host_buffer_fanout_matches_single_device(curve):
 
 
 @pytest.mark.parametrize("parts", [2, 3, 8])
-@pytest.mark.parametrize("kind", ["uniform", "constant", "small31", "pairs_cancel"])
+@pytest.mark.parametrize("kind", ["uniform", "constant", "small31", "top_bucket", "pairs_cancel"])
 def test_streamed_parts_share_one_bucket_set(parts, kind, monkeypatch):
     """msm_host_pipelined: the terms arrive in parts, every part is accumulated INTO the buckets the earlier parts filled and
     the buckets are reduced once.  Forced on small inputs (PORLA_STREAM_PARTS) with the cases that stress the carry-over:
     a constant scalar (one bucket per window, cut by every slice and continued by every part), 31-bit scalars (empty top
-    windows), and points that cancel ACROSS parts (P in one part, -P in another: the bucket returns to infinity)."""
+    windows), digits of the largest magnitude 2^(c-1) (the last bucket of every window), and points that cancel ACROSS
+    parts (P in one part, -P in another: the bucket returns to infinity)."""
     n = 6000
     pts, sc = _inputs(n, 11 + parts)
     if kind == "constant":
         sc = sc[:32] * n
     elif kind == "small31":
         sc = b"".join(bytes(28) + sc[32 * i + 28:32 * i + 32] for i in range(n))
+    elif kind == "top_bucket":
+        # digits of magnitude 2^(c-1) for every window size between 8 and 20, mixed with random scalars
+        pats = [sum(1 << (c * w + c - 1) for w in range(0, 250 // c)) for c in range(8, 21)]
+        sc = b"".join((pats[i % len(pats)] if i % 3 else int.from_bytes(sc[32 * i:32 * i + 32], "big")).to_bytes(32, "big")
+                      for i in range(n))
     elif kind == "pairs_cancel":
         half = n // 2
         P = bytearray(pts)
@@ -233,143 +239,6 @@ def test_two_rank_nccl_sharded_msm_closed_form():
         p.join(timeout=120)
         assert p.exitcode == 0
     assert got == _closed_form_bytes(1 << log2n, a, b).hex()
-
-
-# ---------------------------------------------------------------------------- bucket slices over a replicated table
-@pytest.mark.parametrize("two_part", [False, True])
-@pytest.mark.parametrize("n,ndev", [(20000, 2), (70001, 4), (70001, 8)])
-def test_replicated_table_bucket_slices_match_oracle(n, ndev, two_part, monkeypatch):
-    """porla_mtable_create_replicated: every part holds the whole table and keeps the bucket indices congruent to its own
-    number modulo ndev; the window sums of the parts add up to those of the whole MSM.  One-part (the own range joins the
-    gathered array) and two-part (own range first, the gathered rest into the same buckets) forms, host and resident
-    scalars, the bytes of the oracle."""
-    monkeypatch.setenv("PORLA_SLICE_TWO_PART" if two_part else "PORLA_SLICE_ONE_PART", "1")
-    monkeypatch.setenv("PORLA_SLICES", "1")
-    pts, sc = _inputs(n, 31 + ndev)
-    want = loader.bn254_msm(sc, pts, n, 8)
-    mt = pb.MultiTable(pb.CURVE_BN254, pts, n, ndev=ndev, replicated=True)
-    assert mt.ndev == ndev and mt.slices == ndev
-    assert mt.msm_host_scalars(sc) == want
-    ptrs = mt.upload_scalars(sc)
-    assert mt.msm_resident(ptrs) == want
-    assert mt.msm_resident(ptrs) == want
-    mt.free_scalars(ptrs)
-    monkeypatch.delenv("PORLA_SLICES")                       # the same replicated table, cut by point range (the default)
-    assert mt.msm_host_scalars(sc) == want
-    mt.destroy()
-
-
-@pytest.mark.parametrize("kind", ["constant", "small31", "top_bucket", "pairs_cancel"])
-def test_bucket_slices_on_skewed_scalars(kind, monkeypatch):
-    """Inputs that put every term into ONE slice (a constant scalar: one bucket per window), leave the top windows empty
-    (31-bit scalars), sit on the largest digit magnitude (2^(c-1): last local bucket of the last slice) or cancel across
-    the two parts of a call."""
-    monkeypatch.setenv("PORLA_SLICE_TWO_PART", "1")
-    monkeypatch.setenv("PORLA_SLICES", "1")
-    n, ndev = 40000, 4
-    pts, sc = _inputs(n, 53)
-    if kind == "constant":
-        sc = sc[:32] * n
-    elif kind == "small31":
-        sc = b"".join(bytes(28) + sc[32 * i + 28:32 * i + 32] for i in range(n))
-    elif kind == "top_bucket":
-        # digits of magnitude 2^(c-1) for every window size between 8 and 20, mixed with random scalars
-        pats = [sum(1 << (c * w + c - 1) for w in range(0, 250 // c)) for c in range(8, 21)]
-        sc = b"".join((pats[i % len(pats)] if i % 3 else int.from_bytes(sc[32 * i:32 * i + 32], "big")).to_bytes(32, "big")
-                      for i in range(n))
-    else:
-        half = n // 2
-        P = bytearray(pts)
-        for i in range(half):
-            y = int.from_bytes(pts[64 * i + 32:64 * i + 64], "big")
-            P[64 * (half + i):64 * (half + i + 1)] = pts[64 * i:64 * i + 32] + ((BN.p - y) % BN.p if y else 0).to_bytes(32, "big")
-        pts = bytes(P)
-        sc = sc[:32 * half] + bytes(31) + b"\x05" + sc[32:32 * half]
-    want = loader.bn254_msm(sc, pts, n, 8)
-    mt = pb.MultiTable(pb.CURVE_BN254, pts, n, ndev=ndev, replicated=True)
-    assert mt.slices == ndev
-    assert mt.msm_host_scalars(sc) == want
-    mt.destroy()
-
-
-def test_slice_window_sums_add_up_on_one_device():
-    """porla_msm_slice_window_sums_device called directly: the window sums of the 4 slices, combined like those of range
-    shards, are the MSM; a slice count the plan cannot carry is refused by porla_msm_max_slices."""
-    import torch
-    lib = pb.load()
-    n, S = 50000, 4
-    pts, sc = _inputs(n, 91)
-    want = loader.bn254_msm(sc, pts, n, 8)
-    tab = pb.Table.from_host(pb.CURVE_BN254, pts)
-    c_, w_ = C.c_int(0), C.c_int(0)
-    lib.porla_msm_plan(pb.CURVE_BN254, n, 1, 0, C.byref(c_), C.byref(w_))
-    assert lib.porla_msm_max_slices(pb.CURVE_BN254, c_.value, S) == S
-    assert lib.porla_msm_max_slices(pb.CURVE_BN254, c_.value, 1 << 20) < (1 << 20)
-    d_sc = torch.frombuffer(bytearray(sc), dtype=torch.uint8).cuda()
-    ws = torch.zeros(S * w_.value * 128, dtype=torch.uint8, device="cuda")
-    for r in range(S):
-        lib.porla_msm_slice_window_sums_device(C.c_void_p(tab.handle), 0, C.c_void_p(d_sc.data_ptr()), n, pb.SCALAR_BE32, c_.value,
-                                               r, S, 0, None, C.c_void_p(ws.data_ptr() + r * w_.value * 128), None)
-    torch.cuda.synchronize()
-    host = ws.cpu().numpy().tobytes()
-    out = (C.c_ubyte * 64)()
-    lib.porla_msm_finalize_host(pb.CURVE_BN254, host, S, w_.value, c_.value, pb.POINT_BE64, C.cast(out, C.c_void_p))
-    assert bytes(out) == want
-    tab.destroy()
-
-
-def _nccl_slice_worker(rank, world, port, log2n, a, b, two_part, q):
-    sys.path.insert(0, ROOT)
-    os.environ["MASTER_ADDR"] = "127.0.0.1"
-    os.environ["MASTER_PORT"] = str(port)
-    os.environ["PORLA_DEVICE"] = str(rank)
-    import torch
-    import torch.distributed as dist
-    import porla_b200 as pb2
-    from porla_b200.sharding import SlicedMsm
-    torch.cuda.set_device(rank)
-    dist.init_process_group("nccl", rank=rank, world_size=world, device_id=torch.device("cuda", rank))
-    n = 1 << log2n
-    ks, ss = _closed_form_inputs(torch, n, 0, n, a, b, "cuda:%d" % rank)
-    tab = pb2.Table.multiples_of_generator(pb2.CURVE_BN254, ks.data_ptr(), n, pb2.SCALAR_LE32, on_device=True)
-    eng = SlicedMsm(pb2.CURVE_BN254, n, world, rank, dist, torch.device("cuda", rank), two_part=two_part)
-    own = ss[eng.lo:eng.hi].contiguous()
-    del ss
-    got = eng.msm(tab, own, pb2.SCALAR_LE32)
-    got2 = eng.msm(tab, own, pb2.SCALAR_LE32)                 # the engine's buffers are reusable
-    if rank == 0:
-        q.put((got.hex(), got2.hex()))
-    dist.barrier()
-    dist.destroy_process_group()
-
-
-@pytest.mark.parametrize("two_part", [False, True])
-def test_two_rank_nccl_sliced_msm_closed_form(two_part):
-    """One process per GPU, bucket slices: every rank holds the whole table and its own scalar range, the scalars meet in
-    an NCCL all-gather, rank r accumulates and reduces the buckets congruent to r modulo world."""
-    import torch
-    import torch.multiprocessing as mp
-    if torch.cuda.device_count() < 2:
-        pytest.skip("needs two CUDA devices")
-    log2n, world = 19, 2
-    rnd = random.Random(18)
-    a = rnd.getrandbits(228) | (1 << 227) | 1
-    b = rnd.getrandbits(255) | (1 << 254)
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    port = s.getsockname()[1]
-    s.close()
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    procs = [ctx.Process(target=_nccl_slice_worker, args=(r, world, port, log2n, a, b, two_part, q)) for r in range(world)]
-    for p in procs:
-        p.start()
-    got = q.get(timeout=300)
-    for p in procs:
-        p.join(timeout=120)
-        assert p.exitcode == 0
-    want = _closed_form_bytes(1 << log2n, a, b).hex()
-    assert got == (want, want)
 
 
 def test_fixed_base_window_sums_add_up_on_one_device():

@@ -79,34 +79,6 @@ def test_two_rank_gloo_sharded_msm_matches_single():
     assert got == O.bn254_marshal(want).hex()
 
 
-def test_bucket_slice_plan_host_logic():
-    """Host side of the bucket-slice partition (no GPU needed): a pipeline plan can be cut into a power-of-two number of
-    slices only while every slice keeps whole coarse bins (4 * 2^(c/2) buckets per window); the bucket array of a slice is
-    1 / slices of the whole; and the slice weights tile the digit range exactly once: local bucket k of slice r stands for
-    the digit magnitude (k << shift) + r + 1."""
-    import ctypes as C
-    import porla_b200 as pb
-    lib = pb.load()
-    for n in (1 << 16, 1 << 20, 1 << 24):
-        c_, w_ = C.c_int(0), C.c_int(0)
-        lib.porla_msm_plan(pb.CURVE_BN254, n, 1, 0, C.byref(c_), C.byref(w_))
-        code, c = c_.value, c_.value & 0xff
-        assert code & (pb.lib.PLAN_GLV_ON | pb.lib.PLAN_GLV_OFF)
-        nb = 1 << (c - 1)
-        best = lib.porla_msm_max_slices(pb.CURVE_BN254, code, 1 << 20)
-        assert best >= 1 and best & (best - 1) == 0
-        assert nb // best >= 4 << (c // 2) and (best * 2 > (1 << 20) or nb // (best * 2) < 4 << (c // 2))
-        assert lib.porla_msm_max_slices(pb.CURVE_BN254, code, 8) == min(8, best)
-        assert lib.porla_msm_max_slices(pb.CURVE_BN254, code, 6) == min(4, best)       # not a power of two: rounded down
-        whole = lib.porla_msm_slice_bucket_bytes(pb.CURVE_BN254, code, 1)
-        assert whole % 128 == 0 and whole // 128 % nb == 0                              # whole bucket sets of 128-byte records
-        assert lib.porla_msm_slice_bucket_bytes(pb.CURVE_BN254, code, 8) * 8 == whole
-    # the weights of the slices tile 1 .. 2^(c-1)
-    c, shift = 10, 3
-    seen = sorted(((k << shift) + r + 1) for r in range(1 << shift) for k in range((1 << (c - 1)) >> shift))
-    assert seen == list(range(1, (1 << (c - 1)) + 1))
-
-
 def test_sharded_engine_plan_codes():
     """ShardedMsm's plan: one window layout for all ranks (planned for the largest shard); the fixed-base form exchanges
     ONE partial sum per rank under a code that carries the expansion's window size."""

@@ -83,12 +83,7 @@ os.environ["PORLA_ACC_AFFINE"] = "2"; os.environ["PORLA_NO_SMALL"] = "1"
 r5 = pb.bn254_multi_exp(bytes(hp), hs, n)
 del os.environ["PORLA_ACC_AFFINE"]; del os.environ["PORLA_NO_SMALL"]
 print("streamed / fan-out / sharded table / affine:", r1 == r2 == r3 == r4 == r5, r1.hex()[:16])
-# round 2c: bucket slices over a replicated table (two-part form), the old bucket reduction, the fixed-base sharded form,
-# the four-lane point operations' parity harness
-os.environ["PORLA_SLICES"] = "1"; os.environ["PORLA_SLICE_TWO_PART"] = "1"
-mt = pb.MultiTable(pb.CURVE_BN254, bytes(hp), n, ndev=4, replicated=True)
-r6 = mt.msm_host_scalars(hs); mt.destroy()
-del os.environ["PORLA_SLICES"]; del os.environ["PORLA_SLICE_TWO_PART"]
+# round 2c: the old bucket reduction, the fixed-base sharded form, the four-lane point operations' parity harness
 os.environ["PORLA_REDUCE_V1"] = "1"; os.environ["PORLA_NO_SMALL"] = "1"
 r7 = pb.bn254_multi_exp(bytes(hp), hs, n)
 del os.environ["PORLA_REDUCE_V1"]; del os.environ["PORLA_NO_SMALL"]
@@ -104,7 +99,7 @@ oq = (C.c_ubyte * (64 * 40))()
 for op in range(6):
     lib.porla_debug_quad_op(pb.CURVE_BN254, op, C.c_void_p(tfb.handle), C.c_void_p(tfb.handle), 40, pb.POINT_BE64, oq)
 tfb.destroy()
-print("slices / old reduce / fixed-base sharded form:", r1 == r6 == r7 == r8)
+print("old reduce / fixed-base sharded form:", r1 == r7 == r8)
 tabs = pb.Table.from_host(pb.CURVE_BN254, bytes(hp[:64 * 40]))
 d_sc = torch.frombuffer(bytearray(hs[:32 * 40]), dtype=torch.uint8).cuda()
 d_out = torch.zeros(64 * 40, dtype=torch.uint8, device="cuda")
