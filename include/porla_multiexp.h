@@ -89,6 +89,16 @@ uint64_t porla_launch_count(void);
 extern void compute_multi_exp_batch(GoSlice* scalars, GoSlice* points, GoInt length, GoInt batch,
                                     GoSlice* results_out);
 extern void compute_digest_from_srs_batch(GoSlice* data_in, GoInt batch, GoSlice* data_out);
+/* Batched forms of the client's two KZG symbols: each record is byte-identical to the per-call symbol on that record.
+ * compute_digest_batch: data_in = batch * n_samples * 32 B of big-endian coefficients (each reduced mod r), data_out =
+ * batch * 64 B of [alpha * f(tau)]G1.  alpha * f(tau) is evaluated on the device over powers alpha * tau^i kept in HBM,
+ * the product runs over a resident look-up table of the digest base; both are rebuilt after init_key / init_SRS*.
+ * compute_digest_complement_batch: data_in = batch * 32 B big-endian scalars s_i, each reduced mod r (the per-call
+ * compute_digest_complement reads one scalar of any length), data_out = batch * 64 B of [s_i]h_MAC, over a resident
+ * look-up table of h_MAC rebuilt after every init_SRS (before any init_SRS, h_MAC is infinity: 64 zero bytes per record).
+ * batch == 0 returns without touching the device.  The per-call symbols stay on the host. */
+extern void compute_digest_batch(GoSlice* data_in, GoInt batch, GoSlice* data_out);
+extern void compute_digest_complement_batch(GoSlice* data_in, GoInt batch, GoSlice* data_out);
 
 /* Resident point tables ("SRS and generator tables resident in HBM, uploaded once"). */
 typedef struct porla_table porla_table;
@@ -196,7 +206,9 @@ int porla_choose_window(int curve, int64_t n, int64_t nbatch);
 void porla_stage_timing_enable(int on);
 int porla_stage_timing_read(float* ms_out);
 
-/* Batched single-scalar multiplication out[i] = k_i * table[i] (table of length 1: fixed base). */
+/* Batched single-scalar multiplication out[i] = k_i * table[i] (table of length 1: fixed base).  A length-1 table that
+ * carries a look-up table (porla_table_precompute with window_bits = 0) is multiplied as a sum of nwin table entries per
+ * scalar, without doublings; every other table uses double-and-add.  The output bytes are the same either way. */
 void porla_scalar_mul_batch_device(const porla_table* t, const void* d_scalars, int64_t n,
                                    int scalar_fmt, int out_fmt, void* d_out, void* cuda_stream);
 

@@ -39,8 +39,24 @@ struct KzgState {
     PointTable srs_table;           // resident in HBM
     bool have_table = false;
     bool lut_tried = false;         // the wide-window look-up table of a large batch is attempted once per upload
+    uint64_t gen = 1;               // bumped (under g_srs_mu) whenever init_key / init_SRS* change tau, alpha, the SRS or h_MAC
 };
 KzgState g_kzg;
+
+// Device state of the client's batched symbols (compute_digest_batch, compute_digest_complement_batch): length-1 tables
+// of the digest base (the SRS's first point, [1]G1) and of h_MAC with their look-up tables, and the powers alpha tau^i in
+// HBM.  Guarded by g_srs_mu like the SRS table; each part is rebuilt once its `*_gen` differs from g_kzg.gen.
+struct ClientBase {
+    porla_table t;
+    uint64_t gen = 0;               // 0: never built
+    bool wide_tried = false;        // the wide-window look-up table of a large batch is attempted once per build
+};
+struct ClientState {
+    ClientBase digest, hmac;
+    void* d_powers = nullptr;       // n_samples elements of Fr, Montgomery form
+    uint64_t powers_gen = 0;
+};
+ClientState g_client;
 std::mutex g_io_mu;                 // serialises the staging buffers below
 
 // staging of the default device for the large host-buffer calls (struct Staging: staging.h)
@@ -343,6 +359,87 @@ void upload_srs() {
     upload_srs_locked();
 }
 
+void kzg_state_changed() {
+    std::unique_lock<std::shared_mutex> wr(g_srs_mu);
+    g_kzg.gen++;
+}
+
+// A batch of at least this many scalars over one base is worth the wide-window look-up table (table_precompute's
+// n_hint * batch_hint threshold with n_hint = 1: c = 16, 16 windows, 32 MiB).
+constexpr int64_t kWideBatch = (int64_t)1 << 22;
+
+bool client_base_fresh(const ClientBase& b, int64_t batch) {
+    return b.gen == g_kzg.gen && !(batch >= kWideBatch && !b.wide_tried && !getenv("PORLA_NO_LUT"));
+}
+
+// Caller holds g_srs_mu exclusively.  The base goes through the same import and precompute as any resident table:
+// table_precompute with window_bits = 0 gives a length-1 table the c = 8 look-up table, or the wide one for a large batch.
+void client_base_build(ClientBase* b, const G1A& base, int64_t batch) {
+    device_init();
+    std::lock_guard<std::mutex> io(g_io_mu);
+    g_stage.init();
+    if (b->t.t.d_points) table_free(&b->t.t);   // no reader left: each synchronised its stream before dropping g_srs_mu
+    uint8_t bytes[64];
+    g1_marshal(base, bytes);
+    table_import_host(kCurveBn254, bytes, PORLA_POINT_BE64, 1, &b->t.t, g_stage.stream);
+    table_precompute(&b->t.t, 0, 1, (uint32_t)(batch > 0 ? batch : 1), g_stage.stream);
+    PORLA_CUDA(cudaStreamSynchronize(g_stage.stream));
+    b->gen = g_kzg.gen;
+    b->wide_tried = batch >= kWideBatch;
+}
+
+// Caller holds g_srs_mu exclusively.
+void client_powers_build() {
+    device_init();
+    if (g_client.d_powers) PORLA_CUDA(cudaFree(g_client.d_powers));
+    g_client.d_powers = nullptr;
+    const int64_t n = g_kzg.n_samples;
+    if (n > 0) {
+        std::vector<Fr> p((size_t)n);
+        Fr acc = g_kzg.alpha;
+        for (int64_t i = 0; i < n; i++) {
+            p[(size_t)i] = acc;
+            acc = acc * g_kzg.tau;
+        }
+        PORLA_CUDA(cudaMalloc(&g_client.d_powers, (size_t)n * sizeof(Fr)));
+        PORLA_CUDA(cudaMemcpy(g_client.d_powers, p.data(), (size_t)n * sizeof(Fr), cudaMemcpyHostToDevice));
+    }
+    g_client.powers_gen = g_kzg.gen;
+}
+
+// Shared lock on the client state with the digest table and powers (digest) or the h_MAC table current for the calling
+// state of init_key / init_SRS*, rebuilding what is stale under the exclusive lock first.
+std::shared_lock<std::shared_mutex> client_reader(bool digest, int64_t batch) {
+    auto fresh = [&] {
+        return digest ? client_base_fresh(g_client.digest, batch) && g_client.powers_gen == g_kzg.gen
+                      : client_base_fresh(g_client.hmac, batch);
+    };
+    for (;;) {
+        {
+            std::shared_lock<std::shared_mutex> rd(g_srs_mu);
+            if (fresh()) return rd;
+        }
+        std::unique_lock<std::shared_mutex> wr(g_srs_mu);
+        if (digest) {
+            if (!client_base_fresh(g_client.digest, batch))
+                client_base_build(&g_client.digest, g_kzg.srs_g1.empty() ? g1_generator() : g_kzg.srs_g1[0], batch);
+            if (g_client.powers_gen != g_kzg.gen) client_powers_build();
+        } else if (!client_base_fresh(g_client.hmac, batch)) {
+            client_base_build(&g_client.hmac, g_kzg.h_mac, batch);
+        }
+    }
+}
+
+// `batch` fixed-base products over a resident client base (d_scalars already queued on the lease's stream), copied to data_out.
+void client_fixed_base(const ClientBase& b, const uint8_t* d_scalars, int scalar_fmt, int64_t batch, uint8_t* d_out,
+                       Staging& sg, GoSlice* data_out) {
+    porla_scalar_mul_batch_device(&b.t, d_scalars, batch, scalar_fmt, PORLA_POINT_BE64, d_out, sg.stream);
+    uint8_t* h = sg.pinned((size_t)batch * 64);
+    PORLA_CUDA(cudaMemcpyAsync(h, d_out, (size_t)batch * 64, cudaMemcpyDeviceToHost, sg.stream));
+    PORLA_CUDA(cudaStreamSynchronize(sg.stream));
+    go_copy(data_out, h, (size_t)batch * 64);
+}
+
 }  // namespace
 
 extern "C" {
@@ -351,6 +448,7 @@ extern "C" {
 void init_key(GoSlice* tau_key_in, GoSlice* alpha_key_in) {
     g_kzg.tau = elem_from_be<Fr>((const uint8_t*)tau_key_in->data, (size_t)tau_key_in->len);
     g_kzg.alpha = elem_from_be<Fr>((const uint8_t*)alpha_key_in->data, (size_t)alpha_key_in->len);
+    kzg_state_changed();
 }
 
 void init_SRS(GoInt SRS_size, GoSlice* out, GoInt64* out_len) {
@@ -389,6 +487,7 @@ void init_SRS(GoInt SRS_size, GoSlice* out, GoInt64* out_len) {
     }
     g_kzg.h_mac = g1_mul(g, elem_from_be<Fr>(rb, 32));
     g_kzg.have_table = false;
+    kzg_state_changed();
     if (device_available()) upload_srs();
 }
 
@@ -406,6 +505,7 @@ void init_SRS_from_data(GoInt SRS_size, GoSlice* in) {
     for (uint32_t i = 0; i < cnt; i++)
         if (!g1_unmarshal(b + 132 + 32 * (size_t)i, 32, &g_kzg.srs_g1[i])) die("init_SRS_from_data: bad G1 point");
     g_kzg.have_table = false;
+    kzg_state_changed();
     if (device_available()) upload_srs();
 }
 
@@ -549,6 +649,38 @@ void compute_digest_from_srs_batch(GoSlice* data_in, GoInt batch, GoSlice* data_
     std::vector<uint8_t> buf((size_t)batch * 64);
     if (batch) srs_commit_core((const uint8_t*)data_in->data, g_kzg.n_samples, batch, buf.data());
     go_copy(data_out, buf.data(), buf.size());
+}
+
+void compute_digest_batch(GoSlice* data_in, GoInt batch, GoSlice* data_out) {
+    const int64_t n = g_kzg.n_samples;
+    if (batch < 0 || data_in->len < n * 32 * batch) die("compute_digest_batch: data_in shorter than batch*n_samples*32 bytes");
+    if (batch == 0) return;
+    check_shape(n, batch, "compute_digest_batch");
+    device_init();
+    std::shared_lock<std::shared_mutex> rd = client_reader(true, batch);
+    StageLease lease = lease_stage(n, batch);
+    Staging& sg = *lease.s;
+    auto pad = [](size_t v) { return (v + 255) & ~(size_t)255; };
+    const size_t co_bytes = (size_t)n * batch * 32, sc_off = pad(co_bytes), out_off = sc_off + pad((size_t)batch * 32);
+    uint8_t* d = sg.dev(out_off + (size_t)batch * 64);
+    if (co_bytes) h2d_copy(d, data_in->data, co_bytes, sg.stream);
+    // alpha * f(tau) per record on the device, then [.]G1 over the resident table of the digest base
+    fr_poly_eval_device(d, g_client.d_powers, (uint32_t)n, (uint32_t)batch, d + sc_off, sg.stream);
+    client_fixed_base(g_client.digest, d + sc_off, PORLA_SCALAR_LE32, batch, d + out_off, sg, data_out);
+}
+
+void compute_digest_complement_batch(GoSlice* data_in, GoInt batch, GoSlice* data_out) {
+    if (batch < 0 || data_in->len < batch * 32) die("compute_digest_complement_batch: data_in shorter than batch*32 bytes");
+    if (batch == 0) return;
+    check_shape(1, batch, "compute_digest_complement_batch");
+    device_init();
+    std::shared_lock<std::shared_mutex> rd = client_reader(false, batch);
+    StageLease lease = lease_stage(1, batch);
+    Staging& sg = *lease.s;
+    const size_t sc_bytes = (size_t)batch * 32, out_off = (sc_bytes + 255) & ~(size_t)255;
+    uint8_t* d = sg.dev(out_off + (size_t)batch * 64);
+    h2d_copy(d, data_in->data, sc_bytes, sg.stream);
+    client_fixed_base(g_client.hmac, d, PORLA_SCALAR_BE32, batch, d + out_off, sg, data_out);
 }
 
 porla_table* porla_table_create(int curve, const void* points, int64_t n, int point_fmt, int on_device, void* cuda_stream) {
@@ -768,6 +900,15 @@ void porla_scalar_mul_batch_device(const porla_table* t, const void* d_scalars, 
     if (t->t.n != 1 && n > (int64_t)t->t.n) die("porla_scalar_mul_batch_device: table shorter than the batch");
     device_init();
     cudaStream_t st = (cudaStream_t)cuda_stream;
+    // A length-1 table that carries a look-up table (porla_table_precompute with window_bits = 0) is a fixed base: each
+    // product is a sum of nwin table entries.  Every other table keeps the double-and-add of k_scalar_mul; that includes
+    // the generator table of porla_table_create_multiples, which is imported without a look-up table.  Both paths return
+    // canonical points, so the bytes do not depend on the path.
+    if (t->t.n == 1 && t->t.d_lut) {
+        fixed_base_mul_device(t->t.curve, t->t, (const uint8_t*)d_scalars, scalar_fmt == PORLA_SCALAR_BE32, (uint32_t)n, out_fmt,
+                              (uint8_t*)d_out, st);
+        return;
+    }
     void* d_aff = nullptr;
     PORLA_CUDA(cudaMallocAsync(&d_aff, (size_t)(n ? n : 1) * 64, st));
     scalar_mul_device(t->t.curve, t->t, (const uint8_t*)d_scalars, scalar_fmt == PORLA_SCALAR_BE32, (uint32_t)n, d_aff, st);

@@ -154,6 +154,7 @@ constexpr uint32_t kLutMaxBasesBatched = 8192;
 constexpr int kLutWindow = 8;
 template <class C> void combine_impl(const void*, uint32_t, uint32_t, int, uint8_t*, cudaStream_t);
 template <class C> void scalar_mul_impl(const PointTable&, const uint8_t*, int, uint32_t, void*, cudaStream_t);
+template <class C> void fixed_base_mul_impl(const PointTable&, const uint8_t*, int, uint32_t, int, uint8_t*, cudaStream_t);
 template <class C> void export_impl(const void*, uint32_t, int, uint8_t*, cudaStream_t);
 template <class C> void butterfly_impl(PointTable*, uint32_t, const uint8_t*, int, cudaStream_t);
 template <class C> void align_scalars_impl(uint32_t*, uint32_t, uint8_t*, cudaStream_t);
@@ -442,6 +443,17 @@ void scalar_mul_device(int curve, const PointTable& table, const uint8_t* d_scal
     device_init();
     if (!n) return;
     DISPATCH(curve, scalar_mul_impl, table, d_scalars, scalar_be, n, d_out_affine, stream);
+}
+
+void fixed_base_mul_device(int curve, const PointTable& table, const uint8_t* d_scalars, int scalar_be, uint32_t n, int out_fmt,
+                           uint8_t* d_out, cudaStream_t stream) {
+    device_init();
+    if (table.n != 1 || !table.d_lut || table.curve != curve) {
+        fprintf(stderr, "[libmultiexp/porla_b200] FATAL: fixed_base_mul_device needs a length-1 table of this curve with a look-up table\n");
+        abort();
+    }
+    if (!n) return;
+    DISPATCH(curve, fixed_base_mul_impl, table, d_scalars, scalar_be, n, out_fmt, d_out, stream);
 }
 
 void butterfly_stage_device(PointTable* t, uint32_t m, const uint8_t* d_twiddles, int scalar_be, cudaStream_t stream) {

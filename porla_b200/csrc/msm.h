@@ -146,6 +146,15 @@ void msm_combine_device(int curve, const void* d_parts, uint32_t count, uint32_t
 // Elementwise batched kernels.
 void scalar_mul_device(int curve, const PointTable& table, const uint8_t* d_scalars, int scalar_be,
                        uint32_t n, void* d_out_affine, cudaStream_t stream);
+// out[i] = k_i * B for the ONE base of `table`, which must be a length-1 table carrying a look-up table (table_precompute
+// with window_bits = 0): a sum of nwin table entries per scalar, no doublings.  d_out: n * 64 B, canonical affine in out_fmt.
+void fixed_base_mul_device(int curve, const PointTable& table, const uint8_t* d_scalars, int scalar_be, uint32_t n, int out_fmt,
+                           uint8_t* d_out, cudaStream_t stream);
+// out[b] = sum_i f_(b,i) * powers[i] mod r (BN254 scalar field) for nbatch records of n big-endian 32-byte coefficients,
+// each reduced mod r first (fr.Element.SetBytes); d_powers: n field elements in Montgomery form (Fp<Bn254FrParams>).
+// d_out: nbatch canonical scalars of 8 little-endian 32-bit limbs (PORLA_SCALAR_LE32).
+void fr_poly_eval_device(const uint8_t* d_coeffs_be, const void* d_powers, uint32_t n, uint32_t nbatch, uint8_t* d_out,
+                         cudaStream_t stream);
 // One radix-2 butterfly stage of the "FFT in the exponent", in place on a resident table whose length is a
 // multiple of m (m a power of two >= 2): see k_butterfly.  d_twiddles: m/2 scalars of 32 bytes on the device.
 // Invalidates the table's fixed-base expansion.

@@ -604,6 +604,18 @@ void scalar_mul_impl(const PointTable& table, const uint8_t* d_scalars, int scal
 }
 
 template <class C>
+void fixed_base_mul_impl(const PointTable& table, const uint8_t* d_scalars, int scalar_be, uint32_t n, int out_fmt,
+                         uint8_t* d_out, cudaStream_t stream) {
+    using F = typename C::F;
+    const Affine<F>* lut = reinterpret_cast<const Affine<F>*>(table.d_lut);
+    const uint32_t grid = (n + kFixedBaseThreads - 1) / kFixedBaseThreads;
+    k_fixed_base_mul<C><<<grid, kFixedBaseThreads, 0, stream>>>(lut, table.fb_c, table.fb_nwin, d_scalars, scalar_be, n, out_fmt,
+                                                                d_out);
+    LAUNCHED();
+    PORLA_CUDA(cudaGetLastError());
+}
+
+template <class C>
 void butterfly_impl(PointTable* t, uint32_t m, const uint8_t* d_twiddles, int scalar_be, cudaStream_t stream) {
     const uint32_t nb = t->n / 2;
     if (!nb) return;
@@ -698,6 +710,7 @@ void field_mul_impl(const void* d_a, const void* d_b, uint32_t n, int op, void* 
     template void precompute_impl<C>(PointTable*, int, cudaStream_t);                                                  \
     template void lut_impl<C>(PointTable*, cudaStream_t);                                                              \
     template void scalar_mul_impl<C>(const PointTable&, const uint8_t*, int, uint32_t, void*, cudaStream_t);           \
+    template void fixed_base_mul_impl<C>(const PointTable&, const uint8_t*, int, uint32_t, int, uint8_t*, cudaStream_t); \
     template void export_impl<C>(const void*, uint32_t, int, uint8_t*, cudaStream_t);                                  \
     template void butterfly_impl<C>(PointTable*, uint32_t, const uint8_t*, int, cudaStream_t);                         \
     template void align_scalars_impl<C>(uint32_t*, uint32_t, uint8_t*, cudaStream_t);                                  \

@@ -38,7 +38,7 @@ NEW_SYMBOLS = [
     "porla_device_count", "porla_mtable_create", "porla_mtable_devices", "porla_mtable_len", "porla_mtable_range",
     "porla_mtable_msm_host_scalars", "porla_mtable_msm_resident", "porla_mtable_scalars_upload", "porla_mtable_scalars_free",
     "porla_mtable_destroy", "porla_debug_copy_ring_bytes", "porla_msm_host_devices", "porla_debug_h2d_rate",
-    "porla_debug_quad_op",
+    "porla_debug_quad_op", "compute_digest_batch", "compute_digest_complement_batch",
 ]
 
 
@@ -99,6 +99,8 @@ def load() -> C.CDLL:
         "porla_launch_count": (C.c_uint64, []),
         "compute_multi_exp_batch": (None, [GS, GS, LL, LL, GS]),
         "compute_digest_from_srs_batch": (None, [GS, LL, GS]),
+        "compute_digest_batch": (None, [GS, LL, GS]),
+        "compute_digest_complement_batch": (None, [GS, LL, GS]),
         "porla_table_create": (P, [I, P, C.c_int64, I, I, P]),
         "porla_table_create_multiples": (P, [I, P, C.c_int64, I, I, P]),
         "porla_table_precompute": (I, [P, I, C.c_int64, C.c_int64, P]),
@@ -256,6 +258,19 @@ class Kzg:
     def compute_digest_complement(self, s: bytes) -> bytes:
         out = bytearray(64)
         self.lib.compute_digest_complement(C.byref(_slice(bytearray(s))), C.byref(_slice(out)))
+        return bytes(out)
+
+    def compute_digest_batch(self, data: bytes, batch: int) -> bytes:
+        """`batch` records of n_samples x 32-byte BE coefficients; returns batch x 64 bytes, record j equal to
+        compute_digest of record j."""
+        out = bytearray(64 * batch)
+        self.lib.compute_digest_batch(C.byref(_slice(bytearray(data))), batch, C.byref(_slice(out)))
+        return bytes(out)
+
+    def compute_digest_complement_batch(self, scalars: bytes, batch: int) -> bytes:
+        """`batch` 32-byte BE scalars; returns batch x 64 bytes, record j equal to compute_digest_complement of scalar j."""
+        out = bytearray(64 * batch)
+        self.lib.compute_digest_complement_batch(C.byref(_slice(bytearray(scalars))), batch, C.byref(_slice(out)))
         return bytes(out)
 
     def compute_digest_from_srs(self, data: bytes) -> bytes:
