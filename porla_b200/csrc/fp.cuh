@@ -323,131 +323,6 @@ PORLA_D void sqr_wide_device(const uint32_t* a, uint32_t* T) {
           "+r"(T[8]), "+r"(T[9]), "+r"(T[10]), "+r"(T[11]), "+r"(T[12]), "+r"(T[13]), "+r"(T[14]), "+r"(T[15])
         : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(a[4]), "r"(a[5]), "r"(a[6]), "r"(a[7]));
 }
-
-// T[0..7] = a[0..3] * b[0..3]: the two-row scheme of mul_wide_device on 4 limbs (16 IMAD.WIDE).
-PORLA_D void mul4_wide_device(const uint32_t* a, const uint32_t* b, uint32_t* T) {
-    uint32_t E[8], O[8];
-    {
-        uint64_t p0 = (uint64_t)a[0] * b[0], p1 = (uint64_t)a[1] * b[0], p2 = (uint64_t)a[2] * b[0],
-                 p3 = (uint64_t)a[3] * b[0];
-        E[0] = (uint32_t)p0; E[1] = (uint32_t)(p0 >> 32); E[2] = (uint32_t)p2; E[3] = (uint32_t)(p2 >> 32);
-        O[0] = (uint32_t)p1; O[1] = (uint32_t)(p1 >> 32); O[2] = (uint32_t)p3; O[3] = (uint32_t)(p3 >> 32);
-    }
-#pragma unroll
-    for (int j = 4; j < 8; j++) E[j] = O[j] = 0;
-    mac2(E + 2, E[6], a[1], a[3], b[1]);
-    mac2(O + 0, O[4], a[0], a[2], b[1]);
-    mac2(E + 2, E[6], a[0], a[2], b[2]);
-    mac2(O + 2, O[6], a[1], a[3], b[2]);
-    {
-        uint32_t drop = 0;
-        mac2(E + 4, drop, a[1], a[3], b[3]);
-    }
-    mac2(O + 2, O[6], a[0], a[2], b[3]);
-    T[0] = E[0];
-    asm("add.cc.u32 %0, %7, %14;\n\t"
-        "addc.cc.u32 %1, %8, %15;\n\t"
-        "addc.cc.u32 %2, %9, %16;\n\t"
-        "addc.cc.u32 %3, %10, %17;\n\t"
-        "addc.cc.u32 %4, %11, %18;\n\t"
-        "addc.cc.u32 %5, %12, %19;\n\t"
-        "addc.u32 %6, %13, %20;"
-        : "=r"(T[1]), "=r"(T[2]), "=r"(T[3]), "=r"(T[4]), "=r"(T[5]), "=r"(T[6]), "=r"(T[7])
-        : "r"(E[1]), "r"(E[2]), "r"(E[3]), "r"(E[4]), "r"(E[5]), "r"(E[6]), "r"(E[7]),
-          "r"(O[0]), "r"(O[1]), "r"(O[2]), "r"(O[3]), "r"(O[4]), "r"(O[5]), "r"(O[6]));
-}
-
-// d = |x - y| on 4 limbs; returns 0xffffffff when x < y (the difference was negated), else 0.
-PORLA_D uint32_t absdiff4_device(uint32_t* d, const uint32_t* x, const uint32_t* y) {
-    uint32_t m;
-    asm("sub.cc.u32 %0, %5, %9;\n\t"
-        "subc.cc.u32 %1, %6, %10;\n\t"
-        "subc.cc.u32 %2, %7, %11;\n\t"
-        "subc.cc.u32 %3, %8, %12;\n\t"
-        "subc.u32 %4, 0, 0;\n\t"
-        "xor.b32 %0, %0, %4;\n\t"
-        "xor.b32 %1, %1, %4;\n\t"
-        "xor.b32 %2, %2, %4;\n\t"
-        "xor.b32 %3, %3, %4;\n\t"
-        "sub.cc.u32 %0, %0, %4;\n\t"
-        "subc.cc.u32 %1, %1, %4;\n\t"
-        "subc.cc.u32 %2, %2, %4;\n\t"
-        "subc.u32 %3, %3, %4;"
-        : "=&r"(d[0]), "=&r"(d[1]), "=&r"(d[2]), "=&r"(d[3]), "=&r"(m)
-        : "r"(x[0]), "r"(x[1]), "r"(x[2]), "r"(x[3]), "r"(y[0]), "r"(y[1]), "r"(y[2]), "r"(y[3]));
-    return m;
-}
-
-// T[0..15] = a * b by one level of (subtractive) Karatsuba: three 4x4 products = 48 IMAD.WIDE instead of
-// 64, paid for with ~90 additions/logic ops that issue on the ALU pipe in the shadow of the
-// multiplier (ncu: fmaheavy 89 % busy, issue slots 37 %, ALU pipe 27 % in k_accumulate).
-// MEASURED (B200, 2^20 points): k_accumulate 3.21 ms with it against 2.58 ms without -- ptxas turns ~500
-// of the extra moves/carry additions into IMAD.MOV / IMAD.X, which land on the same FMA pipe and cost
-// more than the 200 IMAD.WIDE saved, and the kernel starts to spill.  Kept behind -DPORLA_KARATSUBA.
-//   a = a0 + a1 W, b = b0 + b1 W, W = 2^128:   a b = z0 + (z0 + z2 - (a0 - a1)(b0 - b1)) W + z2 W^2
-PORLA_D void mul_wide_karatsuba_device(const uint32_t* a, const uint32_t* b, uint32_t* T) {
-    uint32_t z0[8], z2[8], zm[8], da[4], db[4];
-    mul4_wide_device(a, b, z0);
-    mul4_wide_device(a + 4, b + 4, z2);
-    const uint32_t sa = absdiff4_device(da, a, a + 4);
-    const uint32_t sb = absdiff4_device(db, b, b + 4);
-    mul4_wide_device(da, db, zm);
-    // (a0 - a1)(b0 - b1) = +zm when the signs agree: then z1 = z0 + z2 - zm, else z1 = z0 + z2 + zm.
-    const uint32_t nm = ~(sa ^ sb);  // all ones: subtract
-    uint32_t S[9], z1[9];
-    asm("add.cc.u32 %0, %9, %17;\n\t"
-        "addc.cc.u32 %1, %10, %18;\n\t"
-        "addc.cc.u32 %2, %11, %19;\n\t"
-        "addc.cc.u32 %3, %12, %20;\n\t"
-        "addc.cc.u32 %4, %13, %21;\n\t"
-        "addc.cc.u32 %5, %14, %22;\n\t"
-        "addc.cc.u32 %6, %15, %23;\n\t"
-        "addc.cc.u32 %7, %16, %24;\n\t"
-        "addc.u32 %8, 0, 0;"
-        : "=r"(S[0]), "=r"(S[1]), "=r"(S[2]), "=r"(S[3]), "=r"(S[4]), "=r"(S[5]), "=r"(S[6]), "=r"(S[7]), "=r"(S[8])
-        : "r"(z0[0]), "r"(z0[1]), "r"(z0[2]), "r"(z0[3]), "r"(z0[4]), "r"(z0[5]), "r"(z0[6]), "r"(z0[7]),
-          "r"(z2[0]), "r"(z2[1]), "r"(z2[2]), "r"(z2[3]), "r"(z2[4]), "r"(z2[5]), "r"(z2[6]), "r"(z2[7]));
-#pragma unroll
-    for (int k = 0; k < 8; k++) zm[k] ^= nm;
-    // z1 = S + (zm ^ nm) + (nm & 1), nine limbs, two's complement (the true value is in [0, 2^257))
-    {
-        uint32_t t;
-        asm("add.cc.u32 %9, %28, %28;\n\t"   // carry flag := nm != 0
-            "addc.cc.u32 %0, %10, %19;\n\t"
-            "addc.cc.u32 %1, %11, %20;\n\t"
-            "addc.cc.u32 %2, %12, %21;\n\t"
-            "addc.cc.u32 %3, %13, %22;\n\t"
-            "addc.cc.u32 %4, %14, %23;\n\t"
-            "addc.cc.u32 %5, %15, %24;\n\t"
-            "addc.cc.u32 %6, %16, %25;\n\t"
-            "addc.cc.u32 %7, %17, %26;\n\t"
-            "addc.u32 %8, %18, %27;"
-            : "=&r"(z1[0]), "=&r"(z1[1]), "=&r"(z1[2]), "=&r"(z1[3]), "=&r"(z1[4]), "=&r"(z1[5]), "=&r"(z1[6]),
-              "=&r"(z1[7]), "=&r"(z1[8]), "=&r"(t)
-            : "r"(S[0]), "r"(S[1]), "r"(S[2]), "r"(S[3]), "r"(S[4]), "r"(S[5]), "r"(S[6]), "r"(S[7]), "r"(S[8]),
-              "r"(zm[0]), "r"(zm[1]), "r"(zm[2]), "r"(zm[3]), "r"(zm[4]), "r"(zm[5]), "r"(zm[6]), "r"(zm[7]), "r"(nm),
-              "r"(nm));
-        (void)t;
-    }
-    T[0] = z0[0]; T[1] = z0[1]; T[2] = z0[2]; T[3] = z0[3];
-    asm("add.cc.u32 %0, %12, %24;\n\t"
-        "addc.cc.u32 %1, %13, %25;\n\t"
-        "addc.cc.u32 %2, %14, %26;\n\t"
-        "addc.cc.u32 %3, %15, %27;\n\t"
-        "addc.cc.u32 %4, %16, %28;\n\t"
-        "addc.cc.u32 %5, %17, %29;\n\t"
-        "addc.cc.u32 %6, %18, %30;\n\t"
-        "addc.cc.u32 %7, %19, %31;\n\t"
-        "addc.cc.u32 %8, %20, %32;\n\t"
-        "addc.cc.u32 %9, %21, 0;\n\t"
-        "addc.cc.u32 %10, %22, 0;\n\t"
-        "addc.u32 %11, %23, 0;"
-        : "=r"(T[4]), "=r"(T[5]), "=r"(T[6]), "=r"(T[7]), "=r"(T[8]), "=r"(T[9]), "=r"(T[10]), "=r"(T[11]),
-          "=r"(T[12]), "=r"(T[13]), "=r"(T[14]), "=r"(T[15])
-        : "r"(z0[4]), "r"(z0[5]), "r"(z0[6]), "r"(z0[7]), "r"(z2[0]), "r"(z2[1]), "r"(z2[2]), "r"(z2[3]),
-          "r"(z2[4]), "r"(z2[5]), "r"(z2[6]), "r"(z2[7]),
-          "r"(z1[0]), "r"(z1[1]), "r"(z1[2]), "r"(z1[3]), "r"(z1[4]), "r"(z1[5]), "r"(z1[6]), "r"(z1[7]), "r"(z1[8]));
-}
 #endif  // __CUDA_ARCH__
 
 // ------------------------------------------------------------------------------------------
@@ -804,49 +679,6 @@ struct alignas(16) Fp {
         merge_rows(r, even, odd);
     }
 
-    // Montgomery product through the Karatsuba wide product (48 IMAD.WIDE) and a separate REDC of the low
-    // half (64): REDC(lo + hi 2^256) = REDC(lo) + hi with REDC(lo) <= p and hi < p^2 / 2^256 < p / 4.
-    static PORLA_D Fp mul_mont_karatsuba_device(const Fp& a, const Fp& b) {
-        uint32_t T[16], lo[8];
-        mul_wide_karatsuba_device(a.v, b.v, T);
-        redc8_device(T, lo);
-        Fp r;
-        add256(r.v, lo, T + 8);
-        r.final_sub(0);
-        return r;
-    }
-    // (a*b + c*d) / 2^256 mod p: two Karatsuba products summed on 16 limbs (< 2 p^2 < 2^509), one REDC;
-    // the result is below p + 1 + p / 2, one conditional subtraction.
-    static PORLA_D Fp mul2add_mont_karatsuba_device(const Fp& a, const Fp& b, const Fp& c, const Fp& d) {
-        uint32_t T[16], U[16], lo[8];
-        mul_wide_karatsuba_device(a.v, b.v, T);
-        mul_wide_karatsuba_device(c.v, d.v, U);
-        uint32_t carry = add256(T, T, U);
-        asm("add.cc.u32 %0, %0, %16;\n\t"
-            "addc.cc.u32 %1, %1, 0;\n\t"
-            "addc.cc.u32 %2, %2, 0;\n\t"
-            "addc.cc.u32 %3, %3, 0;\n\t"
-            "addc.cc.u32 %4, %4, 0;\n\t"
-            "addc.cc.u32 %5, %5, 0;\n\t"
-            "addc.cc.u32 %6, %6, 0;\n\t"
-            "addc.u32 %7, %7, 0;\n\t"
-            "add.cc.u32 %0, %0, %8;\n\t"
-            "addc.cc.u32 %1, %1, %9;\n\t"
-            "addc.cc.u32 %2, %2, %10;\n\t"
-            "addc.cc.u32 %3, %3, %11;\n\t"
-            "addc.cc.u32 %4, %4, %12;\n\t"
-            "addc.cc.u32 %5, %5, %13;\n\t"
-            "addc.cc.u32 %6, %6, %14;\n\t"
-            "addc.u32 %7, %7, %15;"
-            : "+r"(T[8]), "+r"(T[9]), "+r"(T[10]), "+r"(T[11]), "+r"(T[12]), "+r"(T[13]), "+r"(T[14]), "+r"(T[15])
-            : "r"(U[8]), "r"(U[9]), "r"(U[10]), "r"(U[11]), "r"(U[12]), "r"(U[13]), "r"(U[14]), "r"(U[15]), "r"(carry));
-        redc8_device(T, lo);
-        Fp r;
-        add256(r.v, lo, T + 8);
-        r.final_sub(0);
-        return r;
-    }
-
     // a^2 / 2^256 mod p: 36-multiply wide square, REDC of the low half, plus the high half
     // (REDC(lo + hi 2^256) = REDC(lo) + hi; REDC(lo) <= p and hi < p^2 / 2^256 < p / 4).
     static PORLA_D Fp sqr_mont_device(const Fp& a) {
@@ -1019,11 +851,7 @@ struct alignas(16) Fp {
     // a*b + c*d (one reduction on the Montgomery device path)
     PORLA_HD static Fp mul2add(const Fp& a, const Fp& b, const Fp& c, const Fp& d) {
 #ifdef __CUDA_ARCH__
-#ifdef PORLA_KARATSUBA
-        if constexpr (P::kMontgomery && !kCompact) return mul2add_mont_karatsuba_device(a, b, c, d);
-#else
         if constexpr (P::kMontgomery && !kCompact) return mul2add_mont_device(a, b, c, d);
-#endif
 #endif
         return mul(a, b) + mul(c, d);
     }
@@ -1031,11 +859,7 @@ struct alignas(16) Fp {
     PORLA_HD static Fp mul_inlined(const Fp& a, const Fp& b) {
         if (P::kMontgomery) {
 #ifdef __CUDA_ARCH__
-#ifdef PORLA_KARATSUBA   // measured slower (see mul_wide_karatsuba_device): off by default
-            return mul_mont_karatsuba_device(a, b);
-#else
             return mul_mont_device(a, b);
-#endif
 #else
             return mul_mont_portable(a, b);
 #endif

@@ -1,9 +1,10 @@
 // Modular inversion without multiplications on the field's multiplier: binary extended GCD in the style of
-// T. Pornin, "Optimized Binary GCD for Modular Inversion" (2020).  The bucket-accumulation kernel in affine coordinates
-// (affine_kernels.cuh) shares one inversion among the additions of a batch; a Fermat inversion (~300 field products) would
-// run on the very pipe that bounds the kernel (IMAD.WIDE), while this routine is ~23 k instructions, mostly plain ALU work
-// (shifts, adds, selects), and overlaps with other warps' field products.  Measured on a B200 (tools/inv_probe.py): 77 k
-// cycles on a lone warp against 272 k for the Fermat inversion; 11.7 k SM-cycles per warp under load against 42 k.
+// T. Pornin, "Optimized Binary GCD for Modular Inversion" (2020).  It is Fp::inverse on the device, behind every
+// conversion to affine coordinates (to_affine, k_fixed_base_mul, the butterfly kernels, k_lut_build).  A Fermat inversion
+// (~300 field products) runs on the multiplier pipe (IMAD.WIDE) that bounds those kernels, while this routine is ~23 k
+// instructions, mostly plain ALU work (shifts, adds, selects), and overlaps with other warps' field products.  Measured on a
+// B200 (tools/inv_probe.py): 77 k cycles on a lone warp against 272 k for the Fermat inversion; 11.7 k SM-cycles per warp
+// under load against 42 k.
 //
 //   a = y, b = m, u = 1, v = 0;   invariants  a = u y,  b = v y  (mod m)
 //   repeat: 30 steps of the binary GCD on 64-bit APPROXIMATIONS of (a, b) -- their top 34 bits and their low 30 bits --

@@ -11,7 +11,6 @@
 #include "msm.h"
 #include "msm_kernels.cuh"
 #include "small_kernels.cuh"
-#include "affine_kernels.cuh"
 
 namespace porla {
 
@@ -265,18 +264,6 @@ void msm_impl(const PointTable& table, const uint8_t* d_scalars, uint32_t n, uin
     if (L < 16) L = 16;
     if (L > 64) L = 64;
     if (const char* e = getenv("PORLA_SLICE_LEN")) { if (atoi(e) >= 2) L = (uint32_t)atoi(e); }
-    // Accumulation in affine coordinates with shared inversions (affine_kernels.cuh): slices of 64 pairs reduced as a tree,
-    // 1 or 2 batched rounds.  PORLA_ACC_AFFINE = number of rounds (0: the XYZZ kernel).
-    int aff_rounds = 0;
-    {
-        const char* e = getenv("PORLA_ACC_AFFINE");
-        const bool big = pairs_cap >= (uint64_t)148 * PORLA_AFF_MIN_BLOCKS * kAffThreads * kAffL * 2;
-        const int want = e ? atoi(e) : (big ? kAffDefaultRounds : 0);
-        if (want > 0 && !streamed) {
-            aff_rounds = want > 2 ? 2 : want;
-            L = kAffL;
-        }
-    }
     const uint32_t nslices_cap = (uint32_t)((pairs_cap + L - 1) / L);
     // One serial XYZZ addition is ~7 us of latency: with few slices in flight (small MSMs) a bucket cut into
     // dozens of slices is better finished by a cooperating block; with the machine full, the serial loop in
@@ -472,19 +459,11 @@ void msm_impl(const PointTable& table, const uint8_t* d_scalars, uint32_t n, uin
     }
     if (total_scalars) {
         g_stage_timer.mark(kStageAccumulate, stream);
-        if (aff_rounds > 0)
-            k_accumulate_affine<C><<<(nslices_cap + kAffThreads - 1) / kAffThreads, kAffThreads, 0, stream>>>(
-                points, reinterpret_cast<const F*>(table.d_phi_x), sh.phi_off, sorted, grand, buckets, part_head, part_tail, aff_rounds);
-        else
-            k_accumulate<C><<<(nslices_cap + kAccThreads - 1) / kAccThreads, kAccThreads, 0, stream>>>(
-                points, reinterpret_cast<const F*>(table.d_phi_x), sh.phi_off, sorted, grand, L, buckets, part_head, part_tail, into);
+        k_accumulate<C><<<(nslices_cap + kAccThreads - 1) / kAccThreads, kAccThreads, 0, stream>>>(
+            points, reinterpret_cast<const F*>(table.d_phi_x), sh.phi_off, sorted, grand, L, buckets, part_head, part_tail, into);
         LAUNCHED();
-        if (getenv("PORLA_STITCH_COMPACT"))
-            k_stitch<C, FC><<<(nslices_cap + 63) / 64, 64, 0, stream>>>(sorted, grand, L, (XC*)buckets, (const XC*)part_head,
-                                                                       (const XC*)part_tail, long_count, long_runs, serial_limit);
-        else
-            k_stitch<C, F><<<(nslices_cap + 63) / 64, 64, 0, stream>>>(sorted, grand, L, buckets, part_head, part_tail,
-                                                                      long_count, long_runs, serial_limit);
+        k_stitch<C><<<(nslices_cap + 63) / 64, 64, 0, stream>>>(sorted, grand, L, buckets, part_head, part_tail, long_count,
+                                                               long_runs, serial_limit);
         LAUNCHED();
         k_stitch_long<C><<<148, kLongThreads, 0, stream>>>(sorted, grand, L, (XC*)buckets, (const XC*)part_head, long_count,
                                                           long_runs);
@@ -623,30 +602,28 @@ void butterfly_impl(PointTable* t, uint32_t m, const uint8_t* d_twiddles, int sc
         PORLA_CUDA(cudaMalloc(&t->d_flags, t->n));
         PORLA_CUDA(cudaMemsetAsync(t->d_flags, 0, t->n, stream));
     }
-    // Measured per stage (one B200, warm clocks, tools/butterfly_times.py), BN254:
+    // Measured per stage (one B200, warm clocks), BN254:
     //   n = 1024 (512 butterflies, pure latency): plain double-and-add 2.16 ms inlined / 2.69 ms compact field type;
     //            GLV joint double-and-add (127 doublings, one extra inversion per butterfly) 1.39 / 1.67 ms
     //   n = 2^20: plain 42.1 / 47.3 ms, GLV 26.6 / 31.3 ms
     // so BN254 always runs the inlined GLV form; secp256k1 (no GLV) keeps the inlined type for few butterflies and
     // the compact one when the machine is full.
-    const char* force = getenv("PORLA_BUTTERFLY_FIELD");
-    const bool inlined = force ? force[0] == 'i' : (C::kGlv || nb < 148u * 512u);
-    const char* fg = getenv("PORLA_BUTTERFLY_GLV");
-    const bool glv = C::kGlv && (fg ? fg[0] == '1' : true);
     auto* pf = reinterpret_cast<Affine<typename C::F>*>(t->d_points);
-    auto* pc = reinterpret_cast<Affine<typename C::FC>*>(t->d_points);
     const dim3 grid((nb + 127) / 128);
-    // Few butterflies (at most two warps of quads per scheduler: 148 x 4 x 2 x 8 = 9472): four lanes per butterfly
-    // (k_butterfly_quad; PORLA_BUTTERFLY_QUAD=0 / 1 forces).  Measured per stage at n = 1024: see DESIGN.md section 4.
-    const char* fq = getenv("PORLA_BUTTERFLY_QUAD");
-    bool quad = false;
-    if constexpr (C::kGlv) quad = glv && (fq ? fq[0] == '1' : nb <= 9472u);
-    if (quad) {
-        if constexpr (C::kGlv) k_butterfly_quad<C><<<(nb * 4 + kBflyQuadThreads - 1) / kBflyQuadThreads, kBflyQuadThreads, 0, stream>>>(pf, t->d_flags, t->n, m, d_twiddles, scalar_be);
-    } else if (inlined && glv) k_butterfly<C, typename C::F, true><<<grid, 128, 0, stream>>>(pf, t->d_flags, t->n, m, d_twiddles, scalar_be);
-    else if (inlined) k_butterfly<C, typename C::F, false><<<grid, 128, 0, stream>>>(pf, t->d_flags, t->n, m, d_twiddles, scalar_be);
-    else if (glv) k_butterfly<C, typename C::FC, true><<<grid, 128, 0, stream>>>(pc, t->d_flags, t->n, m, d_twiddles, scalar_be);
-    else k_butterfly<C, typename C::FC, false><<<grid, 128, 0, stream>>>(pc, t->d_flags, t->n, m, d_twiddles, scalar_be);
+    if constexpr (C::kGlv) {
+        // Few butterflies (at most two warps of quads per scheduler: 148 x 4 x 2 x 8 = 9472): four lanes per butterfly
+        // (k_butterfly_quad; PORLA_BUTTERFLY_QUAD=0 / 1 forces).  Measured per stage at n = 1024: see DESIGN.md section 4.
+        const char* fq = getenv("PORLA_BUTTERFLY_QUAD");
+        if (fq ? fq[0] == '1' : nb <= 9472u)
+            k_butterfly_quad<C><<<(nb * 4 + kBflyQuadThreads - 1) / kBflyQuadThreads, kBflyQuadThreads, 0, stream>>>(pf, t->d_flags, t->n, m, d_twiddles, scalar_be);
+        else
+            k_butterfly<C, typename C::F><<<grid, 128, 0, stream>>>(pf, t->d_flags, t->n, m, d_twiddles, scalar_be);
+    } else if (nb < 148u * 512u) {
+        k_butterfly<C, typename C::F><<<grid, 128, 0, stream>>>(pf, t->d_flags, t->n, m, d_twiddles, scalar_be);
+    } else {
+        auto* pc = reinterpret_cast<Affine<typename C::FC>*>(t->d_points);
+        k_butterfly<C, typename C::FC><<<grid, 128, 0, stream>>>(pc, t->d_flags, t->n, m, d_twiddles, scalar_be);
+    }
     LAUNCHED();
     if constexpr (C::kGlv) {
         if (t->phi_off) {   // the points changed: so does their endomorphism image

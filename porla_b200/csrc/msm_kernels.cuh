@@ -727,8 +727,8 @@ k_partition_fine(const uint2* __restrict__ part, const uint32_t* __restrict__ to
     }
 }
 
-// ---------------------------------------------------------------------------- sort without the exact histogram (round 2, opt-in:
-// PORLA_SORT_V2=1 -- measured slower overall than the default, see msm_impl.cuh and profiles/r02b_sort_without_exact_histogram.txt)
+// ---------------------------------------------------------------------------- sort without the exact histogram (round 2: the
+// default radix path when the coarse bins fit a block, see msm_impl.cuh and profiles/r02b_sort_without_exact_histogram.txt)
 // The exact bucket histogram (k_digits<COUNT>: one global atomic per pair, 218 M of them at 2^24) exists only to give every
 // bucket its output range.  The radix path does not need it: a COARSE histogram (one counter per 2^lb consecutive buckets,
 // kept in shared memory while a block walks its share of the scalars) is enough to place the coarse bins, and each coarse
@@ -1135,12 +1135,13 @@ k_accumulate(const Affine<typename C::F>* __restrict__ points, const typename C:
 constexpr uint32_t kStitchSerial = 48;       // throughput setting: many cut buckets, every thread busy
 constexpr uint32_t kStitchSerialSmall = 8;   // latency setting: few slices in total, hand long runs to a block early
 
-template <class C, class F>
+template <class C>
 __global__ void __launch_bounds__(64)
 k_stitch(const uint2* __restrict__ sorted, const uint32_t* __restrict__ total_pairs, uint32_t L,
-         XYZZ<F>* __restrict__ buckets, const XYZZ<F>* __restrict__ part_head,
-         const XYZZ<F>* __restrict__ part_tail, uint32_t* __restrict__ long_count,
+         XYZZ<typename C::F>* __restrict__ buckets, const XYZZ<typename C::F>* __restrict__ part_head,
+         const XYZZ<typename C::F>* __restrict__ part_tail, uint32_t* __restrict__ long_count,
          uint2* __restrict__ long_runs, uint32_t serial_limit) {
+    using F = typename C::F;
     const uint32_t M = *total_pairs;
     const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
     const uint64_t start64 = (uint64_t)t * L;
@@ -1560,7 +1561,7 @@ k_scalar_mul(const Affine<typename C::FC>* __restrict__ points, uint32_t npoints
 // (main.go:196-222) or secp256k1_ecmult + 2 gej_add_var in IPA mode.  One thread per butterfly, in
 // place on the resident affine table; both outputs share one field inversion.  flags[] (1 =
 // infinity) is rewritten so that MSMs over the table keep skipping infinities.
-template <class C, class F, bool GLV>
+template <class C, class F>
 __global__ void __launch_bounds__(128)
 k_butterfly(Affine<F>* __restrict__ pts, uint8_t* __restrict__ flags, uint32_t n, uint32_t m,
             const uint8_t* __restrict__ twiddles, int big_endian) {
@@ -1573,7 +1574,7 @@ k_butterfly(Affine<F>* __restrict__ pts, uint8_t* __restrict__ flags, uint32_t n
     reduce_scalar<C>(s);
     const Affine<F> a0 = ld16(pts + k), a1 = ld16(pts + k + m2);
     XYZZ<F> t = XYZZ<F>::inf();
-    if constexpr (GLV && C::kGlv) {
+    if constexpr (C::kGlv) {
         // w = k1 + k2 lambda: joint double-and-add over (P, phi(P), P + phi(P)), 127 doublings instead of 254.
         // Every lane of the warp adds an AFFINE operand chosen by its two bits (infinity for 00), so the warp
         // executes one doubling and one mixed addition per bit whatever the lanes' digits are.

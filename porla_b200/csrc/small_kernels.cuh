@@ -42,21 +42,13 @@ __device__ __noinline__ void xyzz_add_shared(XYZZ<F>* a, const XYZZ<F>* b) {
 // Sum of v over the first `count` threads of the block (count <= kTreeThreads); every thread must call.
 // The result is returned to thread 0.  Each addition of the tree is carried by FOUR lanes (quad.cuh: 2.35 us against 6.1 us
 // for the dependent addition of a lone warp), so a level of up to 32 additions is one round of the block's 32 quads and the
-// 7 levels of a 128-value sum take 8 rounds of ~2.4 us instead of 7 additions of ~6.3 us.  PORLA_TREE_SERIAL (compile-time)
-// keeps the one-thread-per-addition tree for comparison.
+// 7 levels of a 128-value sum take 8 rounds of ~2.4 us instead of 7 additions of ~6.3 us.
 template <class F>
 PORLA_D XYZZ<F> block_tree_sum(const XYZZ<F>& v, uint32_t count, XYZZ<F>* sh) {
     sh[threadIdx.x] = v;
     __syncthreads();
     uint32_t o = 1;
     while (o < count) o <<= 1;
-#ifdef PORLA_TREE_SERIAL
-#pragma unroll 1
-    for (o >>= 1; o > 0; o >>= 1) {
-        if (threadIdx.x < o && threadIdx.x + o < count) xyzz_add_shared(&sh[threadIdx.x], &sh[threadIdx.x + o]);
-        __syncthreads();
-    }
-#else
     const uint32_t quad = threadIdx.x >> 2, role = threadIdx.x & 3;
 #pragma unroll 1
     for (o >>= 1; o > 0; o >>= 1) {
@@ -76,7 +68,6 @@ PORLA_D XYZZ<F> block_tree_sum(const XYZZ<F>& v, uint32_t count, XYZZ<F>* sh) {
         }
         __syncthreads();
     }
-#endif
     XYZZ<F> r = sh[0];
     __syncthreads();
     return r;

@@ -158,11 +158,11 @@ def test_window_sizes_agree(window, monkeypatch):
     assert got == O.bn254_marshal(O.msm(BN, sc, pts))
 
 
-@pytest.mark.parametrize("switch", ["PORLA_REDUCE_V1=1", "PORLA_SORT_V2=0", "PORLA_SORT_V2=1", "PORLA_ACC_AFFINE=1"])
+@pytest.mark.parametrize("switch", ["PORLA_REDUCE_V1=1", "PORLA_SORT_V2=0", "PORLA_SORT_V2=1"])
 @pytest.mark.parametrize("n,window", [(600, 9), (5000, 0), (70001, 0), ((1 << 19) + 5, 0)])
 def test_opt_in_kernel_variants_agree(switch, n, window, monkeypatch):
-    """The variants behind environment switches (profiles/r02*): the round-1 bucket reduction, the sort with / without the
-    exact histogram, the affine bucket accumulation.  Same bytes as the default pipeline; the large
+    """The variants behind environment switches (profiles/r02*): the round-1 bucket reduction and the sort with / without
+    the exact histogram.  Same bytes as the default pipeline; the large
     sizes go through the resident path with points k_i G and the closed form (sum s_i k_i) G."""
     import torch
     rnd = random.Random(n)

@@ -290,10 +290,14 @@ def test_butterfly_stage_host_buffers_match_oracle_with_edge_cases(route, monkey
     assert bytes(buf) == b"".join(O.bn254_marshal(P) for P in want)
 
 
-@pytest.mark.parametrize("curve,c", [(pb.CURVE_BN254, BN), (pb.CURVE_SECP256K1, SE)])
-def test_fft_in_exponent_all_stages_resident(curve, c):
+@pytest.mark.parametrize("curve,c,quad", [(pb.CURVE_BN254, BN, None), (pb.CURVE_SECP256K1, SE, None), (pb.CURVE_BN254, BN, "0")],
+                         ids=["0-c0", "1-c1", "0-c0-quad0"])
+def test_fft_in_exponent_all_stages_resident(curve, c, quad, monkeypatch):
     """All log2 n stages on a resident table, then an MSM over the transformed table (the infinity flags
-    written by the butterflies must be honoured)."""
+    written by the butterflies must be honoured).  BN254 stages this small take the four-lane kernel; quad = "0" sends
+    them through the one-thread GLV kernel that larger stages use."""
+    if quad is not None:
+        monkeypatch.setenv("PORLA_BUTTERFLY_QUAD", quad)
     rnd = random.Random(5 + curve)
     n = 32
     G = (c.gx, c.gy)
