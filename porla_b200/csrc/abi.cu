@@ -239,10 +239,9 @@ void msm_host_core(int curve, const uint8_t* scalars, const uint8_t* points, int
     if (nbatch == 1 && n >= (1 << 19) && !getenv("PORLA_NO_SPLIT")) {
         // streamed: the terms cross PCIe in parts that are accumulated into one bucket set as they arrive (multi.cu)
         const MsmPlan plan = msm_plan(curve, (uint32_t)n, 1, 0);
-        std::vector<uint8_t> ws((size_t)kMaxPartsPerDevice * plan.nwin * 128);
-        int nparts = 0;
-        msm_host_pipelined(sg, curve, scalars, points, n, scalar_fmt, point_fmt, plan, ws.data(), &nparts);
-        finalize_host_parts(curve, ws.data(), nparts, plan.nwin, plan.c, point_fmt, out);
+        std::vector<uint8_t> ws((size_t)plan.nwin * 128);
+        msm_host_pipelined(sg, curve, scalars, points, n, scalar_fmt, point_fmt, plan, ws.data());
+        finalize_host(curve, ws.data(), plan.nwin, plan.c, point_fmt, out);
         return;
     }
     const size_t total = (size_t)n * (size_t)nbatch;

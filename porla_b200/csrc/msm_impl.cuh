@@ -165,6 +165,19 @@ void msm_small_impl(const PointTable& table, const uint8_t* d_scalars, uint32_t 
 }
 
 // ---------------------------------------------------------------------------- the pipeline
+// f(std::true_type) for a GLV MSM, else f(std::false_type): f launches the kernel instantiation decltype(g)::value selects,
+// and curves without the endomorphism never instantiate the GLV one.
+template <class C, class Fn>
+void with_glv(bool glv, Fn&& f) {
+    if constexpr (C::kGlv) {
+        if (glv) {
+            f(std::true_type{});
+            return;
+        }
+    }
+    f(std::false_type{});
+}
+
 template <class C>
 void msm_impl(const PointTable& table, const uint8_t* d_scalars, uint32_t n, uint32_t nbatch,
                      const MsmOptions& opt, uint8_t* d_out, void* d_out_xyzz, cudaStream_t stream) {
@@ -318,7 +331,7 @@ void msm_impl(const PointTable& table, const uint8_t* d_scalars, uint32_t n, uin
     // 2.07 -> see profiles/r02b_sort_without_exact_histogram.txt.
     const char* sv2 = getenv("PORLA_SORT_V2");
     const bool v2_fits = ncoarse > 0 && pairs_cap / ncoarse <= (uint64_t)(kBigBin * 0.95);
-    const bool sort_v2 = radix && lb <= 10 && (size_t)ncoarse * 4 <= (160u << 10) && (sv2 ? sv2[0] == '1' : v2_fits);
+    const bool sort_v2 = radix && lb <= 10 && (size_t)ncoarse * 4 <= (size_t)kCoarseCountSmem && (sv2 ? sv2[0] == '1' : v2_fits);
     PORLA_CUDA(cudaMemsetAsync(counters, 0, (size_t)nbt * 4, stream));
     PORLA_CUDA(cudaMemsetAsync(grand, 0, 4, stream));
     PORLA_CUDA(cudaMemsetAsync(long_count, 0, 4, stream));
@@ -327,54 +340,41 @@ void msm_impl(const PointTable& table, const uint8_t* d_scalars, uint32_t n, uin
     static_assert(sizeof(XYZZ<F>) == 128, "k_fine_smem / k_big_scan clear 128-byte bucket records");
     if (!into && !sort_v2) PORLA_CUDA(cudaMemsetAsync(buckets, 0, (size_t)nbt * sizeof(XYZZ<F>), stream));
     uint4* zero_buckets = into ? nullptr : reinterpret_cast<uint4*>(buckets);
-    if (total_scalars && sort_v2) {
-        static std::once_flag attr_once_dev2[kMaxDevices];   // function attributes are per device
-        const size_t smem0 = (size_t)ncoarse * 4;
-        const size_t smem1 = ((size_t)9 * kPartTile + 2 * kPartMaxBins) * 4 + (size_t)kPartTile * 8;
-        const size_t smem2 = (size_t)2 * kFineHist * 4 + (size_t)kFineTile * 8;
-        const size_t smem3 = (size_t)kBigBin * 6 + (size_t)kFineLocalBuckets * 4;
-        std::call_once(attr_once_dev2[current_device()], [=] {
-            PORLA_CUDA(cudaFuncSetAttribute(k_coarse_count<C, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 << 10));
-            PORLA_CUDA(cudaFuncSetAttribute(k_partition_coarse<C, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
+    if (radix) {
+        static std::once_flag attr_once[kMaxDevices];   // function attributes are per device
+        std::call_once(attr_once[current_device()], [] {
+            PORLA_CUDA(cudaFuncSetAttribute(k_coarse_count<C, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kCoarseCountSmem));
+            PORLA_CUDA(cudaFuncSetAttribute(k_partition_coarse<C, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPartCoarseSmem));
             if constexpr (C::kGlv) {
-                PORLA_CUDA(cudaFuncSetAttribute(k_coarse_count<C, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 << 10));
-                PORLA_CUDA(cudaFuncSetAttribute(k_partition_coarse<C, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
+                PORLA_CUDA(cudaFuncSetAttribute(k_coarse_count<C, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kCoarseCountSmem));
+                PORLA_CUDA(cudaFuncSetAttribute(k_partition_coarse<C, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPartCoarseSmem));
             }
-            PORLA_CUDA(cudaFuncSetAttribute(k_partition_fine_big, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
-            PORLA_CUDA(cudaFuncSetAttribute(k_fine_smem, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3));
+            PORLA_CUDA(cudaFuncSetAttribute(k_partition_fine<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPartFineSmem));
+            PORLA_CUDA(cudaFuncSetAttribute(k_partition_fine<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPartFineSmem));
+            PORLA_CUDA(cudaFuncSetAttribute(k_fine_smem, cudaFuncAttributeMaxDynamicSharedMemorySize, kFineLocalSmem));
         });
+    }
+    if (total_scalars && sort_v2) {
         uint32_t* coarse_count = offsets;                 // the exact-offset array is not needed on this path: reuse it
         uint32_t* coarse_off = offsets + ncoarse + 1;     // (nbt >= 2 * (ncoarse + 1): 2^lb >= 16 buckets per bin)
         PORLA_CUDA(cudaMemsetAsync(coarse_count, 0, (size_t)(ncoarse + 1) * 4, stream));
         uint32_t cgrid = (uint32_t)((total_scalars + kCoarseCountThreads - 1) / kCoarseCountThreads);
         if (cgrid > 148u * 2u) cgrid = 148u * 2u;
-        bool glv_done = false;
-        if constexpr (C::kGlv) {
-            if (glv) {
-                k_coarse_count<C, true><<<cgrid, kCoarseCountThreads, smem0, stream>>>(d_scalars, opt.scalar_be, table.d_flags, sh, lb, ncoarse, coarse_count);
-                glv_done = true;
-            }
-        }
-        if (!glv_done)
-            k_coarse_count<C, false><<<cgrid, kCoarseCountThreads, smem0, stream>>>(d_scalars, opt.scalar_be, table.d_flags, sh, lb, ncoarse, coarse_count);
+        with_glv<C>(glv, [&](auto g) {
+            k_coarse_count<C, decltype(g)::value><<<cgrid, kCoarseCountThreads, (size_t)ncoarse * 4, stream>>>(
+                d_scalars, opt.scalar_be, table.d_flags, sh, lb, ncoarse, coarse_count);
+        });
         LAUNCHED();
         g_stage_timer.mark(kStageScan, stream);
         k_coarse_scan<<<1, 1024, 0, stream>>>(coarse_count, ncoarse, coarse_off, coarse_cursor, grand);
         LAUNCHED();
         g_stage_timer.mark(kStageScatter, stream);
-        glv_done = false;
-        if constexpr (C::kGlv) {
-            if (glv) {
-                k_partition_coarse<C, true><<<(n + kPartTile - 1) / kPartTile, kPartThreads, smem1, stream>>>(
-                    d_scalars, opt.scalar_be, table.d_flags, sh, lb, coarse_cursor, part);
-                glv_done = true;
-            }
-        }
-        if (!glv_done)
-            k_partition_coarse<C, false><<<(n + kPartTile - 1) / kPartTile, kPartThreads, smem1, stream>>>(
+        with_glv<C>(glv, [&](auto g) {
+            k_partition_coarse<C, decltype(g)::value><<<(n + kPartTile - 1) / kPartTile, kPartThreads, kPartCoarseSmem, stream>>>(
                 d_scalars, opt.scalar_be, table.d_flags, sh, lb, coarse_cursor, part);
+        });
         LAUNCHED();
-        k_fine_smem<<<ncoarse, kFineSmemThreads, smem3, stream>>>(part, coarse_off, lb, sorted, zero_buckets);
+        k_fine_smem<<<ncoarse, kFineSmemThreads, kFineLocalSmem, stream>>>(part, coarse_off, lb, sorted, zero_buckets);
         LAUNCHED();
         // bins too long for one block (skewed inputs): counted, scanned and scattered by tiles; no-ops otherwise
         const uint32_t tiles = (uint32_t)((pairs_cap + kFineTile - 1) / kFineTile);
@@ -382,20 +382,15 @@ void msm_impl(const PointTable& table, const uint8_t* d_scalars, uint32_t n, uin
         LAUNCHED();
         k_big_scan<<<ncoarse, kFineLocalThreads, 0, stream>>>(coarse_off, lb, counters, zero_buckets);
         LAUNCHED();
-        k_partition_fine_big<<<tiles, kFineThreads, smem2, stream>>>(part, grand, coarse_off, lb, counters, sorted);
+        k_partition_fine<true><<<tiles, kFineThreads, kPartFineSmem, stream>>>(part, grand, coarse_off, lb, counters, sorted);
         LAUNCHED();
     } else if (total_scalars) {
         uint32_t grid = (uint32_t)((total_scalars + 255) / 256);
         if (grid > 148u * 32u) grid = 148u * 32u;
-        bool launched_glv = false;
-        if constexpr (C::kGlv) {
-            if (glv) {
-                k_digits<C, false, true><<<grid, 256, 0, stream>>>(d_scalars, opt.scalar_be, table.d_flags, sh, 0, sh.nwin, counters, nullptr);
-                launched_glv = true;
-            }
-        }
-        if (!launched_glv)
-            k_digits<C, false, false><<<grid, 256, 0, stream>>>(d_scalars, opt.scalar_be, table.d_flags, sh, 0, sh.nwin, counters, nullptr);
+        with_glv<C>(glv, [&](auto g) {
+            k_digits<C, false, decltype(g)::value><<<grid, 256, 0, stream>>>(d_scalars, opt.scalar_be, table.d_flags, sh, 0, sh.nwin,
+                                                                              counters, nullptr);
+        });
         LAUNCHED();
         g_stage_timer.mark(kStageScan, stream);
         k_scan_tiles<<<ntiles, kScanThreads, 0, stream>>>(counters, offsets, nbt, tile_sums);
@@ -406,32 +401,15 @@ void msm_impl(const PointTable& table, const uint8_t* d_scalars, uint32_t n, uin
         LAUNCHED();
         g_stage_timer.mark(kStageScatter, stream);
         if (radix) {
-            static std::once_flag attr_once_dev[kMaxDevices];   // function attributes are per device
-            std::once_flag& attr_once = attr_once_dev[current_device()];
-            const size_t smem1 = ((size_t)9 * kPartTile + 2 * kPartMaxBins) * 4 + (size_t)kPartTile * 8;
-            const size_t smem2 = (size_t)2 * kFineHist * 4 + (size_t)kFineTile * 8;
-            std::call_once(attr_once, [=] {
-                PORLA_CUDA(cudaFuncSetAttribute(k_partition_coarse<C, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
-                if constexpr (C::kGlv)
-                    PORLA_CUDA(cudaFuncSetAttribute(k_partition_coarse<C, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
-                PORLA_CUDA(cudaFuncSetAttribute(k_partition_fine, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
-            });
             k_init_coarse<<<(ncoarse + 255) / 256, 256, 0, stream>>>(offsets, nbt, lb, ncoarse, coarse_cursor);
             LAUNCHED();
-            bool coarse_glv = false;
-            if constexpr (C::kGlv) {
-                if (glv) {
-                    k_partition_coarse<C, true><<<(n + kPartTile - 1) / kPartTile, kPartThreads, smem1, stream>>>(
-                        d_scalars, opt.scalar_be, table.d_flags, sh, lb, coarse_cursor, part);
-                    coarse_glv = true;
-                }
-            }
-            if (!coarse_glv)
-                k_partition_coarse<C, false><<<(n + kPartTile - 1) / kPartTile, kPartThreads, smem1, stream>>>(
+            with_glv<C>(glv, [&](auto g) {
+                k_partition_coarse<C, decltype(g)::value><<<(n + kPartTile - 1) / kPartTile, kPartThreads, kPartCoarseSmem, stream>>>(
                     d_scalars, opt.scalar_be, table.d_flags, sh, lb, coarse_cursor, part);
+            });
             LAUNCHED();
-            k_partition_fine<<<(uint32_t)((pairs_cap + kFineTile - 1) / kFineTile), kFineThreads, smem2, stream>>>(part, grand, lb,
-                                                                                                             counters, sorted);
+            k_partition_fine<false><<<(uint32_t)((pairs_cap + kFineTile - 1) / kFineTile), kFineThreads, kPartFineSmem, stream>>>(
+                part, grand, nullptr, lb, counters, sorted);
             LAUNCHED();
         } else {
         // windows per scatter launch: keep the written region of `sorted` (8 B per pair) around 64 MB
@@ -444,15 +422,10 @@ void msm_impl(const PointTable& table, const uint8_t* d_scalars, uint32_t n, uin
         }
         for (int w0 = 0; w0 < sh.nwin; w0 += wgroup) {
             int w1 = w0 + wgroup < sh.nwin ? w0 + wgroup : sh.nwin;
-            bool scatter_glv = false;
-            if constexpr (C::kGlv) {
-                if (glv) {
-                    k_digits<C, true, true><<<grid, 256, 0, stream>>>(d_scalars, opt.scalar_be, table.d_flags, sh, w0, w1, counters, sorted);
-                    scatter_glv = true;
-                }
-            }
-            if (!scatter_glv)
-                k_digits<C, true, false><<<grid, 256, 0, stream>>>(d_scalars, opt.scalar_be, table.d_flags, sh, w0, w1, counters, sorted);
+            with_glv<C>(glv, [&](auto g) {
+                k_digits<C, true, decltype(g)::value><<<grid, 256, 0, stream>>>(d_scalars, opt.scalar_be, table.d_flags, sh, w0, w1,
+                                                                                 counters, sorted);
+            });
             LAUNCHED();
         }
         }

@@ -186,6 +186,37 @@ PORLA_D void glv_split(const uint32_t* k, uint32_t* k1, uint32_t* k2, uint32_t& 
     }
 }
 
+// ---------------------------------------------------------------------------- scalar preparation
+// scalar idx -> canonical magnitude (reduced mod the order; secp256k1: min(s, n - s) with flip = 1 when negated)
+template <class C>
+PORLA_D uint32_t canonical_scalar(const uint8_t* __restrict__ scalars, size_t idx, int big_endian, uint32_t* s) {
+    load_u256(scalars, idx, big_endian, s);
+    reduce_scalar<C>(s);
+    uint32_t flip = 0;
+    if (C::kHalveScalar) {
+        uint32_t ord[8], t[8], u[8];
+#pragma unroll
+        for (int k = 0; k < 8; k++) ord[k] = C::order(k);
+        sub256(t, ord, s);                 // order - s  (s < order)
+        if (sub256(u, t, s)) {             // order - s < s
+            flip = 1;
+#pragma unroll
+            for (int k = 0; k < 8; k++) s[k] = t[k];
+        }
+    }
+    return flip;
+}
+
+// scalar idx, reduced mod r and GLV-split -> |k1|, |k2| (4 limbs each) and their signs (neg = 1: negate the point)
+template <class C>
+PORLA_D void glv_scalar(const uint8_t* __restrict__ scalars, size_t idx, int big_endian, uint32_t* k1, uint32_t* k2,
+                        uint32_t& neg1, uint32_t& neg2) {
+    uint32_t k[8];
+    load_u256(scalars, idx, big_endian, k);
+    reduce_scalar<C>(k);
+    glv_split<C>(k, k1, k2, neg1, neg2);
+}
+
 // out[i] = beta * x_i: the x coordinate of the endomorphism image (beta x_i, y_i) of every table entry
 template <class C>
 __global__ void __launch_bounds__(128)
@@ -337,27 +368,12 @@ k_digits(const uint8_t* __restrict__ scalars, int big_endian,
         uint32_t s[kLimbs];
         uint32_t flip[2] = {0, 0};   // negate the point (per half with GLV)
         if constexpr (GLV) {
-            uint32_t k[8];
-            load_u256(scalars, idx, big_endian, k);
-            reduce_scalar<C>(k);
-            glv_split<C>(k, s, s + 5, flip[0], flip[1]);
+            glv_scalar<C>(scalars, idx, big_endian, s, s + 5, flip[0], flip[1]);
             s[4] = 0;
             s[9] = 0;
         } else {
-            load_u256(scalars, idx, big_endian, s);
             s[8] = 0;
-            reduce_scalar<C>(s);
-            if (C::kHalveScalar) {   // s > order/2: use order - s and the negated point
-                uint32_t ord[8], t[8], u[8];
-#pragma unroll
-                for (int k = 0; k < 8; k++) ord[k] = C::order(k);
-                sub256(t, ord, s);                 // order - s  (s < order)
-                if (sub256(u, t, s)) {             // order - s < s
-                    flip[0] = 1;
-#pragma unroll
-                    for (int k = 0; k < 8; k++) s[k] = t[k];
-                }
-            }
+            flip[0] = canonical_scalar<C>(scalars, idx, big_endian, s);
         }
         uint32_t carry = 0;
         // general: one bucket set per (msm, window); fixed-base: one per msm, the window selects the
@@ -530,6 +546,7 @@ constexpr int kFinePerThread = 8;
 constexpr int kFineTile = kFineThreads * kFinePerThread;   // 4096 pairs
 constexpr uint32_t kFineHist = 4096;                       // shared histogram entries of pass 2
 constexpr uint32_t kMetaSkip = 1u << 30, kMetaFlip = 1u << 31, kMetaFlip2 = 1u << 29;
+constexpr uint32_t kBigBin = 34816;   // pairs per bin k_fine_smem keeps in shared memory (6 B each: 204 KB + the histogram)
 
 static __global__ void k_init_coarse(const uint32_t* __restrict__ offsets, uint32_t nbt, int lb, uint32_t ncoarse,
                                      uint32_t* __restrict__ coarse_cursor) {
@@ -537,6 +554,7 @@ static __global__ void k_init_coarse(const uint32_t* __restrict__ offsets, uint3
     if (g < ncoarse) coarse_cursor[g] = offsets[(size_t)g << lb];
 }
 
+constexpr int kPartCoarseSmem = (9 * kPartTile + 2 * kPartMaxBins) * 4 + kPartTile * 8;   // dynamic shared memory: the layout below
 template <class C, bool GLV>
 __global__ void __launch_bounds__(kPartThreads, PORLA_PART_MIN_BLOCKS)
 k_partition_coarse(const uint8_t* __restrict__ scalars, int big_endian, const uint8_t* __restrict__ inf_flags,
@@ -560,27 +578,12 @@ k_partition_coarse(const uint8_t* __restrict__ scalars, int big_endian, const ui
         uint32_t m = kMetaSkip;
         uint32_t s[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};     // GLV: |k1| in s[0..3], |k2| in s[4..7]
         if (i < sh.n && !(inf_flags && inf_flags[i])) {
-            m = 0;
             if constexpr (GLV) {
-                uint32_t k[8], n1, n2;
-                load_u256(scalars, i, big_endian, k);
-                reduce_scalar<C>(k);
-                glv_split<C>(k, s, s + 4, n1, n2);
+                uint32_t n1, n2;
+                glv_scalar<C>(scalars, i, big_endian, s, s + 4, n1, n2);
                 m = (n1 ? kMetaFlip : 0u) | (n2 ? kMetaFlip2 : 0u);
             } else {
-                load_u256(scalars, i, big_endian, s);
-                reduce_scalar<C>(s);
-                if (C::kHalveScalar) {
-                    uint32_t ord[8], t[8], u[8];
-#pragma unroll
-                    for (int k = 0; k < 8; k++) ord[k] = C::order(k);
-                    sub256(t, ord, s);
-                    if (sub256(u, t, s)) {
-                        m = kMetaFlip;
-#pragma unroll
-                        for (int k = 0; k < 8; k++) s[k] = t[k];
-                    }
-                }
+                m = canonical_scalar<C>(scalars, i, big_endian, s) ? kMetaFlip : 0u;
             }
         }
 #pragma unroll
@@ -665,9 +668,17 @@ k_partition_coarse(const uint8_t* __restrict__ scalars, int big_endian, const ui
     }
 }
 
+PORLA_D bool bin_is_big(const uint32_t* __restrict__ coarse_off, uint32_t bin) {
+    return coarse_off[bin + 1] - coarse_off[bin] > kBigBin;
+}
+
+constexpr int kPartFineSmem = 2 * kFineHist * 4 + kFineTile * 8;   // dynamic shared memory: the layout below
+// kBigOnly: only the pairs of bins above kBigBin pairs, for the sort without the exact histogram (cursor = the offsets
+// k_big_scan wrote; tiles without such pairs return at once).  Otherwise coarse_off is not read.
+template <bool kBigOnly>
 static __global__ void __launch_bounds__(kFineThreads, 3)
-k_partition_fine(const uint2* __restrict__ part, const uint32_t* __restrict__ total_pairs, int lb,
-                 uint32_t* __restrict__ cursor, uint2* __restrict__ sorted) {
+k_partition_fine(const uint2* __restrict__ part, const uint32_t* __restrict__ total_pairs, const uint32_t* __restrict__ coarse_off,
+                 int lb, uint32_t* __restrict__ cursor, uint2* __restrict__ sorted) {
     extern __shared__ uint32_t smem[];
     uint32_t* cnt = smem;                                   // [kFineHist] counts, then local offsets
     uint32_t* delta = cnt + kFineHist;                      // [kFineHist] reserved global base - local offset
@@ -678,8 +689,15 @@ k_partition_fine(const uint2* __restrict__ part, const uint32_t* __restrict__ to
     if (lo64 >= M) return;
     const uint32_t lo = (uint32_t)lo64;
     const uint32_t hi = M - lo > (uint32_t)kFineTile ? lo + kFineTile : M;
+    const uint32_t bin_lo = __ldg(&part[lo].x) >> lb;
+    if constexpr (kBigOnly) {   // the tile covers the bins of its first .. last pair
+        const uint32_t bin_hi = __ldg(&part[hi - 1].x) >> lb;
+        bool any = false;
+        for (uint32_t b = bin_lo; b <= bin_hi && !any; b++) any = bin_is_big(coarse_off, b);
+        if (!any) return;
+    }
     for (uint32_t b = threadIdx.x; b < kFineHist; b += kFineThreads) cnt[b] = 0;
-    const uint32_t kbase = (__ldg(&part[lo].x) >> lb) << lb;
+    const uint32_t kbase = bin_lo << lb;
     __syncthreads();
     uint2 e[kFinePerThread];
     uint32_t rank[kFinePerThread];
@@ -688,9 +706,12 @@ k_partition_fine(const uint2* __restrict__ part, const uint32_t* __restrict__ to
         const uint32_t idx = lo + q * kFineThreads + threadIdx.x;
         e[q] = make_uint2(0xffffffffu, 0u);
         if (idx < hi) {
-            e[q] = __ldg(&part[idx]);
-            const uint32_t rel = e[q].x - kbase;      // pass 1 keeps coarse bins in order, so rel >= 0
-            if (rel < kFineHist) rank[q] = atomicAdd(&cnt[rel], 1u);
+            const uint2 v = __ldg(&part[idx]);
+            if (!kBigOnly || bin_is_big(coarse_off, v.x >> lb)) {
+                e[q] = v;
+                const uint32_t rel = v.x - kbase;      // pass 1 keeps coarse bins in order, so rel >= 0
+                if (rel < kFineHist) rank[q] = atomicAdd(&cnt[rel], 1u);
+            }
         }
     }
     __syncthreads();
@@ -739,12 +760,12 @@ k_partition_fine(const uint2* __restrict__ part, const uint32_t* __restrict__ to
 //   k_fine_smem      block b owns coarse bin b: histogram of its buckets, scan, placement in shared memory, ordered write-out
 // Skewed inputs (a constant scalar, 31-bit scalars' empty top windows ...) put up to all pairs of a window into one coarse
 // bin; bins above kBigBin pairs are left to the tile-based route, which is the round-1 fine pass preceded by its own
-// counting pass over the same tiles (k_big_count, k_big_scan, k_partition_fine_big) and costs nothing when no bin is big.
-constexpr uint32_t kBigBin = 34816;   // pairs per bin k_fine_smem keeps in shared memory (6 B each: 204 KB + the histogram)
+// counting pass over the same tiles (k_big_count, k_big_scan, k_partition_fine<true>) and costs nothing when no bin is big.
 constexpr int kCoarseCountThreads = 512;
 constexpr int kFineLocalThreads = 256;
 constexpr uint32_t kFineLocalBuckets = 1024;   // 2^lb <= 2^10 buckets per coarse bin (c <= 20)
 
+constexpr int kCoarseCountSmem = 160 << 10;   // dynamic shared memory limit: one counter per coarse bin of every window
 template <class C, bool GLV>
 __global__ void __launch_bounds__(kCoarseCountThreads)
 k_coarse_count(const uint8_t* __restrict__ scalars, int big_endian, const uint8_t* __restrict__ inf_flags, MsmShape sh, int lb,
@@ -758,23 +779,10 @@ k_coarse_count(const uint8_t* __restrict__ scalars, int big_endian, const uint8_
         if (inf_flags && inf_flags[i]) continue;
         uint32_t s[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};     // GLV: |k1| in s[0..3], |k2| in s[4..7]
         if constexpr (GLV) {
-            uint32_t k[8], n1, n2;
-            load_u256(scalars, i, big_endian, k);
-            reduce_scalar<C>(k);
-            glv_split<C>(k, s, s + 4, n1, n2);
+            uint32_t n1, n2;
+            glv_scalar<C>(scalars, i, big_endian, s, s + 4, n1, n2);
         } else {
-            load_u256(scalars, i, big_endian, s);
-            reduce_scalar<C>(s);
-            if (C::kHalveScalar) {
-                uint32_t ord[8], t[8], u[8];
-#pragma unroll
-                for (int k = 0; k < 8; k++) ord[k] = C::order(k);
-                sub256(t, ord, s);
-                if (sub256(u, t, s)) {
-#pragma unroll
-                    for (int k = 0; k < 8; k++) s[k] = t[k];
-                }
-            }
+            canonical_scalar<C>(scalars, i, big_endian, s);
         }
         // Walk the value word by word with a 64-bit shift register: the limbs are indexed statically (a dynamically indexed
         // register array cost ~40 instructions of compare / select chains per window here), one c-bit digit per turn.
@@ -840,6 +848,7 @@ k_coarse_scan(const uint32_t* __restrict__ coarse_count, uint32_t ncoarse, uint3
 // global memory: 3.85 ms at 2^24 with 2.6 % of the issue slots used, 5.1 GB read and 3.5 GB written for 1.75 GB of pairs;
 // profiles/r02b_sort_without_exact_histogram.txt).  Six bytes of shared memory per pair: bins of up to kBigBin pairs.
 constexpr int kFineSmemThreads = 1024;
+constexpr int kFineLocalSmem = kBigBin * 6 + kFineLocalBuckets * 4;   // dynamic shared memory: the layout below
 static __global__ void __launch_bounds__(kFineSmemThreads, 1)
 k_fine_smem(const uint2* __restrict__ part, const uint32_t* __restrict__ coarse_off, int lb, uint2* __restrict__ sorted,
             uint4* __restrict__ zero_buckets) {
@@ -912,10 +921,6 @@ k_fine_smem(const uint2* __restrict__ part, const uint32_t* __restrict__ coarse_
 }
 
 // ---- bins above kBigBin pairs: the tile-based fine pass with its own counting pass
-PORLA_D bool bin_is_big(const uint32_t* __restrict__ coarse_off, uint32_t bin) {
-    return coarse_off[bin + 1] - coarse_off[bin] > kBigBin;
-}
-
 static __global__ void __launch_bounds__(kFineThreads)
 k_big_count(const uint2* __restrict__ part, const uint32_t* __restrict__ total_pairs, const uint32_t* __restrict__ coarse_off,
             int lb, uint32_t* __restrict__ counters) {
@@ -967,76 +972,6 @@ k_big_scan(const uint32_t* __restrict__ coarse_off, int lb, uint32_t* __restrict
         if (i < nb) c[i] = carry + ex;
         carry += total;
         __syncthreads();
-    }
-}
-
-// k_partition_fine restricted to the pairs of big bins (cursor = the offsets k_big_scan wrote)
-static __global__ void __launch_bounds__(kFineThreads, 3)
-k_partition_fine_big(const uint2* __restrict__ part, const uint32_t* __restrict__ total_pairs, const uint32_t* __restrict__ coarse_off,
-                     int lb, uint32_t* __restrict__ cursor, uint2* __restrict__ sorted) {
-    extern __shared__ uint32_t smem[];
-    uint32_t* cnt = smem;                                   // [kFineHist] counts, then local offsets
-    uint32_t* delta = cnt + kFineHist;                      // [kFineHist] reserved global base - local offset
-    uint2* stage = reinterpret_cast<uint2*>(delta + kFineHist);   // [kFineTile] pairs grouped by bucket
-    __shared__ uint32_t s_total;
-    const uint32_t M = *total_pairs;
-    const uint64_t lo64 = (uint64_t)blockIdx.x * kFineTile;
-    if (lo64 >= M) return;
-    const uint32_t lo = (uint32_t)lo64;
-    const uint32_t hi = M - lo > (uint32_t)kFineTile ? lo + kFineTile : M;
-    const uint32_t bin_lo = __ldg(&part[lo].x) >> lb, bin_hi = __ldg(&part[hi - 1].x) >> lb;
-    bool any = false;
-    for (uint32_t b = bin_lo; b <= bin_hi && !any; b++) any = bin_is_big(coarse_off, b);
-    if (!any) return;
-    for (uint32_t b = threadIdx.x; b < kFineHist; b += kFineThreads) cnt[b] = 0;
-    const uint32_t kbase = bin_lo << lb;
-    __syncthreads();
-    uint2 e[kFinePerThread];
-    uint32_t rank[kFinePerThread];
-#pragma unroll
-    for (int q = 0; q < kFinePerThread; q++) {
-        const uint32_t idx = lo + q * kFineThreads + threadIdx.x;
-        e[q] = make_uint2(0xffffffffu, 0u);
-        if (idx < hi) {
-            const uint2 v = __ldg(&part[idx]);
-            if (bin_is_big(coarse_off, v.x >> lb)) {
-                e[q] = v;
-                const uint32_t rel = v.x - kbase;
-                if (rel < kFineHist) rank[q] = atomicAdd(&cnt[rel], 1u);
-            }
-        }
-    }
-    __syncthreads();
-    {
-        constexpr uint32_t ept = kFineHist / kFineThreads;   // 8
-        uint32_t v[ept], sum = 0;
-        const uint32_t b0 = threadIdx.x * ept;
-#pragma unroll
-        for (uint32_t k = 0; k < ept; k++) {
-            v[k] = cnt[b0 + k];
-            sum += v[k];
-        }
-        uint32_t ex = block_exclusive_scan(sum, &s_total);
-#pragma unroll
-        for (uint32_t k = 0; k < ept; k++) {
-            cnt[b0 + k] = ex;
-            delta[b0 + k] = v[k] ? atomicAdd(&cursor[kbase + b0 + k], v[k]) - ex : 0u;
-            ex += v[k];
-        }
-    }
-    __syncthreads();
-#pragma unroll
-    for (int q = 0; q < kFinePerThread; q++) {
-        if (e[q].x == 0xffffffffu) continue;
-        const uint32_t rel = e[q].x - kbase;
-        if (rel < kFineHist) stage[cnt[rel] + rank[q]] = e[q];
-        else sorted[atomicAdd(&cursor[e[q].x], 1u)] = e[q];
-    }
-    __syncthreads();
-    const uint32_t total = s_total;
-    for (uint32_t j = threadIdx.x; j < total; j += kFineThreads) {
-        const uint2 x = stage[j];
-        sorted[delta[x.x - kbase] + j] = x;
     }
 }
 
@@ -1660,10 +1595,8 @@ k_butterfly_quad(Affine<typename C::F>* __restrict__ pts, uint8_t* __restrict__ 
     const bool live = b < n / 2;
     const uint32_t bb = live ? b : 0u;
     const uint32_t j = bb % m2, k = (bb / m2) * m + j;
-    uint32_t s[8], k1[4], k2[4], n1, n2;
-    load_u256(twiddles, j, big_endian, s);
-    reduce_scalar<C>(s);
-    glv_split<C>(s, k1, k2, n1, n2);
+    uint32_t k1[4], k2[4], n1, n2;
+    glv_scalar<C>(twiddles, j, big_endian, k1, k2, n1, n2);
     Q a1 = Q::load_affine(pts + k + m2, false);
     if (!live) a1 = Q::inf();
     {

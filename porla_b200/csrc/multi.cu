@@ -291,8 +291,33 @@ static int stream_parts_for(int64_t n, const MsmPlan& plan) {
     return p < 1 ? 1 : (p > 8 ? 8 : (int)p);
 }
 
+// End of part h of n terms in `nparts` streamed parts: the first part is half a regular part (its copy is the exposed one),
+// the last part takes what that leaves.
+static int64_t part_end(int64_t n, int h, int nparts) {
+    return h == nparts - 1 ? n : (n * (2 * h + 1)) / (2 * nparts);
+}
+
+static int part_mode(int h, int nparts) {
+    return nparts == 1 ? kPartWhole : (h == 0 ? kPartFirst : (h == nparts - 1 ? kPartLast : kPartMiddle));
+}
+
+// Options of an MSM that hands its plan.nwin window sums to the caller: the window layout is forced to `plan`, so that all
+// parts of one MSM fill the same buckets and all devices produce window sums that add up.
+static MsmOptions window_sums_options(const MsmPlan& plan, int scalar_fmt, int out_fmt, void* d_window_sums) {
+    MsmOptions opt;
+    opt.scalar_be = scalar_fmt == PORLA_SCALAR_BE32;
+    opt.out_fmt = out_fmt;
+    opt.shared_points = 1;
+    opt.window_bits = plan.c;
+    opt.glv = plan.glv;
+    opt.no_fixed_base = 1;
+    opt.no_small = 1;
+    opt.d_window_sums = d_window_sums;
+    return opt;
+}
+
 void msm_host_pipelined(Staging& sg, int curve, const uint8_t* scalars, const uint8_t* points, int64_t n, int scalar_fmt,
-                        int point_fmt, const MsmPlan& plan, uint8_t* h_ws, int* nparts_out) {
+                        int point_fmt, const MsmPlan& plan, uint8_t* h_ws) {
     auto pad = [](size_t v) { return (v + 255) & ~(size_t)255; };
     const int nparts = stream_parts_for(n, plan);
     const size_t ws_bytes = (size_t)plan.nwin * 128;
@@ -302,20 +327,11 @@ void msm_host_pipelined(Staging& sg, int curve, const uint8_t* scalars, const ui
            ws_off = fl_off + pad((size_t)n), bk_off = ws_off + pad(ws_bytes);
     uint8_t* d = sg.dev(bk_off + pad(bk_bytes));
     cudaStream_t st = sg.stream, cs = sg.copy_stream;
-    MsmOptions opt;
-    opt.scalar_be = scalar_fmt == PORLA_SCALAR_BE32;
-    opt.out_fmt = point_fmt;
-    opt.shared_points = 1;
-    opt.window_bits = plan.c;
-    opt.glv = plan.glv;           // every part with the same layout: they fill the same buckets
-    opt.no_fixed_base = 1;
-    opt.no_small = 1;
-    opt.d_window_sums = d + ws_off;
+    MsmOptions opt = window_sums_options(plan, scalar_fmt, point_fmt, d + ws_off);
     if (nparts > 1) opt.d_buckets = d + bk_off;
     int64_t first = 0;
     for (int h = 0; h < nparts; h++) {
-        // the first part is half a regular part (its copy is the exposed one), the last part takes what that leaves
-        const int64_t last = h == nparts - 1 ? n : (n * (2 * h + 1)) / (2 * nparts);
+        const int64_t last = part_end(n, h, nparts);
         const size_t a = (size_t)first, m = (size_t)(last - first);
         h2d_copy(d + sc_off + a * 32, scalars + a * 32, m * 32, cs);
         h2d_copy(d + pt_off + a * 64, points + a * 64, m * 64, cs);
@@ -323,7 +339,7 @@ void msm_host_pipelined(Staging& sg, int curve, const uint8_t* scalars, const ui
         PORLA_CUDA(cudaStreamWaitEvent(st, sg.ev[h], 0));
         PointTable tab;
         table_import_into(curve, d + pt_off + a * 64, point_fmt, (uint32_t)m, d + tab_off + a * 128, d + fl_off + a, &tab, st);
-        opt.part_mode = nparts == 1 ? kPartWhole : (h == 0 ? kPartFirst : (h == nparts - 1 ? kPartLast : kPartMiddle));
+        opt.part_mode = part_mode(h, nparts);
         msm_device(curve, tab, d + sc_off + a * 32, (uint32_t)m, 1, opt, nullptr, nullptr, st);
         first = last;
     }
@@ -331,7 +347,6 @@ void msm_host_pipelined(Staging& sg, int curve, const uint8_t* scalars, const ui
     PORLA_CUDA(cudaMemcpyAsync(hbuf, d + ws_off, ws_bytes, cudaMemcpyDeviceToHost, st));
     PORLA_CUDA(cudaStreamSynchronize(st));
     memcpy(h_ws, hbuf, ws_bytes);
-    *nparts_out = 1;
 }
 
 // ---------------------------------------------------------------------------- fan-out over the devices of the box
@@ -347,25 +362,16 @@ static void device_ranges(int64_t n, int ndev, int64_t* first, int64_t* count) {
 void msm_host_fanout(int curve, const uint8_t* scalars, const uint8_t* points, int64_t n, int scalar_fmt, int point_fmt,
                      int ndev, uint8_t* out64) {
     int64_t first[kMaxDevices], count[kMaxDevices];
-    int nparts[kMaxDevices];
     device_ranges(n, ndev, first, count);
     const MsmPlan plan = msm_plan(curve, (uint32_t)count[ndev - 1], 1, 0);
     const size_t ws_bytes = (size_t)plan.nwin * 128;
-    std::vector<uint8_t> ws((size_t)ndev * kMaxPartsPerDevice * ws_bytes);
+    std::vector<uint8_t> ws((size_t)ndev * ws_bytes);
     run_on_devices(ndev, [&](int p) {
         msm_host_pipelined(worker_staging(), curve, scalars + (size_t)first[p] * 32, points + (size_t)first[p] * 64, count[p],
-                           scalar_fmt, point_fmt, plan, ws.data() + (size_t)p * kMaxPartsPerDevice * ws_bytes, &nparts[p]);
+                           scalar_fmt, point_fmt, plan, ws.data() + (size_t)p * ws_bytes);
     });
-    // compact the parts (a device may have produced one or two) and combine: add window by window, Horner, normalise
-    std::vector<uint8_t> all;
-    all.reserve(ws.size());
-    int total = 0;
-    for (int p = 0; p < ndev; p++) {
-        const uint8_t* src = ws.data() + (size_t)p * kMaxPartsPerDevice * ws_bytes;
-        all.insert(all.end(), src, src + (size_t)nparts[p] * ws_bytes);
-        total += nparts[p];
-    }
-    finalize_host_parts(curve, all.data(), total, plan.nwin, plan.c, point_fmt, out64);
+    // one set of window sums per device: add window by window, Horner, normalise
+    finalize_host_parts(curve, ws.data(), ndev, plan.nwin, plan.c, point_fmt, out64);
 }
 
 }  // namespace porla
@@ -466,33 +472,23 @@ static void mtable_msm(const porla_mtable* mt, const uint8_t* h_scalars, void* c
         const size_t m = (size_t)mt->count[p];
         const uint8_t* d_sc;
         const int nparts = d_scalars_per_part ? 1 : stream_parts_for((int64_t)m, plan);
+        MsmOptions opt = window_sums_options(plan, scalar_fmt, out_fmt, mt->d_ws[p]);
         if (d_scalars_per_part) {
             d_sc = (const uint8_t*)d_scalars_per_part[p];
         } else if (nparts > 1) {
             // host scalars of a large range: streamed like msm_host_pipelined -- the scalars of part h+1 cross PCIe while
             // part h (a view of the resident table) is accumulated into the shared bucket set
-            const size_t bk_bytes = msm_bucket_bytes(plan);
-            uint8_t* d_bk = sg.dev(bk_bytes);
-            MsmOptions so;
-            so.scalar_be = scalar_fmt == PORLA_SCALAR_BE32;
-            so.out_fmt = out_fmt;
-            so.shared_points = 1;
-            so.window_bits = plan.c;
-            so.glv = plan.glv;
-            so.no_fixed_base = 1;
-            so.no_small = 1;
-            so.d_window_sums = mt->d_ws[p];
-            so.d_buckets = d_bk;
+            opt.d_buckets = sg.dev(msm_bucket_bytes(plan));
             size_t a = 0;
             for (int h = 0; h < nparts; h++) {
-                const size_t last = h == nparts - 1 ? m : (m * (2 * (size_t)h + 1)) / (2 * (size_t)nparts);
+                const size_t last = (size_t)part_end((int64_t)m, h, nparts);
                 const size_t len = last - a;
                 h2d_copy(mt->d_scalars[p] + a * 32, h_scalars + ((size_t)mt->first[p] + a) * 32, len * 32, sg.copy_stream);
                 PORLA_CUDA(cudaEventRecord(sg.ev[h], sg.copy_stream));
                 PORLA_CUDA(cudaStreamWaitEvent(sg.stream, sg.ev[h], 0));
                 const PointTable view = table_view(mt->part[p], a, len);   // entries [a, a + len) of this device's range
-                so.part_mode = h == 0 ? kPartFirst : (h == nparts - 1 ? kPartLast : kPartMiddle);
-                msm_device(mt->curve, view, mt->d_scalars[p] + a * 32, (uint32_t)len, 1, so, nullptr, nullptr, sg.stream);
+                opt.part_mode = part_mode(h, nparts);
+                msm_device(mt->curve, view, mt->d_scalars[p] + a * 32, (uint32_t)len, 1, opt, nullptr, nullptr, sg.stream);
                 a = last;
             }
             d_sc = nullptr;
@@ -500,15 +496,6 @@ static void mtable_msm(const porla_mtable* mt, const uint8_t* h_scalars, void* c
             h2d_copy(mt->d_scalars[p], h_scalars + (size_t)mt->first[p] * 32, m * 32, sg.stream);
             d_sc = mt->d_scalars[p];
         }
-        MsmOptions opt;
-        opt.scalar_be = scalar_fmt == PORLA_SCALAR_BE32;
-        opt.out_fmt = out_fmt;
-        opt.shared_points = 1;
-        opt.window_bits = plan.c;
-        opt.glv = plan.glv;
-        opt.no_fixed_base = 1;
-        opt.no_small = 1;
-        opt.d_window_sums = mt->d_ws[p];
         if (m && d_sc)
             msm_device(mt->curve, mt->part[p], d_sc, (uint32_t)m, 1, opt, nullptr, nullptr, sg.stream);
         else if (!m) PORLA_CUDA(cudaMemsetAsync(mt->d_ws[p], 0, ws_bytes, sg.stream));

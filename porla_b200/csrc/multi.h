@@ -26,13 +26,11 @@ int part_device(int part);
 // The staging area of the calling worker thread's device (valid inside run_on_devices only).
 Staging& worker_staging();
 
-// One MSM over host buffers on the CURRENT device in one or two pipelined parts (the copy of the second part runs
-// under the first part's kernels): writes `*nparts_out` sets of plan.nwin window sums (128 B each) to h_ws and
-// returns after the stream has been synchronised.  `plan` must be a pipeline plan; all parts of one MSM, on every
-// device, share it.
+// One MSM over host buffers on the CURRENT device, streamed in parts that accumulate into one bucket set (the copy of
+// part h+1 runs under part h's kernels): writes plan.nwin window sums (128 B each) to h_ws and returns after the stream
+// has been synchronised.  `plan` must be a pipeline plan; all parts of one MSM, on every device, share it.
 void msm_host_pipelined(Staging& sg, int curve, const uint8_t* scalars, const uint8_t* points, int64_t n, int scalar_fmt,
-                        int point_fmt, const MsmPlan& plan, uint8_t* h_ws, int* nparts_out);
-constexpr int kMaxPartsPerDevice = 2;
+                        int point_fmt, const MsmPlan& plan, uint8_t* h_ws);
 
 // The n-term MSM over host buffers partitioned over `ndev` devices (devices 0 .. ndev-1), result to out64.
 void msm_host_fanout(int curve, const uint8_t* scalars, const uint8_t* points, int64_t n, int scalar_fmt, int point_fmt,

@@ -106,26 +106,6 @@ PORLA_D void fold_blocks(const XYZZ<F>& v, uint32_t slot, uint32_t blk, uint32_t
     if (threadIdx.x == 0) st16(out + slot, r);
 }
 
-// scalar idx -> canonical magnitude (reduced mod the order; secp256k1: min(s, n - s) with flip = 1 when negated)
-template <class C>
-PORLA_D uint32_t canonical_scalar(const uint8_t* __restrict__ scalars, size_t idx, int big_endian, uint32_t* s) {
-    load_u256(scalars, idx, big_endian, s);
-    reduce_scalar<C>(s);
-    uint32_t flip = 0;
-    if (C::kHalveScalar) {
-        uint32_t ord[8], t[8], u[8];
-#pragma unroll
-        for (int k = 0; k < 8; k++) ord[k] = C::order(k);
-        sub256(t, ord, s);
-        if (sub256(u, t, s)) {
-            flip = 1;
-#pragma unroll
-            for (int k = 0; k < 8; k++) s[k] = t[k];
-        }
-    }
-    return flip;
-}
-
 // ---------------------------------------------------------------------------- variable bases, one bit per window
 // grid = (chunks of 2*kTreeThreads points, nbits, nbatch); out[m * nbits + b] = W_b of MSM m.
 template <class C>
