@@ -224,13 +224,14 @@ static WindowChoice choose_window_ex(int curve, uint32_t n, uint32_t nbatch, int
     const int bits = scalar_bits(curve);
     const bool glv_ok = glv_allowed(curve);
     const char* force_glv = getenv("PORLA_GLV");
+    // a plan code fixes the whole layout, whatever the window size (the search below only covers 3 .. 20)
+    if (forced_c > 0 && forced_glv == 1 && glv_ok) return WindowChoice{forced_c, 1};
+    if (forced_c > 0 && forced_glv == 0) return WindowChoice{forced_c, 0};
     double best = 1e300;
     WindowChoice ch{forced_c > 0 ? forced_c : 4, 0};
     for (int c = 3; c <= 20; c++) {   // 20: the widest window the shared-memory radix partition packs
         if (forced_c > 0 && c != forced_c) continue;
         double plain = window_cost(bits, (double)n, nbatch, c);
-        if (forced_glv == 1 && glv_ok && forced_c > 0) return WindowChoice{forced_c, 1};
-        if (forced_glv == 0 && forced_c > 0) return WindowChoice{forced_c, 0};
         if (force_glv && force_glv[0] == '1' && glv_ok) plain = -1;
         if (plain >= 0 && plain < best) {
             best = plain;

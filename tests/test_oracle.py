@@ -185,6 +185,49 @@ def test_glv_constants_in_the_kernel_header_and_split_bounds():
         assert abs(k1) < 1 << 127 and abs(k2) < 1 << 127
 
 
+def test_recoding_restatement_on_its_edge_families():
+    """oracle/recoding_py.py is the specification the radix-route GPU tests check the window sums against: its digits must
+    rebuild s mod the order (k1 + k2 lambda with GLV), stay within 2^(c-1), never carry out of the top window, and come in
+    as many windows as porla_msm_plan (host-only) reports, for every window size on both curves, on the families that sit
+    on the recoding's edges."""
+    import ctypes as C
+    import porla_b200 as pb
+    from oracle import recoding_py as R
+    lam = R.glv_consts()["lambda"]
+    lib = pb.load()
+    for curve, cv, glv in ((pb.CURVE_BN254, BN, False), (pb.CURVE_BN254, BN, True), (pb.CURVE_SECP256K1, SE, False)):
+        signs = set()
+        for c in range(2, 25):
+            code = c | (pb.lib.PLAN_GLV_ON if glv else pb.lib.PLAN_GLV_OFF)
+            got, nwin = C.c_int(0), C.c_int(0)
+            lib.porla_msm_plan(curve, (1 << 19) + 37, 1, code, C.byref(got), C.byref(nwin))
+            assert got.value == code and nwin.value == R.num_windows(cv, glv, c), (cv.name, glv, c)
+            half = 1 << (c - 1)
+            for name, vals in R.families(cv, glv, c, 24, seed=c).items():
+                for s in vals:
+                    parts = R.recode(cv, glv, c, s)
+                    total = 0
+                    for h, ((sign, digits, carry), (_, mag)) in enumerate(zip(parts, R.halves(cv, glv, s))):
+                        where = (cv.name, glv, c, name, hex(s), h)
+                        assert len(digits) == nwin.value and carry == 0, where
+                        assert all(abs(d) <= half for d in digits), where
+                        assert sum(d << (c * w) for w, d in enumerate(digits)) == mag, where
+                        if mag and name == "tie":
+                            assert digits[0] == half, where
+                        if mag and name == "carry_chain":
+                            assert digits[0] < 0, where
+                        total += sign * (lam if h else 1) * mag
+                        signs.add((h, sign, mag == 0))
+                    assert (total - s) % cv.n == 0, (cv.name, glv, c, name, hex(s))
+                    deltas = R.window_multipliers(cv, glv, c, s)
+                    assert (sum(d << (c * w) for w, d in enumerate(deltas)) - s) % cv.n == 0, (cv.name, glv, c, name, hex(s))
+        # the families reach the sign cases the kernels handle: the secp256k1 flip, and k2 < 0 and k2 = 0 with GLV
+        if cv is SE:
+            assert {(0, -1, False), (0, 1, False)} <= signs
+        if glv:
+            assert {(1, -1, False), (1, 1, True)} <= signs
+
+
 def test_ipa_transcript_sha_matches_the_reference_object():
     """Porla's IPA prover keeps ONE secp256k1_sha256 and finalizes it again and again (Server.hpp:2306-2310, 2386-2387):
     the oracle's restatement of that object against the reference's own hash_impl.h compiled into oracle/_ref."""
