@@ -290,6 +290,14 @@ size_t porla_secp256k1_inner_product_prove(const porla_table* gens_and_u, size_t
  * proof's L / R points and one look-up-table multi-exponentiation over the table. */
 int porla_secp256k1_inner_product_verify(const porla_table* gens_and_u, size_t n, const porla_secp256k1_gej* commitment,
                                          const unsigned char* proof);
+/* One stage of the FFT in the exponent on IPA-mode MACs (the rebuild butterflies of Server.hpp:1548-1830 / Client.hpp:921-976,
+ * secp256k1_ecmult + 2 gej_add_var each), in place: for every j < m/2, k = j, j+m, ... < n
+ *   t = w_j * P[k + m/2];  P[k] <- P[k] + t;  P[k + m/2] <- P[k] - t
+ * points: n secp256k1_gej (any z, any field magnitude, infinity flag honoured); twiddles: m/2 secp256k1_scalar, taken mod n.
+ * Outputs: z = 1, normalised limbs, infinity as gej_set_infinity writes it.  Returns 0 (buffer untouched) unless m is a
+ * power of two >= 2 dividing n, else 1.  Stages of at most PORLA_HOST_BUTTERFLIES butterflies (default 32) run on the
+ * calling host without touching the device; larger ones on the GPU (k_butterfly_quad / k_butterfly). */
+int porla_secp256k1_butterfly_stage(porla_secp256k1_gej* points, size_t n, size_t m, const porla_secp256k1_scalar* twiddles);
 /* 33-byte SEC1 compressed form of a gej/ge result (eckey_impl.h:36-52); returns 0 for infinity. */
 int porla_secp256k1_gej_serialize(const porla_secp256k1_gej* a, unsigned char out33[33]);
 

@@ -33,5 +33,6 @@ from .lib import (  # noqa: F401
     msm_host,
     msm_host_devices,
     secp256k1_ecmult_multi_var,
+    secp256k1_butterfly_stage,
     SecpGenerators,
 )

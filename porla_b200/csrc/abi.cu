@@ -4,6 +4,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <mutex>
 #include <shared_mutex>
 #include <thread>
@@ -57,10 +58,14 @@ struct ClientState {
     uint64_t powers_gen = 0;
 };
 ClientState g_client;
-std::mutex g_io_mu;                 // serialises the staging buffers below
+}  // namespace
 
-// staging of the default device for the large host-buffer calls (struct Staging: staging.h)
+namespace porla {
+std::mutex g_io_mu;
 Staging g_stage;
+}  // namespace porla
+
+namespace {
 
 // Small calls (Porla's 16..766-term MSMs and 128-term commitments) lease one of a few persistent staging slots (device
 // buffer, pinned buffer, stream, scratch block) and do not take g_io_mu: the pool threads of Server.hpp:1077-1078 /
@@ -1018,28 +1023,21 @@ void porla_butterfly_stage_device(porla_table* t, int64_t m, const void* twiddle
     }
 }
 
+}  // extern "C"
+
+namespace porla {
 // A stage of at most this many butterflies runs on the calling host (up to 8 threads), like the single-point symbols it
 // replaces: one butterfly is a dependent chain of ~127 doublings and additions, 1.4 ms on one GPU thread against 0.1 ms on a
 // host core, so the device only wins once there are enough butterflies to fill it (measured with tools/replay_config1:
-// Porla's per-update hierarchy rebuilds issue stages of 1 .. 512 butterflies).  PORLA_HOST_BUTTERFLIES overrides (0: always device).
-static int64_t host_butterfly_limit() {
+// Porla's per-update hierarchy rebuilds issue stages of 1 .. 512 butterflies).  secp256k1 crosses over sooner: its host
+// stage takes 0.39 / 0.92 ms at 32 / 64 butterflies against ~0.56 ms for a stage through the device (one B200, 1000 W;
+// tools/secp_butterfly_times.py).  PORLA_HOST_BUTTERFLIES overrides (0: always device).
+int64_t host_butterfly_limit(int curve) {
     const char* e = getenv("PORLA_HOST_BUTTERFLIES");
-    return e ? (int64_t)atoll(e) : (int64_t)96;
+    return e ? (int64_t)atoll(e) : (curve == kCurveBn254 ? (int64_t)96 : (int64_t)32);
 }
 
-static void butterfly_stage_host(uint8_t* pts, int64_t n, int64_t m, const uint8_t* tw) {
-    const int64_t m2 = m / 2, nb = n / 2;
-    auto body = [&](int64_t lo, int64_t hi) {
-        for (int64_t b = lo; b < hi; b++) {
-            const int64_t j = b % m2, k = (b / m2) * m + j;
-            G1A a0 = G1A::inf(), a1 = G1A::inf();
-            g1_unmarshal(pts + 64 * k, 64, &a0);
-            g1_unmarshal(pts + 64 * (k + m2), 64, &a1);
-            const G1A t = g1_mul(a1, elem_from_be<Fr>(tw + 32 * j, 32));
-            g1_marshal(g1_add(a0, t), pts + 64 * k);
-            g1_marshal(g1_add(a0, t.neg()), pts + 64 * (k + m2));
-        }
-    };
+void for_each_butterfly_host(int64_t nb, const std::function<void(int64_t, int64_t)>& body) {
     const int64_t nt = nb >= 16 ? 8 : (nb >= 4 ? 4 : 1);
     if (nt == 1) {
         body(0, nb);
@@ -1049,6 +1047,24 @@ static void butterfly_stage_host(uint8_t* pts, int64_t n, int64_t m, const uint8
     for (int64_t t = 0; t < nt; t++) th.emplace_back(body, nb * t / nt, nb * (t + 1) / nt);
     for (auto& x : th) x.join();
 }
+}  // namespace porla
+
+static void butterfly_stage_host(uint8_t* pts, int64_t n, int64_t m, const uint8_t* tw) {
+    const int64_t m2 = m / 2;
+    for_each_butterfly_host(n / 2, [&](int64_t lo, int64_t hi) {
+        for (int64_t b = lo; b < hi; b++) {
+            const int64_t j = b % m2, k = (b / m2) * m + j;
+            G1A a0 = G1A::inf(), a1 = G1A::inf();
+            g1_unmarshal(pts + 64 * k, 64, &a0);
+            g1_unmarshal(pts + 64 * (k + m2), 64, &a1);
+            const G1A t = g1_mul(a1, elem_from_be<Fr>(tw + 32 * j, 32));
+            g1_marshal(g1_add(a0, t), pts + 64 * k);
+            g1_marshal(g1_add(a0, t.neg()), pts + 64 * (k + m2));
+        }
+    });
+}
+
+extern "C" {
 
 void bn254_butterfly_stage(GoSlice* points, GoInt n, GoInt m, GoSlice* twiddles) {
     if (n < 0 || points->len < n * 64 || twiddles->len < (m / 2) * 32)
@@ -1056,7 +1072,7 @@ void bn254_butterfly_stage(GoSlice* points, GoInt n, GoInt m, GoSlice* twiddles)
     if (m < 2 || (m & (m - 1)) || n % m) die("bn254_butterfly_stage: m must be a power of two dividing n");
     if (n == 0) return;
     check_shape(n, 1, "bn254_butterfly_stage");
-    if (n / 2 <= host_butterfly_limit()) {
+    if (n / 2 <= host_butterfly_limit(kCurveBn254)) {
         butterfly_stage_host((uint8_t*)points->data, n, m, (const uint8_t*)twiddles->data);
         return;
     }

@@ -5,11 +5,13 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <mutex>
 #include <vector>
 
 #include "../../include/porla_multiexp.h"
 #include "host_bn254.hpp"
 #include "msm.h"
+#include "staging.h"
 
 using namespace porla;
 
@@ -73,6 +75,46 @@ void canonical_to_fe(const uint32_t in[8], porla_secp256k1_fe* r) {
 void gej_set_infinity(porla_secp256k1_gej* r) {
     memset(r, 0, sizeof(*r));
     r->infinity = 1;
+}
+
+using SF = host::Fp64<host::SecpFq64Params>;
+
+// secp256k1_gej (Jacobian, any z, any field magnitude) -> canonical affine x = X / Z^2, y = Y / Z^3 (no inversion when
+// Z = 1); infinity -> Affine::inf()
+Affine<SF> gej_to_affine(const porla_secp256k1_gej* a) {
+    if (a->infinity) return Affine<SF>::inf();
+    uint32_t x[8], y[8], z[8];
+    fe_to_canonical(&a->x, x);
+    fe_to_canonical(&a->y, y);
+    fe_to_canonical(&a->z, z);
+    Affine<SF> r;
+    SF zf;
+    memcpy(r.x.v, x, 32);
+    memcpy(r.y.v, y, 32);
+    memcpy(zf.v, z, 32);
+    if (zf != SF::one()) {
+        const SF zi = zf.inverse(), zi2 = zi.sqr();
+        r.x = r.x * zi2;
+        r.y = r.y * zi2 * zi;
+    }
+    return r;
+}
+
+// 64 bytes of canonical LE affine x || y (all zero: infinity) -> gej with z = 1, or infinity as gej_set_infinity writes it
+void gej_from_le64(const uint8_t* b, porla_secp256k1_gej* r) {
+    uint32_t xy[16];
+    memcpy(xy, b, 64);
+    bool inf = true;
+    for (int i = 0; i < 16; i++) inf = inf && xy[i] == 0;
+    if (inf) {
+        gej_set_infinity(r);
+        return;
+    }
+    canonical_to_fe(xy, &r->x);
+    canonical_to_fe(xy + 8, &r->y);
+    memset(&r->z, 0, sizeof(r->z));
+    r->z.n[0] = 1;
+    r->infinity = 0;
 }
 
 const uint8_t kGenLE[64] = {
@@ -271,9 +313,112 @@ struct TranscriptSha256 {
         }
     }
 };
+
+// ---------------------------------------------------------------------------- FFT in the exponent on IPA-mode MACs
+// k * p on the host for small stages: k = k1 + k2 lambda (glv_split_secp256k1, the device routine), then joint 2 + 2-bit
+// windows over (k1, k2) -- 15 combinations i (+-p) + j (+-phi(p)), 64 steps of two doublings and at most one addition,
+// as g1_mul does for BN254.
+XYZZ<SF> secp_mul_host(const Affine<SF>& p, const porla_secp256k1_scalar& w) {
+    const Sn kn = sn_from_le32((const unsigned char*)w.d);
+    if (p.is_inf() || !(kn.v[0] | kn.v[1] | kn.v[2] | kn.v[3])) return XYZZ<SF>::inf();
+    uint32_t k[8], k1[4], k2[4], n1, n2;
+    memcpy(k, kn.v, 32);
+    glv_split_secp256k1(k, k1, k2, n1, n2);
+    Affine<SF> p1 = p, p2 = p;
+    for (int i = 0; i < 4; i++)
+        p2.x.v[i] = (uint64_t)Secp256k1::glv_beta_mont(2 * i) | ((uint64_t)Secp256k1::glv_beta_mont(2 * i + 1) << 32);
+    p2.x = p.x * p2.x;
+    if (n1) p1.y = p1.y.neg();
+    if (n2) p2.y = p2.y.neg();
+    XYZZ<SF> tab[16];   // tab[4 j + i] = i p1 + j p2
+    tab[0] = XYZZ<SF>::inf();
+    for (int i = 1; i < 4; i++) {
+        tab[i] = tab[i - 1];
+        tab[i].madd(p1);
+    }
+    for (int j = 1; j < 4; j++)
+        for (int i = 0; i < 4; i++) {
+            tab[4 * j + i] = tab[4 * (j - 1) + i];
+            tab[4 * j + i].madd(p2);
+        }
+    auto digit = [&](int d) { return ((k1[d >> 4] >> (2 * (d & 15))) & 3u) | (((k2[d >> 4] >> (2 * (d & 15))) & 3u) << 2); };
+    int top = 63;
+    while (top > 0 && digit(top) == 0) top--;
+    XYZZ<SF> r = tab[digit(top)];
+    for (int d = top - 1; d >= 0; d--) {
+        r = r.dbl().dbl();
+        const uint32_t e = digit(d);
+        if (e) r.add(tab[e]);
+    }
+    return r;
+}
+
+void gej_from_affine(const Affine<SF>& a, porla_secp256k1_gej* r) {
+    uint8_t b[64];
+    memcpy(b, a.x.v, 32);
+    memcpy(b + 32, a.y.v, 32);
+    gej_from_le64(b, r);
+}
+
+void butterfly_stage_host(porla_secp256k1_gej* pts, size_t n, size_t m, const porla_secp256k1_scalar* tw) {
+    const size_t m2 = m / 2;
+    for_each_butterfly_host((int64_t)(n / 2), [&](int64_t lo, int64_t hi) {
+        for (int64_t b = lo; b < hi; b++) {
+            const size_t j = (size_t)b % m2, k = ((size_t)b / m2) * m + j;
+            const Affine<SF> a0 = gej_to_affine(pts + k);
+            const XYZZ<SF> t = secp_mul_host(gej_to_affine(pts + k + m2), tw[j]);
+            XYZZ<SF> r0 = XYZZ<SF>::from_affine(a0), r1 = r0;
+            r0.add(t);
+            r1.add(t.neg());
+            gej_from_affine(r0.to_affine(), pts + k);
+            gej_from_affine(r1.to_affine(), pts + k + m2);
+        }
+    });
+}
+
+// The same stage on the device: limbs normalised here, Jacobian -> affine in k_import_jacobian, the butterfly kernels of
+// butterfly_stage_device, canonical affine back.
+void butterfly_stage_gpu(porla_secp256k1_gej* pts, size_t n, size_t m, const porla_secp256k1_scalar* tw) {
+    std::vector<uint32_t> xyz(24 * n, 0);
+    std::vector<uint8_t> inf(n);
+    for (size_t i = 0; i < n; i++) {
+        inf[i] = pts[i].infinity ? 1 : 0;
+        if (inf[i]) continue;
+        fe_to_canonical(&pts[i].x, &xyz[24 * i]);
+        fe_to_canonical(&pts[i].y, &xyz[24 * i + 8]);
+        fe_to_canonical(&pts[i].z, &xyz[24 * i + 16]);
+    }
+    device_init();
+    std::lock_guard<std::mutex> lock(g_io_mu);
+    g_stage.init();
+    auto pad = [](size_t v) { return (v + 255) & ~(size_t)255; };
+    const size_t o_inf = pad(96 * n), o_tw = o_inf + pad(n), o_pts = o_tw + pad(32 * (m / 2)), o_flags = o_pts + pad(64 * n),
+                 o_out = o_flags + pad(n);
+    uint8_t* d = g_stage.dev(o_out + 64 * n);
+    cudaStream_t st = g_stage.stream;
+    h2d_copy(d, xyz.data(), 96 * n, st);
+    PORLA_CUDA(cudaMemcpyAsync(d + o_inf, inf.data(), n, cudaMemcpyHostToDevice, st));
+    PORLA_CUDA(cudaMemcpyAsync(d + o_tw, tw, 32 * (m / 2), cudaMemcpyHostToDevice, st));
+    PointTable t;
+    table_import_jacobian_secp256k1(reinterpret_cast<const uint32_t*>(d), d + o_inf, (uint32_t)n, d + o_pts, d + o_flags, &t, st);
+    butterfly_stage_device(&t, (uint32_t)m, d + o_tw, 0, st);
+    export_points_device(kCurveSecp256k1, t.d_points, (uint32_t)n, PORLA_POINT_LE64, d + o_out, st);
+    std::vector<uint8_t> out(64 * n);
+    PORLA_CUDA(cudaMemcpyAsync(out.data(), d + o_out, 64 * n, cudaMemcpyDeviceToHost, st));
+    PORLA_CUDA(cudaStreamSynchronize(st));
+    for (size_t i = 0; i < n; i++) gej_from_le64(out.data() + 64 * i, pts + i);
+}
 }  // namespace
 
 extern "C" {
+
+int porla_secp256k1_butterfly_stage(porla_secp256k1_gej* points, size_t n, size_t m, const porla_secp256k1_scalar* twiddles) {
+    if (m < 2 || (m & (m - 1)) || n % m || n > 0xffffffffu) return 0;
+    if (n == 0) return 1;
+    if ((int64_t)(n / 2) <= host_butterfly_limit(kCurveSecp256k1)) butterfly_stage_host(points, n, m, twiddles);
+    else butterfly_stage_gpu(points, n, m, twiddles);
+    return 1;
+}
 
 int porla_secp256k1_ecmult_multi_var(const porla_secp256k1_callback* error_callback, void* scratch,
                                      porla_secp256k1_gej* r, const porla_secp256k1_scalar* inp_g_sc,
@@ -309,16 +454,7 @@ int porla_secp256k1_ecmult_multi_var(const porla_secp256k1_callback* error_callb
     uint8_t res[64];
     porla_msm_host(PORLA_CURVE_SECP256K1, scalars.data(), points.data(), (int64_t)m, 1, PORLA_SCALAR_LE32,
                    PORLA_POINT_LE64, res);
-    uint32_t xy[16];
-    memcpy(xy, res, 64);
-    bool inf = true;
-    for (int i = 0; i < 16; i++) inf = inf && xy[i] == 0;
-    if (inf) return 1;
-    canonical_to_fe(xy, &r->x);
-    canonical_to_fe(xy + 8, &r->y);
-    memset(&r->z, 0, sizeof(r->z));
-    r->z.n[0] = 1;
-    r->infinity = 0;
+    gej_from_le64(res, r);
     return 1;
 }
 
@@ -349,16 +485,7 @@ int porla_secp256k1_ecmult_multi_table(const porla_table* t, size_t first, const
     if ((int64_t)(first + n) > porla_table_len(t)) return 0;
     uint8_t res[64];
     porla_msm_table_host_scalars(t, (int64_t)first, scalars, (int64_t)n, PORLA_SCALAR_LE32, PORLA_POINT_LE64, res);
-    uint32_t xy[16];
-    memcpy(xy, res, 64);
-    bool inf = true;
-    for (int i = 0; i < 16; i++) inf = inf && xy[i] == 0;
-    if (inf) return 1;
-    canonical_to_fe(xy, &r->x);
-    canonical_to_fe(xy + 8, &r->y);
-    memset(&r->z, 0, sizeof(r->z));
-    r->z.n[0] = 1;
-    r->infinity = 0;
+    gej_from_le64(res, r);
     return 1;
 }
 
@@ -446,7 +573,6 @@ int porla_secp256k1_inner_product_verify(const porla_table* gens_and_u, size_t n
     //     commitment + c u + sum_rounds (x^2 L + x^-2 R)   with   (a0 b0 + a1 b1) u + sum_even a0 xv_j g_j + sum_odd a1 xv_j g_j ;
     // here the c u term moves to the right, so the left side is the commitment plus ONE variable-base multi-exponentiation
     // over the proof's points and the right side ONE look-up-table multi-exponentiation over the resident table.
-    using SF = host::Fp64<host::SecpFq64Params>;
     if (n < 4 || (n & (n - 1)) || (int64_t)(n + 1) != porla_table_len(gens_and_u)) return 0;
     size_t rounds = 0;
     for (size_t h = n / 2; h > 1; h >>= 1) rounds++;
@@ -523,20 +649,7 @@ int porla_secp256k1_inner_product_verify(const porla_table* gens_and_u, size_t n
         memcpy(a.y.v, b + 32, 32);
         return a;
     };
-    XYZZ<SF> lhs = XYZZ<SF>::inf();
-    if (!commitment->infinity) {
-        SecpFp cx, cy, cz;
-        fe_to_canonical(&commitment->x, cx.v);
-        fe_to_canonical(&commitment->y, cy.v);
-        fe_to_canonical(&commitment->z, cz.v);
-        const SecpFp zi = cz.inverse(), zi2 = zi.sqr();
-        cx = cx * zi2;
-        cy = cy * zi2 * zi;
-        Affine<SF> ca;
-        memcpy(ca.x.v, cx.v, 32);
-        memcpy(ca.y.v, cy.v, 32);
-        lhs = XYZZ<SF>::from_affine(ca);
-    }
+    XYZZ<SF> lhs = XYZZ<SF>::from_affine(gej_to_affine(commitment));
     lhs.madd(load_affine(lr64));             // all-zero bytes = infinity: madd ignores it
     const Affine<SF> l = lhs.to_affine(), rr = load_affine(rhs64);
     return l.x == rr.x && l.y == rr.y ? 1 : 0;
@@ -544,15 +657,11 @@ int porla_secp256k1_inner_product_verify(const porla_table* gens_and_u, size_t n
 
 int porla_secp256k1_gej_serialize(const porla_secp256k1_gej* a, unsigned char out33[33]) {
     if (a->infinity) return 0;
-    SecpFp x, y, z;
-    fe_to_canonical(&a->x, x.v);
-    fe_to_canonical(&a->y, y.v);
-    fe_to_canonical(&a->z, z.v);
-    SecpFp zi = z.inverse(), zi2 = zi.sqr();
-    x = x * zi2;
-    y = y * zi2 * zi;
-    out33[0] = (y.v[0] & 1u) ? 0x03 : 0x02;  // SECP256K1_TAG_PUBKEY_ODD / EVEN
-    host::limbs_to_be32(x.v, out33 + 1);
+    const Affine<SF> p = gej_to_affine(a);
+    uint32_t x[8];
+    memcpy(x, p.x.v, 32);
+    out33[0] = (p.y.v[0] & 1u) ? 0x03 : 0x02;  // SECP256K1_TAG_PUBKEY_ODD / EVEN
+    host::limbs_to_be32(x, out33 + 1);
     return 1;
 }
 

@@ -80,6 +80,11 @@ int choose_window_fixed_base(int curve, uint32_t n, uint32_t nbatch);
 // no allocation, no sync.  The returned table borrows the buffers (do not table_free it).
 void table_import_into(int curve, const uint8_t* d_bytes, int point_fmt, uint32_t n, void* d_points_out,
                        uint8_t* d_flags_out, PointTable* out, cudaStream_t stream, bool with_phi = true);
+// Import `n` secp256k1 Jacobian points (IPA-mode MACs) into caller-provided device buffers (n * 64 B points, n B flags):
+// d_xyz holds canonical X, Y, Z (8 LE 32-bit limbs each), d_inf their infinity flags; one inversion per point with Z != 1.
+// No allocation, no sync.  The returned table borrows the buffers (do not table_free it).
+void table_import_jacobian_secp256k1(const uint32_t* d_xyz, const uint8_t* d_inf, uint32_t n, void* d_points_out,
+                                     uint8_t* d_flags_out, PointTable* out, cudaStream_t stream);
 
 struct MsmOptions {
     int window_bits = 0;      // 0 = choose from n

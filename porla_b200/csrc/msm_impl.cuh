@@ -579,23 +579,17 @@ void butterfly_impl(PointTable* t, uint32_t m, const uint8_t* d_twiddles, int sc
     //   n = 1024 (512 butterflies, pure latency): plain double-and-add 2.16 ms inlined / 2.69 ms compact field type;
     //            GLV joint double-and-add (127 doublings, one extra inversion per butterfly) 1.39 / 1.67 ms
     //   n = 2^20: plain 42.1 / 47.3 ms, GLV 26.6 / 31.3 ms
-    // so BN254 always runs the inlined GLV form; secp256k1 (no GLV) keeps the inlined type for few butterflies and
-    // the compact one when the machine is full.
+    // so both curves run the GLV forms on the inlined type.  secp256k1 (profiles/r04_secp_butterfly_times.txt): the compact
+    // type no longer pays off once the GLV form halves the doublings (2.720 / 5.500 ms against 2.717 / 5.396 ms inlined at
+    // 65 536 / 131 072 butterflies).
+    // Few butterflies (C::kButterflyQuadMax): four lanes per butterfly (k_butterfly_quad; PORLA_BUTTERFLY_QUAD=0 / 1 forces).
     auto* pf = reinterpret_cast<Affine<typename C::F>*>(t->d_points);
     const dim3 grid((nb + 127) / 128);
-    if constexpr (C::kGlv) {
-        // Few butterflies (at most two warps of quads per scheduler: 148 x 4 x 2 x 8 = 9472): four lanes per butterfly
-        // (k_butterfly_quad; PORLA_BUTTERFLY_QUAD=0 / 1 forces).  Measured per stage at n = 1024: see DESIGN.md section 4.
-        const char* fq = getenv("PORLA_BUTTERFLY_QUAD");
-        if (fq ? fq[0] == '1' : nb <= 9472u)
-            k_butterfly_quad<C><<<(nb * 4 + kBflyQuadThreads - 1) / kBflyQuadThreads, kBflyQuadThreads, 0, stream>>>(pf, t->d_flags, t->n, m, d_twiddles, scalar_be);
-        else
-            k_butterfly<C, typename C::F><<<grid, 128, 0, stream>>>(pf, t->d_flags, t->n, m, d_twiddles, scalar_be);
-    } else if (nb < 148u * 512u) {
-        k_butterfly<C, typename C::F><<<grid, 128, 0, stream>>>(pf, t->d_flags, t->n, m, d_twiddles, scalar_be);
+    const char* fq = getenv("PORLA_BUTTERFLY_QUAD");
+    if (fq ? fq[0] == '1' : nb <= C::kButterflyQuadMax) {
+        k_butterfly_quad<C><<<(nb * 4 + kBflyQuadThreads - 1) / kBflyQuadThreads, kBflyQuadThreads, 0, stream>>>(pf, t->d_flags, t->n, m, d_twiddles, scalar_be);
     } else {
-        auto* pc = reinterpret_cast<Affine<typename C::FC>*>(t->d_points);
-        k_butterfly<C, typename C::FC><<<grid, 128, 0, stream>>>(pc, t->d_flags, t->n, m, d_twiddles, scalar_be);
+        k_butterfly<C, typename C::F><<<grid, 128, 0, stream>>>(pf, t->d_flags, t->n, m, d_twiddles, scalar_be);
     }
     LAUNCHED();
     if constexpr (C::kGlv) {

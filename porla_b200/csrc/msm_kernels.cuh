@@ -104,27 +104,7 @@ PORLA_D void reduce_scalar(uint32_t* s) {
     }
 }
 
-// ---------------------------------------------------------------------------- GLV scalar split (BN254)
-// out = a * b mod 2^(32*NO) on 32-bit limbs (schoolbook; a few dozen IMADs per scalar)
-template <int NA, int NB, int NO>
-PORLA_D void mul_limbs(const uint32_t* a, const uint32_t* b, uint32_t* out) {
-#pragma unroll
-    for (int i = 0; i < NO; i++) out[i] = 0;
-#pragma unroll
-    for (int i = 0; i < NA; i++) {
-        uint64_t carry = 0;
-#pragma unroll
-        for (int j = 0; j < NB; j++) {
-            if (i + j < NO) {
-                uint64_t v = (uint64_t)a[i] * b[j] + out[i + j] + carry;
-                out[i + j] = (uint32_t)v;
-                carry = v >> 32;
-            }
-        }
-        if (i + NB < NO) out[i + NB] = (uint32_t)carry;
-    }
-}
-
+// ---------------------------------------------------------------------------- GLV scalar split
 // k (reduced mod r) -> |k1|, |k2| < 2^127 and their signs, k = k1 + k2 * lambda (mod r).
 //   c1 = floor(k * g1 / 2^256) ~ k b2 / r,  c2 = floor(k * g2 / 2^256) ~ -k b1 / r
 //   k1 = k - c1 a1 - c2 a2,  k2 = -c1 b1 - c2 b2        (exact, evaluated mod 2^192 in two's complement)
@@ -184,6 +164,12 @@ PORLA_D void glv_split(const uint32_t* k, uint32_t* k1, uint32_t* k2, uint32_t& 
         k1[i] = v1[i];
         k2[i] = v2[i];
     }
+}
+
+// secp256k1: its own routine (rounded c1, c2 and its limb sizes: ec.cuh), shared with the host butterfly
+template <>
+PORLA_D void glv_split<Secp256k1>(const uint32_t* k, uint32_t* k1, uint32_t* k2, uint32_t& neg1, uint32_t& neg2) {
+    glv_split_secp256k1(k, k1, k2, neg1, neg2);
 }
 
 // ---------------------------------------------------------------------------- scalar preparation
@@ -306,6 +292,36 @@ __global__ void k_import_points(const uint8_t* __restrict__ in, int fmt, int mas
     st16(out + i, p);
     if (flags) flags[i] = inf ? 1 : 0;
     if (inf && inf_count) atomicAdd(inf_count, 1u);
+}
+
+// Jacobian points (IPA-mode MACs, secp256k1_gej) -> internal affine records and their flags: x = X / Z^2, y = Y / Z^3 with
+// one inversion per point, skipped when Z = 1 (every point this library returns).  xyz: canonical X, Y, Z, 8 LE limbs
+// each; inf: the gej's infinity flag.
+template <class C>
+__global__ void __launch_bounds__(128)
+k_import_jacobian(const uint32_t* __restrict__ xyz, const uint8_t* __restrict__ inf, uint32_t n,
+                  Affine<typename C::F>* __restrict__ out, uint8_t* __restrict__ flags) {
+    using F = typename C::F;
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    F x, y, z;
+#pragma unroll
+    for (int q = 0; q < 8; q++) {
+        x.v[q] = xyz[24 * (size_t)i + q];
+        y.v[q] = xyz[24 * (size_t)i + 8 + q];
+        z.v[q] = xyz[24 * (size_t)i + 16 + q];
+    }
+    x = x.to_internal();
+    y = y.to_internal();
+    z = z.to_internal();
+    Affine<F> p = Affine<F>::inf();
+    if (!inf[i] && !z.is_zero()) {
+        const F zi = z == F::one() ? z : z.inverse(), zi2 = zi.sqr();
+        p.x = x * zi2;
+        p.y = y * zi2 * zi;
+    }
+    st16(out + i, p);
+    flags[i] = p.is_inf() ? 1 : 0;
 }
 
 // internal affine -> external bytes (inverse of the above)
@@ -1509,43 +1525,35 @@ k_butterfly(Affine<F>* __restrict__ pts, uint8_t* __restrict__ flags, uint32_t n
     reduce_scalar<C>(s);
     const Affine<F> a0 = ld16(pts + k), a1 = ld16(pts + k + m2);
     XYZZ<F> t = XYZZ<F>::inf();
-    if constexpr (C::kGlv) {
-        // w = k1 + k2 lambda: joint double-and-add over (P, phi(P), P + phi(P)), 127 doublings instead of 254.
-        // Every lane of the warp adds an AFFINE operand chosen by its two bits (infinity for 00), so the warp
-        // executes one doubling and one mixed addition per bit whatever the lanes' digits are.
-        if (!a1.is_inf()) {
-            uint32_t k1[4], k2[4], n1, n2;
-            glv_split<C>(s, k1, k2, n1, n2);
-            Affine<F> tab[3];
-            tab[0] = a1;
-            if (n1) tab[0].y = tab[0].y.neg();
-            F beta;
+    // w = k1 + k2 lambda: joint double-and-add over (P, phi(P), P + phi(P)), 127 (BN254) or 128 (secp256k1) doublings
+    // instead of 254 or 256.
+    // Every lane of the warp adds an AFFINE operand chosen by its two bits (infinity for 00), so the warp
+    // executes one doubling and one mixed addition per bit whatever the lanes' digits are.
+    if (!a1.is_inf()) {
+        uint32_t k1[4], k2[4], n1, n2;
+        glv_split<C>(s, k1, k2, n1, n2);
+        Affine<F> tab[3];
+        tab[0] = a1;
+        if (n1) tab[0].y = tab[0].y.neg();
+        F beta;
 #pragma unroll
-            for (int q = 0; q < 8; q++) beta.v[q] = C::glv_beta_mont(q);
-            tab[1].x = a1.x * beta;
-            tab[1].y = n2 ? a1.y.neg() : a1.y;
-            XYZZ<F> both = XYZZ<F>::from_affine(tab[0]);
-            both.madd(tab[1]);
-            tab[2] = both.to_affine();          // (+-1 +- lambda) P is never infinity: lambda != +-1
-            int top = 127;
-            while (top >= 0 && !(((k1[top >> 5] | k2[top >> 5]) >> (top & 31)) & 1u)) top--;
+        for (int q = 0; q < 8; q++) beta.v[q] = C::glv_beta_mont(q);
+        tab[1].x = a1.x * beta;
+        tab[1].y = n2 ? a1.y.neg() : a1.y;
+        XYZZ<F> both = XYZZ<F>::from_affine(tab[0]);
+        both.madd(tab[1]);
+        tab[2] = both.to_affine();          // (+-1 +- lambda) P is never infinity: lambda != +-1
+        int top = 127;
+        while (top >= 0 && !(((k1[top >> 5] | k2[top >> 5]) >> (top & 31)) & 1u)) top--;
 #pragma unroll 1
-            for (int i = top; i >= 0; i--) {
-                t = t.dbl();
-                const uint32_t b = ((k1[i >> 5] >> (i & 31)) & 1u) | (((k2[i >> 5] >> (i & 31)) & 1u) << 1);
-                Affine<F> q = Affine<F>::inf();
-                if (b == 1) q = tab[0];
-                else if (b == 2) q = tab[1];
-                else if (b == 3) q = tab[2];
-                t.madd(q);
-            }
-        }
-    } else if (!a1.is_inf()) {
-        int top = 255;
-        while (top >= 0 && !((s[top >> 5] >> (top & 31)) & 1u)) top--;
         for (int i = top; i >= 0; i--) {
             t = t.dbl();
-            if ((s[i >> 5] >> (i & 31)) & 1u) t.madd(a1);
+            const uint32_t b = ((k1[i >> 5] >> (i & 31)) & 1u) | (((k2[i >> 5] >> (i & 31)) & 1u) << 1);
+            Affine<F> q = Affine<F>::inf();
+            if (b == 1) q = tab[0];
+            else if (b == 2) q = tab[1];
+            else if (b == 3) q = tab[2];
+            t.madd(q);
         }
     }
     XYZZ<F> r0 = t, r1 = t.neg();
@@ -1574,7 +1582,7 @@ k_butterfly(Affine<F>* __restrict__ pts, uint8_t* __restrict__ flags, uint32_t n
 }
 
 // The same stage with FOUR lanes per butterfly (quad.cuh), for stages of few butterflies where the 127 dependent doublings and
-// additions are pure latency (Porla's rebuild of 1024 blocks: 512 butterflies per stage on a 148-SM part).  BN254 / GLV only.
+// additions are pure latency (Porla's rebuild of 1024 blocks: 512 butterflies per stage on a 148-SM part).
 // Differences from k_butterfly besides the lane layout:
 //   - joint 2-bit windows over the halves of w = k1 + k2 lambda: a table of the 15 combinations d1 (+-P) + d2 (+-phi(P)),
 //     0 <= d1, d2 <= 3, kept in shared memory in XYZZ form (the four-lane addition takes general operands, so nothing is

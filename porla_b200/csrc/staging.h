@@ -10,6 +10,9 @@
 #include <stddef.h>
 #include <stdint.h>
 
+#include <functional>
+#include <mutex>
+
 #include "msm.h"
 
 namespace porla {
@@ -63,6 +66,15 @@ bool host_pointer_is_pinned(const void* p);
 // sources; for pinned sources the usual stream ordering applies (every caller in this library synchronises the
 // stream before it returns to the user, which covers both).
 void h2d_copy(void* d_dst, const void* h_src, size_t bytes, cudaStream_t stream);
+
+// The staging of the default device for the large host-buffer calls (abi.cu, abi_secp.cu) and the mutex that serialises it.
+extern std::mutex g_io_mu;
+extern Staging g_stage;
+
+// Host-buffer butterfly stages (bn254_butterfly_stage, porla_secp256k1_butterfly_stage): the largest stage, in butterflies,
+// that runs on the calling host, and the split of a stage's nb butterflies over host threads (body(lo, hi) per thread).
+int64_t host_butterfly_limit(int curve);
+void for_each_butterfly_host(int64_t nb, const std::function<void(int64_t, int64_t)>& body);
 
 // Statistics of the copy pool (test / bench hook): bytes moved through the pinned ring so far.
 uint64_t h2d_ring_bytes();

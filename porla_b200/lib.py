@@ -35,6 +35,7 @@ NEW_SYMBOLS = [
     "porla_butterfly_stage_device", "bn254_butterfly_stage", "bn254_align_mac_batch", "bn254_audit_aggregate", "porla_data_butterfly_stage", "porla_data_butterfly_stage_device",
     "porla_msm_table_host_scalars", "porla_msm_table_host_scalars_batch", "porla_secp256k1_table_create", "porla_secp256k1_ecmult_multi_table",
     "porla_debug_pairing_selfcheck", "porla_debug_latency", "porla_secp256k1_inner_product_prove", "porla_secp256k1_inner_product_verify",
+    "porla_secp256k1_butterfly_stage",
     "porla_device_count", "porla_mtable_create", "porla_mtable_devices", "porla_mtable_len", "porla_mtable_range",
     "porla_mtable_msm_host_scalars", "porla_mtable_msm_resident", "porla_mtable_scalars_upload", "porla_mtable_scalars_free",
     "porla_mtable_destroy", "porla_debug_copy_ring_bytes", "porla_msm_host_devices", "porla_debug_h2d_rate",
@@ -135,6 +136,7 @@ def load() -> C.CDLL:
         "porla_debug_pairing_selfcheck": (I, [I]),
         "porla_secp256k1_inner_product_prove": (C.c_size_t, [P, C.c_size_t, C.c_char_p, C.c_char_p, C.c_char_p]),
         "porla_secp256k1_inner_product_verify": (I, [P, C.c_size_t, C.POINTER(SecpGej), C.c_char_p]),
+        "porla_secp256k1_butterfly_stage": (I, [C.POINTER(SecpGej), C.c_size_t, C.c_size_t, C.POINTER(SecpScalar)]),
         "porla_debug_latency": (I, [I, I, I, I, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
         "porla_debug_quad_op": (None, [I, I, P, P, C.c_int64, I, P]),
         "porla_debug_field_mul": (None, [I, P, P, C.c_int64, P]),
@@ -518,6 +520,17 @@ class SecpGenerators:
         if self.handle:
             load().porla_table_destroy(C.c_void_p(self.handle))
             self.handle = 0
+
+
+def secp256k1_butterfly_stage(gejs, m: int, twiddles: Sequence[int]) -> int:
+    """One stage of the FFT in the exponent on IPA-mode MACs, in place on `gejs` (a ctypes array of SecpGej: any z, any
+    field magnitude).  twiddles: m/2 integers below 2^256, taken mod n.  Returns the C entry's result (0: m is not a power
+    of two >= 2 dividing len(gejs), buffer untouched)."""
+    tw = (SecpScalar * max(1, len(twiddles)))()
+    for k, w in enumerate(twiddles):
+        for i in range(4):
+            tw[k].d[i] = (w >> (64 * i)) & 0xFFFFFFFFFFFFFFFF
+    return load().porla_secp256k1_butterfly_stage(gejs, len(gejs), m, tw)
 
 
 def secp256k1_ecmult_multi_var(scalars: Sequence[int], points: Sequence, g_scalar: Optional[int] = None):
