@@ -298,6 +298,32 @@ int porla_secp256k1_inner_product_verify(const porla_table* gens_and_u, size_t n
  * power of two >= 2 dividing n, else 1.  Stages of at most PORLA_HOST_BUTTERFLIES butterflies (default 32) run on the
  * calling host without touching the device; larger ones on the GPU (k_butterfly_quad / k_butterfly). */
 int porla_secp256k1_butterfly_stage(porla_secp256k1_gej* points, size_t n, size_t m, const porla_secp256k1_scalar* twiddles);
+/* Server::align_MAC, IPA branch (Server.hpp:481-518; SURVEY 8(f)2), for `batch` blocks of n_chunks chunks -- 64-byte
+ * little-endian integers below LCM = PRIME_MODULUS * n (utils.h:32) -- in ONE launch sequence:
+ *       mod = A[i] % PRIME_MODULUS;   c[i] = (mod - A[i]) % n;   A[i] = mod;   align_out[b] = sum_i c[i] * gens[i]
+ * `data` is updated in place (upper 32 bytes of every chunk become zero).  gens: any secp256k1 table with at least
+ * n_chunks entries (porla_secp256k1_table_create; entries [0, n_chunks) are used, so the prover's generators-then-u table
+ * serves as it is).  Results: z = 1, normalised limbs.  Returns 0 (buffers untouched) for a bad shape -- NULL or
+ * non-secp256k1 table, n_chunks 0 or longer than the table, batch * n_chunks >= 2^31 -- else 1; batch == 0 does not touch
+ * the device.  Calls of a few blocks lease a staging slot of their own, so Porla's pool threads (Server.hpp:1077-1078)
+ * overlap on the device. */
+int porla_secp256k1_align_mac_batch(const porla_table* gens, size_t n_chunks, void* data, size_t batch,
+                                    porla_secp256k1_gej* align_out);
+/* Server::audit's aggregation and its alignment, IPA branch (Server.hpp:790-828 then align_MAC; SURVEY 8(f)4):
+ *       B[j] = sum_i coefs[i] * blocks[i][j]     plain integers (31-bit coefs, n x n_chunks chunks of 64 bytes LE)
+ *       b_out[j] = B[j] % PRIME_MODULUS;   align_out = sum_j ((B[j] % PRIME_MODULUS - B[j]) % n) * gens[j]
+ * b_out_le32: n_chunks x 32 bytes little-endian (the convert_ZZ_to_arr layout porla_secp256k1_inner_product_prove reads).
+ * Returns 0 (buffers untouched) for a bad table / n_chunks as above or n >= 2^24 blocks, else 1; n == 0 gives B = 0 and an
+ * infinity alignment without touching the device.  One aggregation kernel and one look-up-table commitment. */
+int porla_secp256k1_audit_aggregate(const porla_table* gens, size_t n_chunks, const uint32_t* coefs, const void* blocks,
+                                    size_t n, unsigned char* b_out_le32, porla_secp256k1_gej* align_out);
+/* r[b] = sum_i scalars[b n + i] * points[b n + i] for b < nbatch on the MACs as stored (the audit's combined_MAC /
+ * combined_align, Client::audit): points are secp256k1_gej with any z and field magnitude, infinity flag honoured;
+ * scalars are taken mod n.  No host inversion: each point with z != 1 costs one inversion on the device.  Results:
+ * z = 1, normalised limbs, the same as porla_secp256k1_ecmult_multi_var on the same points as secp256k1_ge.  n * nbatch
+ * == 0 sets every r[b] to infinity without touching the device; n * nbatch >= 2^31 returns 0, otherwise 1. */
+int porla_secp256k1_ecmult_multi_gej(const porla_secp256k1_gej* points, const porla_secp256k1_scalar* scalars, size_t n,
+                                     size_t nbatch, porla_secp256k1_gej* r);
 /* 33-byte SEC1 compressed form of a gej/ge result (eckey_impl.h:36-52); returns 0 for infinity. */
 int porla_secp256k1_gej_serialize(const porla_secp256k1_gej* a, unsigned char out33[33]);
 

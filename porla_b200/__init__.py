@@ -34,5 +34,6 @@ from .lib import (  # noqa: F401
     msm_host_devices,
     secp256k1_ecmult_multi_var,
     secp256k1_butterfly_stage,
+    secp256k1_ecmult_multi_gej,
     SecpGenerators,
 )

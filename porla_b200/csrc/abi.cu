@@ -21,10 +21,6 @@
 using namespace porla;
 using namespace porla::host;
 
-struct porla_table {
-    PointTable t;
-};
-
 namespace {
 
 // ---------------------------------------------------------------------------- process state
@@ -446,6 +442,113 @@ void client_fixed_base(const ClientBase& b, const uint8_t* d_scalars, int scalar
 
 }  // namespace
 
+namespace porla {
+
+PointTable table_window(const PointTable& t, int64_t first, int64_t n) {
+    PointTable view = t;
+    view.d_points = (uint8_t*)t.d_points + (size_t)first * 64;
+    view.d_flags = t.d_flags ? t.d_flags + first : nullptr;
+    view.n = (uint32_t)n;
+    if (t.d_phi_x) {                           // image of entry first + i: same index arithmetic on the beta*x array
+        view.d_phi_x = (uint8_t*)t.d_phi_x + (size_t)first * 32;
+        view.phi_off = (uint32_t)n;
+    }
+    if (t.fb_c > 0) {                          // the expansion's rows keep their stride; start them at `first`
+        view.d_fb_points = (uint8_t*)t.d_fb_points + (size_t)first * 64;
+        if (t.d_lut) view.d_lut = (uint8_t*)t.d_lut + ((((size_t)first * t.fb_nwin) << (t.fb_c - 1)) * 64);
+    }
+    return view;
+}
+
+void align_mac_core(int curve, const PointTable& gens, void* data, int64_t n, int64_t batch, int out_fmt, uint8_t* out) {
+    if (batch == 0) return;
+    device_init();
+    StageLease lease = lease_stage(n, batch);
+    Staging& sg = *lease.s;
+    const size_t total = (size_t)batch * n;
+    auto pad = [](size_t v) { return (v + 255) & ~(size_t)255; };
+    const size_t sc_off = pad(total * 64), out_off = sc_off + pad(total * 32),
+                 scr_off = out_off + pad(result_scratch_bytes(curve, n, batch));
+    uint8_t* d = sg.dev(scr_off + (lease.local() ? kSlotScratch : 0));
+    cudaStream_t st = sg.stream;
+    h2d_copy(d, data, total * 64, st);
+    align_scalars_device(curve, reinterpret_cast<uint32_t*>(d), (uint32_t)total, d + sc_off, st);
+    PORLA_CUDA(cudaMemcpyAsync(data, d, total * 64, cudaMemcpyDeviceToHost, st));   // A[i] <- A[i] % PRIME_MODULUS
+    MsmOptions opt;
+    opt.scalar_be = 1;
+    opt.out_fmt = out_fmt;
+    opt.shared_points = 1;
+    if (lease.local()) {
+        opt.d_scratch = d + scr_off;
+        opt.scratch_bytes = kSlotScratch;
+    }
+    run_and_fetch(curve, gens, d + sc_off, n, batch, opt, d + out_off, out, st, sg);
+}
+
+void audit_aggregate_core(int curve, const PointTable& gens, const void* coefs, const void* blocks, int64_t n, int64_t chunks,
+                          int out_fmt, uint8_t* b_mod_be, uint8_t* out64) {
+    device_init();
+    // the blocks are the call's volume: a slot is leased when they are no more than a small MSM's terms
+    StageLease lease = lease_stage((n > 0 ? n : 1) * chunks, 1);
+    Staging& sg = *lease.s;
+    auto pad = [](size_t v) { return (v + 255) & ~(size_t)255; };
+    const size_t blk_bytes = (size_t)n * chunks * 64;
+    const size_t cf_off = pad(blk_bytes), b_off = cf_off + pad((size_t)n * 4 + 4), c_off = b_off + pad((size_t)chunks * 32),
+                 out_off = c_off + pad((size_t)chunks * 32), scr_off = out_off + pad(result_scratch_bytes(curve, chunks, 1));
+    uint8_t* d = sg.dev(scr_off + (lease.local() ? kSlotScratch : 0));
+    cudaStream_t st = sg.stream;
+    if (n) {
+        h2d_copy(d, blocks, blk_bytes, st);
+        PORLA_CUDA(cudaMemcpyAsync(d + cf_off, coefs, (size_t)n * 4, cudaMemcpyHostToDevice, st));
+    }
+    audit_aggregate_device(curve, reinterpret_cast<const uint32_t*>(d + cf_off), reinterpret_cast<const uint32_t*>(d), (uint32_t)n,
+                           (uint32_t)chunks, d + b_off, d + c_off, st);
+    PORLA_CUDA(cudaMemcpyAsync(b_mod_be, d + b_off, (size_t)chunks * 32, cudaMemcpyDeviceToHost, st));
+    MsmOptions opt;
+    opt.scalar_be = 1;
+    opt.out_fmt = out_fmt;
+    opt.shared_points = 1;
+    if (lease.local()) {
+        opt.d_scratch = d + scr_off;
+        opt.scratch_bytes = kSlotScratch;
+    }
+    run_and_fetch(curve, gens, d + c_off, chunks, 1, opt, d + out_off, out64, st, sg);
+}
+
+void msm_host_jacobian_secp256k1(const uint32_t* xyz, const uint8_t* inf, const void* scalars, int64_t n, int64_t nbatch,
+                                 uint8_t* out) {
+    check_shape(n, nbatch, "secp256k1 Jacobian MSM");
+    device_init();
+    StageLease lease = lease_stage(n, nbatch);
+    Staging& sg = *lease.s;
+    const size_t total = (size_t)n * nbatch;
+    // staging layout: scalars | X, Y, Z | infinity flags in | affine table | its flags | result scratch | small-path scratch
+    auto pad = [](size_t v) { return (v + 255) & ~(size_t)255; };
+    const size_t xyz_off = pad(total * 32), inf_off = xyz_off + pad(total * 96), tab_off = inf_off + pad(total),
+                 fl_off = tab_off + pad(total * 64), out_off = fl_off + pad(total),
+                 scr_off = out_off + pad(result_scratch_bytes(kCurveSecp256k1, n, nbatch));
+    uint8_t* d = sg.dev(scr_off + (lease.local() ? kSlotScratch : 0));
+    cudaStream_t st = sg.stream;
+    h2d_copy(d, scalars, total * 32, st);
+    h2d_copy(d + xyz_off, xyz, total * 96, st);
+    h2d_copy(d + inf_off, inf, total, st);
+    MsmOptions opt;
+    opt.scalar_be = 0;
+    opt.out_fmt = PORLA_POINT_LE64;
+    opt.shared_points = 0;
+    if (lease.local()) {
+        opt.d_scratch = d + scr_off;
+        opt.scratch_bytes = kSlotScratch;
+    }
+    if (total <= 4096) opt.max_scalar_bits = host_max_scalar_bits(kCurveSecp256k1, (const uint8_t*)scalars, total, 0);
+    PointTable tab;
+    table_import_jacobian_secp256k1(reinterpret_cast<const uint32_t*>(d + xyz_off), d + inf_off, (uint32_t)total, d + tab_off,
+                                    d + fl_off, &tab, st);
+    run_and_fetch(kCurveSecp256k1, tab, d, n, nbatch, opt, d + out_off, out, st, sg);
+}
+
+}  // namespace porla
+
 extern "C" {
 
 // ============================================================================ legacy cgo ABI
@@ -824,18 +927,7 @@ void porla_msm_table_host_scalars_batch(const porla_table* t, int64_t first, con
     uint8_t* d = sg.dev(scr_off + (lease.local() ? kSlotScratch : 0));
     cudaStream_t st = sg.stream;
     h2d_copy(d, scalars, sc_bytes, st);
-    PointTable view = t->t;                       // a window [first, first + n) of the resident table
-    view.d_points = (uint8_t*)t->t.d_points + (size_t)first * 64;
-    view.d_flags = t->t.d_flags ? t->t.d_flags + first : nullptr;
-    view.n = (uint32_t)n;
-    if (t->t.d_phi_x) {                           // image of entry first + i: same index arithmetic on the beta*x array
-        view.d_phi_x = (uint8_t*)t->t.d_phi_x + (size_t)first * 32;
-        view.phi_off = (uint32_t)n;
-    }
-    if (t->t.fb_c > 0) {                          // the expansion's rows keep their stride; start them at `first`
-        view.d_fb_points = (uint8_t*)t->t.d_fb_points + (size_t)first * 64;
-        if (t->t.d_lut) view.d_lut = (uint8_t*)t->t.d_lut + ((((size_t)first * t->t.fb_nwin) << (t->t.fb_c - 1)) * 64);
-    }
+    const PointTable view = table_window(t->t, first, n);
     MsmOptions opt;
     opt.scalar_be = scalar_fmt == PORLA_SCALAR_BE32;
     opt.out_fmt = out_fmt;
@@ -928,22 +1020,7 @@ void bn254_align_mac_batch(GoSlice* data, GoInt batch, GoSlice* align_out) {
     device_init();
     std::shared_lock<std::shared_mutex> srs = srs_reader(n, 0, batch);   // also refuses n_samples above the SRS length
     std::vector<uint8_t> res((size_t)batch * 64);
-    {
-        std::lock_guard<std::mutex> lock(g_io_mu);
-        const size_t total = (size_t)batch * n;
-        auto pad = [](size_t v) { return (v + 255) & ~(size_t)255; };
-        size_t sc_off = pad(total * 64), out_off = sc_off + pad(total * 32);
-        uint8_t* d = g_stage.dev(out_off + result_scratch_bytes(kCurveBn254, n, batch));
-        cudaStream_t st = g_stage.stream;
-        h2d_copy(d, data->data, total * 64, st);
-        align_scalars_device(reinterpret_cast<uint32_t*>(d), (uint32_t)total, d + sc_off, st);
-        PORLA_CUDA(cudaMemcpyAsync(data->data, d, total * 64, cudaMemcpyDeviceToHost, st));   // A[i] <- A[i] % PRIME_MODULUS
-        MsmOptions opt;
-        opt.scalar_be = 1;
-        opt.out_fmt = PORLA_POINT_BE64;
-        opt.shared_points = 1;
-        run_and_fetch(kCurveBn254, g_kzg.srs_table, d + sc_off, n, batch, opt, d + out_off, res.data(), st);
-    }
+    align_mac_core(kCurveBn254, g_kzg.srs_table, data->data, n, batch, PORLA_POINT_BE64, res.data());
     go_copy(align_out, res.data(), res.size());
 }
 
@@ -955,27 +1032,8 @@ void bn254_audit_aggregate(GoSlice* coefs, GoSlice* blocks, GoInt n, GoSlice* b_
     device_init();
     std::shared_lock<std::shared_mutex> srs = srs_reader(chunks, 0, 1);   // also refuses n_samples above the SRS length
     std::vector<uint8_t> b_mod((size_t)chunks * 32), res(64);
-    {
-        std::lock_guard<std::mutex> lock(g_io_mu);
-        auto pad = [](size_t v) { return (v + 255) & ~(size_t)255; };
-        const size_t blk_bytes = (size_t)n * chunks * 64;
-        size_t cf_off = pad(blk_bytes), b_off = cf_off + pad((size_t)n * 4 + 4), c_off = b_off + pad((size_t)chunks * 32),
-               out_off = c_off + pad((size_t)chunks * 32);
-        uint8_t* d = g_stage.dev(out_off + result_scratch_bytes(kCurveBn254, chunks, 1));
-        cudaStream_t st = g_stage.stream;
-        if (n) {
-            h2d_copy(d, blocks->data, blk_bytes, st);
-            PORLA_CUDA(cudaMemcpyAsync(d + cf_off, coefs->data, (size_t)n * 4, cudaMemcpyHostToDevice, st));
-        }
-        audit_aggregate_device(reinterpret_cast<const uint32_t*>(d + cf_off), reinterpret_cast<const uint32_t*>(d), (uint32_t)n,
-                               (uint32_t)chunks, d + b_off, d + c_off, st);
-        PORLA_CUDA(cudaMemcpyAsync(b_mod.data(), d + b_off, b_mod.size(), cudaMemcpyDeviceToHost, st));
-        MsmOptions opt;
-        opt.scalar_be = 1;
-        opt.out_fmt = PORLA_POINT_BE64;
-        opt.shared_points = 1;
-        run_and_fetch(kCurveBn254, g_kzg.srs_table, d + c_off, chunks, 1, opt, d + out_off, res.data(), st);
-    }
+    audit_aggregate_core(kCurveBn254, g_kzg.srs_table, coefs->data, blocks->data, n, chunks, PORLA_POINT_BE64, b_mod.data(),
+                         res.data());
     go_copy(b_out, b_mod.data(), b_mod.size());
     go_copy(align_out, res.data(), res.size());
 }

@@ -376,18 +376,26 @@ void butterfly_stage_host(porla_secp256k1_gej* pts, size_t n, size_t m, const po
     });
 }
 
+// gej as stored -> what k_import_jacobian reads: canonical X, Y, Z (8 LE 32-bit limbs each, zero for infinity) and the
+// infinity flags.  The limbs are normalised here; the Jacobian -> affine conversion happens on the device.
+void gej_to_device_form(const porla_secp256k1_gej* pts, size_t n, std::vector<uint32_t>* xyz, std::vector<uint8_t>* inf) {
+    xyz->assign(24 * n, 0);
+    inf->resize(n);
+    for (size_t i = 0; i < n; i++) {
+        (*inf)[i] = pts[i].infinity ? 1 : 0;
+        if ((*inf)[i]) continue;
+        fe_to_canonical(&pts[i].x, &(*xyz)[24 * i]);
+        fe_to_canonical(&pts[i].y, &(*xyz)[24 * i + 8]);
+        fe_to_canonical(&pts[i].z, &(*xyz)[24 * i + 16]);
+    }
+}
+
 // The same stage on the device: limbs normalised here, Jacobian -> affine in k_import_jacobian, the butterfly kernels of
 // butterfly_stage_device, canonical affine back.
 void butterfly_stage_gpu(porla_secp256k1_gej* pts, size_t n, size_t m, const porla_secp256k1_scalar* tw) {
-    std::vector<uint32_t> xyz(24 * n, 0);
-    std::vector<uint8_t> inf(n);
-    for (size_t i = 0; i < n; i++) {
-        inf[i] = pts[i].infinity ? 1 : 0;
-        if (inf[i]) continue;
-        fe_to_canonical(&pts[i].x, &xyz[24 * i]);
-        fe_to_canonical(&pts[i].y, &xyz[24 * i + 8]);
-        fe_to_canonical(&pts[i].z, &xyz[24 * i + 16]);
-    }
+    std::vector<uint32_t> xyz;
+    std::vector<uint8_t> inf;
+    gej_to_device_form(pts, n, &xyz, &inf);
     device_init();
     std::lock_guard<std::mutex> lock(g_io_mu);
     g_stage.init();
@@ -407,6 +415,12 @@ void butterfly_stage_gpu(porla_secp256k1_gej* pts, size_t n, size_t m, const por
     PORLA_CUDA(cudaMemcpyAsync(out.data(), d + o_out, 64 * n, cudaMemcpyDeviceToHost, st));
     PORLA_CUDA(cudaStreamSynchronize(st));
     for (size_t i = 0; i < n; i++) gej_from_le64(out.data() + 64 * i, pts + i);
+}
+
+// A resident secp256k1 table holding at least n_chunks generators; a staged call indexes terms with 32 bits
+bool align_shape_ok(const porla_table* gens, size_t n_chunks, size_t batch) {
+    return gens && gens->t.curve == kCurveSecp256k1 && n_chunks && n_chunks <= gens->t.n &&
+           (uint64_t)n_chunks * batch < (1ull << 31);
 }
 }  // namespace
 
@@ -486,6 +500,58 @@ int porla_secp256k1_ecmult_multi_table(const porla_table* t, size_t first, const
     uint8_t res[64];
     porla_msm_table_host_scalars(t, (int64_t)first, scalars, (int64_t)n, PORLA_SCALAR_LE32, PORLA_POINT_LE64, res);
     gej_from_le64(res, r);
+    return 1;
+}
+
+// ---- the data side of an IPA-mode server (SURVEY 8(f)2 and (f)4): align_MAC and the audit's aggregation over the resident
+// generators, on the kernels and staging of their KZG twins (align_mac_core, audit_aggregate_core), with secp256k1's n as
+// GROUP_ORDER (utils.h:32).
+int porla_secp256k1_align_mac_batch(const porla_table* gens, size_t n_chunks, void* data, size_t batch,
+                                    porla_secp256k1_gej* align_out) {
+    if (!align_shape_ok(gens, n_chunks, batch)) return 0;
+    if (batch == 0) return 1;
+    std::vector<uint8_t> res(64 * batch);
+    align_mac_core(kCurveSecp256k1, table_window(gens->t, 0, (int64_t)n_chunks), data, (int64_t)n_chunks, (int64_t)batch,
+                   PORLA_POINT_LE64, res.data());
+    for (size_t b = 0; b < batch; b++) gej_from_le64(res.data() + 64 * b, align_out + b);
+    return 1;
+}
+
+int porla_secp256k1_audit_aggregate(const porla_table* gens, size_t n_chunks, const uint32_t* coefs, const void* blocks,
+                                    size_t n, unsigned char* b_out_le32, porla_secp256k1_gej* align_out) {
+    if (!align_shape_ok(gens, n_chunks, 1) || n >= (1u << 24)) return 0;
+    if (n == 0) {   // B = 0: already reduced, nothing to align
+        memset(b_out_le32, 0, 32 * n_chunks);
+        gej_set_infinity(align_out);
+        return 1;
+    }
+    std::vector<uint8_t> b_be(32 * n_chunks);
+    uint8_t res[64];
+    audit_aggregate_core(kCurveSecp256k1, table_window(gens->t, 0, (int64_t)n_chunks), coefs, blocks, (int64_t)n,
+                         (int64_t)n_chunks, PORLA_POINT_LE64, b_be.data(), res);
+    for (size_t j = 0; j < n_chunks; j++)   // convert_ZZ_to_arr's order: least significant byte first
+        for (int k = 0; k < 32; k++) b_out_le32[32 * j + k] = b_be[32 * j + 31 - k];
+    gej_from_le64(res, align_out);
+    return 1;
+}
+
+// The audit's combined_MAC / combined_align and Client::audit on the MACs as stored: the drop-in above needs
+// secp256k1_ge, i.e. one host inversion per MAC first (SURVEY App. E); here the Jacobian points go to the device as they
+// are (the butterfly stage's route: limbs normalised here, one device inversion per point with z != 1).
+int porla_secp256k1_ecmult_multi_gej(const porla_secp256k1_gej* points, const porla_secp256k1_scalar* scalars, size_t n,
+                                     size_t nbatch, porla_secp256k1_gej* r) {
+    if (nbatch && n >= (1ull << 31) / nbatch) return 0;
+    if (n == 0) {
+        for (size_t b = 0; b < nbatch; b++) gej_set_infinity(r + b);
+        return 1;
+    }
+    if (nbatch == 0) return 1;
+    std::vector<uint32_t> xyz;
+    std::vector<uint8_t> inf;
+    gej_to_device_form(points, n * nbatch, &xyz, &inf);
+    std::vector<uint8_t> res(64 * nbatch);
+    msm_host_jacobian_secp256k1(xyz.data(), inf.data(), scalars, (int64_t)n, (int64_t)nbatch, res.data());
+    for (size_t b = 0; b < nbatch; b++) gej_from_le64(res.data() + 64 * b, r + b);
     return 1;
 }
 

@@ -25,7 +25,7 @@
 #include "msm_kernels.cuh"
 #include "quad.cuh"
 
-struct porla_table {   // as in abi.cu
+struct porla_table {   // as in staging.h
     porla::PointTable t;
 };
 

@@ -470,15 +470,15 @@ void butterfly_stage_device(PointTable* t, uint32_t m, const uint8_t* d_twiddles
     DISPATCH(t->curve, butterfly_impl, t, m, d_twiddles, scalar_be, stream);
 }
 
-void align_scalars_device(uint32_t* d_data, uint32_t total, uint8_t* d_scalars_be, cudaStream_t stream) {
+void align_scalars_device(int curve, uint32_t* d_data, uint32_t total, uint8_t* d_scalars_be, cudaStream_t stream) {
     device_init();
-    align_scalars_impl<Bn254>(d_data, total, d_scalars_be, stream);   // the reference's KZG branch only (BN254 order)
+    DISPATCH(curve, align_scalars_impl, d_data, total, d_scalars_be, stream);   // KZG mode: BN254 order, IPA mode: secp256k1's
 }
 
-void audit_aggregate_device(const uint32_t* d_coefs, const uint32_t* d_blocks, uint32_t n, uint32_t chunks, uint8_t* d_b_mod_be,
-                            uint8_t* d_c_be, cudaStream_t stream) {
+void audit_aggregate_device(int curve, const uint32_t* d_coefs, const uint32_t* d_blocks, uint32_t n, uint32_t chunks,
+                            uint8_t* d_b_mod_be, uint8_t* d_c_be, cudaStream_t stream) {
     device_init();
-    audit_aggregate_impl<Bn254>(d_coefs, d_blocks, n, chunks, d_b_mod_be, d_c_be, stream);   // KZG branch: BN254 order
+    DISPATCH(curve, audit_aggregate_impl, d_coefs, d_blocks, n, chunks, d_b_mod_be, d_c_be, stream);
 }
 
 void data_butterfly_launch(uint32_t*, uint32_t, uint32_t, uint32_t, const uint8_t*, const uint32_t*, const uint32_t*, cudaStream_t);

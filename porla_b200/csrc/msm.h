@@ -165,13 +165,14 @@ void fr_poly_eval_device(const uint8_t* d_coeffs_be, const void* d_powers, uint3
 // Invalidates the table's fixed-base expansion.
 void butterfly_stage_device(PointTable* t, uint32_t m, const uint8_t* d_twiddles, int scalar_be, cudaStream_t stream);
 // Server::align_MAC's scalar preparation for `total` chunks of 64 bytes (16 LE limbs, values below
-// PRIME_MODULUS * r): chunk <- chunk % PRIME_MODULUS in place, scalars_be[i] = (chunk % PRIME_MODULUS - chunk) % r.
-void align_scalars_device(uint32_t* d_data, uint32_t total, uint8_t* d_scalars_be, cudaStream_t stream);
+// PRIME_MODULUS * r): chunk <- chunk % PRIME_MODULUS in place, scalars_be[i] = (chunk % PRIME_MODULUS - chunk) % r,
+// r the group order of `curve` (BN254 in KZG mode, secp256k1 in IPA mode).
+void align_scalars_device(int curve, uint32_t* d_data, uint32_t total, uint8_t* d_scalars_be, cudaStream_t stream);
 // Server::audit's aggregation of `n` data blocks of `chunks` 64-byte chunks (16 LE limbs) with 31-bit coefficients,
 // followed by align_MAC's arithmetic on the sums: b_mod_be[j] = B_j % PRIME_MODULUS and
 // c_be[j] = (B_j % PRIME_MODULUS - B_j) % r as 32-byte big-endian scalars, B_j = sum_i coefs[i] * blocks[i][j].
-void audit_aggregate_device(const uint32_t* d_coefs, const uint32_t* d_blocks, uint32_t n, uint32_t chunks, uint8_t* d_b_mod_be,
-                            uint8_t* d_c_be, cudaStream_t stream);
+void audit_aggregate_device(int curve, const uint32_t* d_coefs, const uint32_t* d_blocks, uint32_t n, uint32_t chunks,
+                            uint8_t* d_b_mod_be, uint8_t* d_c_be, cudaStream_t stream);
 // One radix-2 stage of the FFT on the data blocks themselves (Server.hpp:1582-1588): n_blocks x chunks chunks of 64 bytes
 // (16 LE limbs, values below lcm), in place; twiddles: m/2 scalars of 32 bytes, little-endian; lcm_le64: the modulus
 // (utils.h:42-43), whose Barrett constant is derived on the host per call.

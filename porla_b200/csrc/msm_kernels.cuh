@@ -1701,7 +1701,8 @@ PORLA_D void mod512(const uint32_t* a, const uint32_t* m, uint32_t* rem) {
 }
 
 // One thread per chunk:  mod = A % PRIME_MODULUS;  c = (mod - A) % r;  A <- mod;  c -> 32-byte big-endian
-// scalar for the commitment.  PRIME_MODULUS = 207 * 2^248 + 1 (utils.h:40), r = BN254 group order (utils.h:37).
+// scalar for the commitment.  PRIME_MODULUS = 207 * 2^248 + 1 (utils.h:40), r = C's group order: BN254's in KZG mode
+// (utils.h:37), secp256k1's n in IPA mode (GROUP_ORDER, utils.h:32).
 template <class C>
 __global__ void __launch_bounds__(128)
 k_align_scalars(uint32_t* __restrict__ data, uint32_t total, uint8_t* __restrict__ scalars_be) {

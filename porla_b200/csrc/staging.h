@@ -71,6 +71,24 @@ void h2d_copy(void* d_dst, const void* h_src, size_t bytes, cudaStream_t stream)
 extern std::mutex g_io_mu;
 extern Staging g_stage;
 
+// A window [first, first + n) of a resident table: the same points, flags, endomorphism image and look-up rows.
+PointTable table_window(const PointTable& t, int64_t first, int64_t n);
+
+// Server::align_MAC on either curve (bn254_align_mac_batch, porla_secp256k1_align_mac_batch): `batch` blocks of n chunks
+// of 64 bytes (LE integers below PRIME_MODULUS * order) are reduced mod PRIME_MODULUS in place in `data`, and out receives
+// batch x 64 bytes (out_fmt) of sum_i c_i * gens[i], c_i = (A_i % PRIME_MODULUS - A_i) % order.  One staging area, one
+// scalar kernel, one batch of MSMs over the table's first n entries; small calls lease a staging slot.
+void align_mac_core(int curve, const PointTable& gens, void* data, int64_t n, int64_t batch, int out_fmt, uint8_t* out);
+// Server::audit's B = sum_j coefs[j] * blocks[j] over n blocks of `chunks` chunks, then align_MAC on B: b_mod_be receives
+// chunks x 32 bytes big-endian of B % PRIME_MODULUS, out64 the alignment (out_fmt).  n < 2^24.
+void audit_aggregate_core(int curve, const PointTable& gens, const void* coefs, const void* blocks, int64_t n, int64_t chunks,
+                          int out_fmt, uint8_t* b_mod_be, uint8_t* out64);
+// nbatch secp256k1 MSMs of n terms over Jacobian points: xyz holds canonical X, Y, Z (8 LE 32-bit limbs each) of the
+// n * nbatch points, inf their infinity flags, scalars n * nbatch x 8 LE 32-bit limbs; MSM m uses terms [m n, (m + 1) n).
+// One device inversion per point with Z != 1 (table_import_jacobian_secp256k1); out: nbatch x 64 bytes LE64.
+void msm_host_jacobian_secp256k1(const uint32_t* xyz, const uint8_t* inf, const void* scalars, int64_t n, int64_t nbatch,
+                                 uint8_t* out);
+
 // Host-buffer butterfly stages (bn254_butterfly_stage, porla_secp256k1_butterfly_stage): the largest stage, in butterflies,
 // that runs on the calling host, and the split of a stage's nb butterflies over host threads (body(lo, hi) per thread).
 int64_t host_butterfly_limit(int curve);
@@ -80,3 +98,8 @@ void for_each_butterfly_host(int64_t nb, const std::function<void(int64_t, int64
 uint64_t h2d_ring_bytes();
 
 }  // namespace porla
+
+// The opaque handle of include/porla_multiexp.h.
+struct porla_table {
+    porla::PointTable t;
+};

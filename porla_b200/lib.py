@@ -35,7 +35,8 @@ NEW_SYMBOLS = [
     "porla_butterfly_stage_device", "bn254_butterfly_stage", "bn254_align_mac_batch", "bn254_audit_aggregate", "porla_data_butterfly_stage", "porla_data_butterfly_stage_device",
     "porla_msm_table_host_scalars", "porla_msm_table_host_scalars_batch", "porla_secp256k1_table_create", "porla_secp256k1_ecmult_multi_table",
     "porla_debug_pairing_selfcheck", "porla_debug_latency", "porla_secp256k1_inner_product_prove", "porla_secp256k1_inner_product_verify",
-    "porla_secp256k1_butterfly_stage",
+    "porla_secp256k1_butterfly_stage", "porla_secp256k1_align_mac_batch", "porla_secp256k1_audit_aggregate",
+    "porla_secp256k1_ecmult_multi_gej",
     "porla_device_count", "porla_mtable_create", "porla_mtable_devices", "porla_mtable_len", "porla_mtable_range",
     "porla_mtable_msm_host_scalars", "porla_mtable_msm_resident", "porla_mtable_scalars_upload", "porla_mtable_scalars_free",
     "porla_mtable_destroy", "porla_debug_copy_ring_bytes", "porla_msm_host_devices", "porla_debug_h2d_rate",
@@ -137,6 +138,10 @@ def load() -> C.CDLL:
         "porla_secp256k1_inner_product_prove": (C.c_size_t, [P, C.c_size_t, C.c_char_p, C.c_char_p, C.c_char_p]),
         "porla_secp256k1_inner_product_verify": (I, [P, C.c_size_t, C.POINTER(SecpGej), C.c_char_p]),
         "porla_secp256k1_butterfly_stage": (I, [C.POINTER(SecpGej), C.c_size_t, C.c_size_t, C.POINTER(SecpScalar)]),
+        "porla_secp256k1_align_mac_batch": (I, [P, C.c_size_t, P, C.c_size_t, C.POINTER(SecpGej)]),
+        "porla_secp256k1_audit_aggregate": (I, [P, C.c_size_t, P, P, C.c_size_t, P, C.POINTER(SecpGej)]),
+        "porla_secp256k1_ecmult_multi_gej": (I, [C.POINTER(SecpGej), C.POINTER(SecpScalar), C.c_size_t, C.c_size_t,
+                                                 C.POINTER(SecpGej)]),
         "porla_debug_latency": (I, [I, I, I, I, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
         "porla_debug_quad_op": (None, [I, I, P, P, C.c_int64, I, P]),
         "porla_debug_field_mul": (None, [I, P, P, C.c_int64, P]),
@@ -497,6 +502,25 @@ class SecpGenerators:
             return ok, None
         return ok, (_fe_to_int(r.x), _fe_to_int(r.y))
 
+    def align_mac_batch(self, data: bytearray, batch: int, n_chunks: int):
+        """Server::align_MAC, IPA branch, for `batch` blocks of n_chunks chunks over generators [0, n_chunks): data =
+        batch*n_chunks*64 bytes of LE values below PRIME_MODULUS*n, reduced mod PRIME_MODULUS in place.  Returns (the C
+        entry's result, a ctypes array of `batch` SecpGej alignments)."""
+        out = (SecpGej * max(1, batch))()
+        ok = load().porla_secp256k1_align_mac_batch(C.c_void_p(self.handle), n_chunks, _as_void_p(data) if data else None,
+                                                    batch, out)
+        return ok, out
+
+    def audit_aggregate(self, coefs: bytes, blocks: bytes, n: int, n_chunks: int):
+        """Server::audit's B = sum coef_j * block_j, then align_MAC on B: coefs n x 4 B LE, blocks n x n_chunks x 64 B LE.
+        Returns (the C entry's result, B % PRIME_MODULUS as n_chunks x 32 B LE, the alignment as a SecpGej)."""
+        b_out, al = bytearray(32 * n_chunks), SecpGej()
+        cf, bl = bytearray(coefs), bytearray(blocks)
+        ok = load().porla_secp256k1_audit_aggregate(C.c_void_p(self.handle), n_chunks, _as_void_p(cf) if cf else None,
+                                                    _as_void_p(bl) if bl else None, n, _as_void_p(b_out) if b_out else None,
+                                                    C.byref(al))
+        return ok, bytes(b_out), al
+
     def inner_product_prove(self, a: Sequence[int], b: Sequence[int]) -> bytes:
         """Server::inner_product_prove (Server.hpp:2279-2443); the table must hold the generators followed by u."""
         n = self.n - 1
@@ -531,6 +555,16 @@ def secp256k1_butterfly_stage(gejs, m: int, twiddles: Sequence[int]) -> int:
         for i in range(4):
             tw[k].d[i] = (w >> (64 * i)) & 0xFFFFFFFFFFFFFFFF
     return load().porla_secp256k1_butterfly_stage(gejs, len(gejs), m, tw)
+
+
+def secp256k1_ecmult_multi_gej(gejs, scalars: Sequence[int], n: int, nbatch: int = 1):
+    """r[b] = sum_i scalars[b*n + i] * gejs[b*n + i] on MACs as stored (a ctypes array of SecpGej: any z, any field
+    magnitude); scalars: n*nbatch integers below 2^256, taken mod the group order.  Returns (the C entry's result, a
+    ctypes array of nbatch SecpGej with z = 1)."""
+    sc = (SecpScalar * max(1, n * nbatch)).from_buffer_copy(
+        b"".join((s % (1 << 256)).to_bytes(32, "little") for s in scalars[:n * nbatch]).ljust(32 * max(1, n * nbatch), b"\0"))
+    r = (SecpGej * max(1, nbatch))()
+    return load().porla_secp256k1_ecmult_multi_gej(gejs, sc, n, nbatch, r), r
 
 
 def secp256k1_ecmult_multi_var(scalars: Sequence[int], points: Sequence, g_scalar: Optional[int] = None):
