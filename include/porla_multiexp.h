@@ -271,10 +271,35 @@ int porla_secp256k1_ecmult_multi_var(const porla_secp256k1_callback* error_callb
  * commitment, align_MAC and inner-product round (data.pt = &generators[start_chunk], Server.hpp:347,507,
  * 2345,2395; Client.hpp:393,1588).  Upload them once (any field magnitude, infinity flags honoured), then
  * r = sum_i scalars[i] * generators[first + i] with only the scalars crossing PCIe.  Same result
- * conventions as porla_secp256k1_ecmult_multi_var; returns 0 if the range leaves the table. */
+ * conventions as porla_secp256k1_ecmult_multi_var: r is set to infinity first, n == 0 returns 1; returns 0 if the table
+ * is NULL or not secp256k1 or the range leaves it. */
 porla_table* porla_secp256k1_table_create(const porla_secp256k1_ge* points, size_t n);
 int porla_secp256k1_ecmult_multi_table(const porla_table* t, size_t first, const porla_secp256k1_scalar* scalars,
                                        size_t n, porla_secp256k1_gej* r);
+/* Per-block commitments of an IPA-mode client or server in one call (Client::initialize's Sum A_i (alpha g_i) over 128
+ * chunks, Client.hpp:377-406 / :393; Server::compute_commitment, Server.hpp:329-360 / :347):
+ *       r[b] = sum_i scalars[b n + i] * t[first + i]     for b < batch
+ * scalars: batch x n secp256k1_scalar, taken mod n.  One batch of look-up-table sums over the resident table, the same
+ * path as porla_secp256k1_ecmult_multi_table (which is this entry with batch = 1).  With h appended to the alpha-generator
+ * table and n_chunks + 1 scalars per block (the chunks, then the PRF value) each r[b] is the block's whole MAC,
+ * commitment plus complement.  Results: z = 1, normalised limbs, infinity as gej_set_infinity writes it.  Returns 0 (r
+ * untouched) for a NULL or non-secp256k1 table, first + n beyond the table, or n * batch >= 2^31, else 1; batch == 0 does
+ * nothing and n == 0 sets every r[b] to infinity, neither touching the device.  Calls of at most 4 blocks and 4 096 terms
+ * lease a staging slot of their own, so Porla's pool threads overlap on the device. */
+int porla_secp256k1_ecmult_multi_table_batch(const porla_table* t, size_t first, const porla_secp256k1_scalar* scalars,
+                                             size_t n, size_t batch, porla_secp256k1_gej* r);
+/* The client's MAC complements batched (secp256k1_ecmult_const, ecmult_const_impl.h:137, one call per PRF value in
+ * Client::initialize after CRebuild, in every update and in Client::audit's precomputation, Client.hpp:639-654):
+ *       r[i] = scalars[i] * h     for i < n
+ * base: a length-1 secp256k1 table holding h (porla_secp256k1_table_create(&h, 1), which also builds the look-up table of
+ * its window multiples); scalars: n secp256k1_scalar as stored, not reduced (taken mod n).  k_fixed_base_mul: one thread
+ * per scalar, a sum of at most 32 look-up-table entries, no doublings.  Results: z = 1, normalised limbs, infinity as
+ * gej_set_infinity writes it (every r[i] when h is infinity).  Returns 0 (r untouched) for a NULL or non-secp256k1 base, a
+ * base whose length is not 1, or n >= 2^31, else 1; n == 0 does not touch the device.  Calls of at most 4 scalars lease a
+ * staging slot of their own.  Below 4 scalars, one porla_secp256k1_ecmult_multi_table(base, 0, &k, 1, &r) per scalar is
+ * faster (profiles/r06_ipa_client_times.txt). */
+int porla_secp256k1_ecmult_const_batch(const porla_table* base, const porla_secp256k1_scalar* scalars, size_t n,
+                                       porla_secp256k1_gej* r);
 /* Server::inner_product_prove (Server.hpp:2279-2443; SURVEY 8(f)3) over a resident table: entries 0 .. n-1 are the
  * generators (n = NUM_CHUNKS, a power of two >= 4) and entry n is the point u (Server.hpp:2376).  a, b: n scalars of 32
  * bytes, little-endian (convert_ZZ_to_arr, utils.h:353-364), any value below 2^256.  Each round's L and R are one

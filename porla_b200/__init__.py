@@ -35,5 +35,6 @@ from .lib import (  # noqa: F401
     secp256k1_ecmult_multi_var,
     secp256k1_butterfly_stage,
     secp256k1_ecmult_multi_gej,
+    secp256k1_ecmult_const_batch,
     SecpGenerators,
 )

@@ -430,14 +430,15 @@ std::shared_lock<std::shared_mutex> client_reader(bool digest, int64_t batch) {
     }
 }
 
-// `batch` fixed-base products over a resident client base (d_scalars already queued on the lease's stream), copied to data_out.
-void client_fixed_base(const ClientBase& b, const uint8_t* d_scalars, int scalar_fmt, int64_t batch, uint8_t* d_out,
-                       Staging& sg, GoSlice* data_out) {
-    porla_scalar_mul_batch_device(&b.t, d_scalars, batch, scalar_fmt, PORLA_POINT_BE64, d_out, sg.stream);
+// `batch` fixed-base products over a length-1 table (d_scalars already queued on the lease's stream); returns the lease's
+// pinned buffer holding the batch x 64 result bytes (out_fmt).
+const uint8_t* fixed_base_products(const porla_table* base, const uint8_t* d_scalars, int scalar_fmt, int64_t batch, int out_fmt,
+                                   uint8_t* d_out, Staging& sg) {
+    porla_scalar_mul_batch_device(base, d_scalars, batch, scalar_fmt, out_fmt, d_out, sg.stream);
     uint8_t* h = sg.pinned((size_t)batch * 64);
     PORLA_CUDA(cudaMemcpyAsync(h, d_out, (size_t)batch * 64, cudaMemcpyDeviceToHost, sg.stream));
     PORLA_CUDA(cudaStreamSynchronize(sg.stream));
-    go_copy(data_out, h, (size_t)batch * 64);
+    return h;
 }
 
 }  // namespace
@@ -545,6 +546,17 @@ void msm_host_jacobian_secp256k1(const uint32_t* xyz, const uint8_t* inf, const 
     table_import_jacobian_secp256k1(reinterpret_cast<const uint32_t*>(d + xyz_off), d + inf_off, (uint32_t)total, d + tab_off,
                                     d + fl_off, &tab, st);
     run_and_fetch(kCurveSecp256k1, tab, d, n, nbatch, opt, d + out_off, out, st, sg);
+}
+
+void fixed_base_mul_core(const porla_table* base, const void* scalars, int64_t n, int scalar_fmt, int out_fmt,
+                         const std::function<void(const uint8_t*)>& take) {
+    device_init();
+    StageLease lease = lease_stage(1, n);
+    Staging& sg = *lease.s;
+    const size_t sc_bytes = (size_t)n * 32, out_off = (sc_bytes + 255) & ~(size_t)255;
+    uint8_t* d = sg.dev(out_off + (size_t)n * 64);
+    h2d_copy(d, scalars, sc_bytes, sg.stream);
+    take(fixed_base_products(base, d, scalar_fmt, n, out_fmt, d + out_off, sg));
 }
 
 }  // namespace porla
@@ -773,7 +785,8 @@ void compute_digest_batch(GoSlice* data_in, GoInt batch, GoSlice* data_out) {
     if (co_bytes) h2d_copy(d, data_in->data, co_bytes, sg.stream);
     // alpha * f(tau) per record on the device, then [.]G1 over the resident table of the digest base
     fr_poly_eval_device(d, g_client.d_powers, (uint32_t)n, (uint32_t)batch, d + sc_off, sg.stream);
-    client_fixed_base(g_client.digest, d + sc_off, PORLA_SCALAR_LE32, batch, d + out_off, sg, data_out);
+    const uint8_t* h = fixed_base_products(&g_client.digest.t, d + sc_off, PORLA_SCALAR_LE32, batch, PORLA_POINT_BE64, d + out_off, sg);
+    go_copy(data_out, h, (size_t)batch * 64);
 }
 
 void compute_digest_complement_batch(GoSlice* data_in, GoInt batch, GoSlice* data_out) {
@@ -782,12 +795,8 @@ void compute_digest_complement_batch(GoSlice* data_in, GoInt batch, GoSlice* dat
     check_shape(1, batch, "compute_digest_complement_batch");
     device_init();
     std::shared_lock<std::shared_mutex> rd = client_reader(false, batch);
-    StageLease lease = lease_stage(1, batch);
-    Staging& sg = *lease.s;
-    const size_t sc_bytes = (size_t)batch * 32, out_off = (sc_bytes + 255) & ~(size_t)255;
-    uint8_t* d = sg.dev(out_off + (size_t)batch * 64);
-    h2d_copy(d, data_in->data, sc_bytes, sg.stream);
-    client_fixed_base(g_client.hmac, d, PORLA_SCALAR_BE32, batch, d + out_off, sg, data_out);
+    fixed_base_mul_core(&g_client.hmac.t, data_in->data, batch, PORLA_SCALAR_BE32, PORLA_POINT_BE64,
+                        [&](const uint8_t* h) { go_copy(data_out, h, (size_t)batch * 64); });
 }
 
 porla_table* porla_table_create(int curve, const void* points, int64_t n, int point_fmt, int on_device, void* cuda_stream) {

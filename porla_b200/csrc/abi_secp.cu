@@ -492,14 +492,39 @@ porla_table* porla_secp256k1_table_create(const porla_secp256k1_ge* points, size
     return t;
 }
 
+int porla_secp256k1_ecmult_multi_table_batch(const porla_table* t, size_t first, const porla_secp256k1_scalar* scalars,
+                                             size_t n, size_t batch, porla_secp256k1_gej* r) {
+    if (!t || t->t.curve != kCurveSecp256k1 || first > t->t.n || n > t->t.n - first) return 0;
+    if (batch && n > ((1ull << 31) - 1) / batch) return 0;   // n * batch >= 2^31: a staged call indexes terms with 32 bits
+    if (batch == 0) return 1;
+    if (n == 0) {
+        for (size_t b = 0; b < batch; b++) gej_set_infinity(r + b);
+        return 1;
+    }
+    std::vector<uint8_t> res(64 * batch);
+    porla_msm_table_host_scalars_batch(t, (int64_t)first, scalars, (int64_t)n, (int64_t)batch, PORLA_SCALAR_LE32,
+                                       PORLA_POINT_LE64, res.data());
+    for (size_t b = 0; b < batch; b++) gej_from_le64(res.data() + 64 * b, r + b);
+    return 1;
+}
+
 int porla_secp256k1_ecmult_multi_table(const porla_table* t, size_t first, const porla_secp256k1_scalar* scalars, size_t n,
                                        porla_secp256k1_gej* r) {
     gej_set_infinity(r);
     if (n == 0) return 1;
-    if ((int64_t)(first + n) > porla_table_len(t)) return 0;
-    uint8_t res[64];
-    porla_msm_table_host_scalars(t, (int64_t)first, scalars, (int64_t)n, PORLA_SCALAR_LE32, PORLA_POINT_LE64, res);
-    gej_from_le64(res, r);
+    return porla_secp256k1_ecmult_multi_table_batch(t, first, scalars, n, 1, r);
+}
+
+// The client's MAC complements (SURVEY §2 row 10): secp256k1_ecmult_const of one fixed base h by each PRF value, through
+// the fixed-base kernel of the KZG twin compute_digest_complement_batch.  porla_secp256k1_table_create(&h, 1) already
+// carries what that kernel reads: table_precompute gives a length-1 table the c = 8 look-up table of window multiples.
+int porla_secp256k1_ecmult_const_batch(const porla_table* base, const porla_secp256k1_scalar* scalars, size_t n,
+                                       porla_secp256k1_gej* r) {
+    if (!base || base->t.curve != kCurveSecp256k1 || base->t.n != 1 || n >= (1ull << 31)) return 0;
+    if (n == 0) return 1;
+    fixed_base_mul_core(base, scalars, (int64_t)n, PORLA_SCALAR_LE32, PORLA_POINT_LE64, [&](const uint8_t* h) {
+        for (size_t i = 0; i < n; i++) gej_from_le64(h + 64 * i, r + i);
+    });
     return 1;
 }
 

@@ -103,3 +103,12 @@ uint64_t h2d_ring_bytes();
 struct porla_table {
     porla::PointTable t;
 };
+
+namespace porla {
+// n products k_i * B over the ONE point of a length-1 table (compute_digest_complement_batch, porla_secp256k1_ecmult_const_batch):
+// host scalars (n x 32 bytes, scalar_fmt) copied in, porla_scalar_mul_batch_device (k_fixed_base_mul over the table's
+// look-up table), and take() handed the n x 64 result bytes (out_fmt) in the staging's pinned buffer while the staging is
+// still held.  Calls of a few scalars lease a staging slot of their own.
+void fixed_base_mul_core(const porla_table* base, const void* scalars, int64_t n, int scalar_fmt, int out_fmt,
+                         const std::function<void(const uint8_t*)>& take);
+}  // namespace porla

@@ -36,7 +36,7 @@ NEW_SYMBOLS = [
     "porla_msm_table_host_scalars", "porla_msm_table_host_scalars_batch", "porla_secp256k1_table_create", "porla_secp256k1_ecmult_multi_table",
     "porla_debug_pairing_selfcheck", "porla_debug_latency", "porla_secp256k1_inner_product_prove", "porla_secp256k1_inner_product_verify",
     "porla_secp256k1_butterfly_stage", "porla_secp256k1_align_mac_batch", "porla_secp256k1_audit_aggregate",
-    "porla_secp256k1_ecmult_multi_gej",
+    "porla_secp256k1_ecmult_multi_gej", "porla_secp256k1_ecmult_multi_table_batch", "porla_secp256k1_ecmult_const_batch",
     "porla_device_count", "porla_mtable_create", "porla_mtable_devices", "porla_mtable_len", "porla_mtable_range",
     "porla_mtable_msm_host_scalars", "porla_mtable_msm_resident", "porla_mtable_scalars_upload", "porla_mtable_scalars_free",
     "porla_mtable_destroy", "porla_debug_copy_ring_bytes", "porla_msm_host_devices", "porla_debug_h2d_rate",
@@ -134,6 +134,9 @@ def load() -> C.CDLL:
         "porla_msm_table_host_scalars_batch": (None, [P, C.c_int64, P, C.c_int64, C.c_int64, I, I, P]),
         "porla_secp256k1_table_create": (P, [C.POINTER(SecpGe), C.c_size_t]),
         "porla_secp256k1_ecmult_multi_table": (I, [P, C.c_size_t, C.POINTER(SecpScalar), C.c_size_t, C.POINTER(SecpGej)]),
+        "porla_secp256k1_ecmult_multi_table_batch": (I, [P, C.c_size_t, C.POINTER(SecpScalar), C.c_size_t, C.c_size_t,
+                                                         C.POINTER(SecpGej)]),
+        "porla_secp256k1_ecmult_const_batch": (I, [P, C.POINTER(SecpScalar), C.c_size_t, C.POINTER(SecpGej)]),
         "porla_debug_pairing_selfcheck": (I, [I]),
         "porla_secp256k1_inner_product_prove": (C.c_size_t, [P, C.c_size_t, C.c_char_p, C.c_char_p, C.c_char_p]),
         "porla_secp256k1_inner_product_verify": (I, [P, C.c_size_t, C.POINTER(SecpGej), C.c_char_p]),
@@ -476,6 +479,16 @@ def _fe_to_int(fe: SecpFe) -> int:
     return sum(int(fe.n[i]) << (52 * i) for i in range(5))
 
 
+def _scalar_array(values: Sequence[int]):
+    """ctypes array of SecpScalar (at least one element) holding integers below 2^256 as stored, not reduced."""
+    return (SecpScalar * max(1, len(values))).from_buffer_copy(
+        b"".join((s % (1 << 256)).to_bytes(32, "little") for s in values).ljust(32 * max(1, len(values)), b"\0"))
+
+
+def _affine_or_none(g: SecpGej):
+    return None if g.infinity else (_fe_to_int(g.x), _fe_to_int(g.y))
+
+
 class SecpGenerators:
     """secp256k1 generator array resident in HBM (the `generators[]` of Server.hpp:347 / Client.hpp:393)."""
 
@@ -501,6 +514,15 @@ class SecpGenerators:
         if r.infinity:
             return ok, None
         return ok, (_fe_to_int(r.x), _fe_to_int(r.y))
+
+    def multi_batch(self, first: int, scalars: Sequence[int], n: int, batch: int):
+        """(ok, list of `batch` affine results or None) of sum_i scalars[b*n + i] * generators[first + i] for b < batch:
+        the per-block commitments of Client::initialize / Server::compute_commitment in one call.  (0, None) when the
+        shape is refused."""
+        r = (SecpGej * max(1, batch))()
+        ok = load().porla_secp256k1_ecmult_multi_table_batch(C.c_void_p(self.handle), first, _scalar_array(scalars[:n * batch]),
+                                                             n, batch, r)
+        return (ok, [_affine_or_none(g) for g in r[:batch]]) if ok else (0, None)
 
     def align_mac_batch(self, data: bytearray, batch: int, n_chunks: int):
         """Server::align_MAC, IPA branch, for `batch` blocks of n_chunks chunks over generators [0, n_chunks): data =
@@ -561,10 +583,17 @@ def secp256k1_ecmult_multi_gej(gejs, scalars: Sequence[int], n: int, nbatch: int
     """r[b] = sum_i scalars[b*n + i] * gejs[b*n + i] on MACs as stored (a ctypes array of SecpGej: any z, any field
     magnitude); scalars: n*nbatch integers below 2^256, taken mod the group order.  Returns (the C entry's result, a
     ctypes array of nbatch SecpGej with z = 1)."""
-    sc = (SecpScalar * max(1, n * nbatch)).from_buffer_copy(
-        b"".join((s % (1 << 256)).to_bytes(32, "little") for s in scalars[:n * nbatch]).ljust(32 * max(1, n * nbatch), b"\0"))
     r = (SecpGej * max(1, nbatch))()
-    return load().porla_secp256k1_ecmult_multi_gej(gejs, sc, n, nbatch, r), r
+    return load().porla_secp256k1_ecmult_multi_gej(gejs, _scalar_array(scalars[:n * nbatch]), n, nbatch, r), r
+
+
+def secp256k1_ecmult_const_batch(base: SecpGenerators, scalars: Sequence[int]):
+    """The client's MAC complements in one call: scalars[i] * h for the one point h of `base` (a SecpGenerators of length
+    1).  scalars: integers below 2^256, taken mod the group order.  Returns (ok, list of affine results or None), or
+    (0, None) when the base is refused."""
+    r = (SecpGej * max(1, len(scalars)))()
+    ok = load().porla_secp256k1_ecmult_const_batch(C.c_void_p(base.handle), _scalar_array(scalars), len(scalars), r)
+    return (ok, [_affine_or_none(g) for g in r[:len(scalars)]]) if ok else (0, None)
 
 
 def secp256k1_ecmult_multi_var(scalars: Sequence[int], points: Sequence, g_scalar: Optional[int] = None):
