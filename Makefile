@@ -4,7 +4,7 @@ ARCH      := -gencode arch=compute_100a,code=sm_100a
 NVFLAGS   := $(ARCH) -O3 -std=c++17 -lineinfo -Xcompiler -fPIC -Xcompiler -Wall -Xcompiler -Wno-unknown-pragmas -diag-suppress 128
 CSRC      := porla_b200/csrc
 OBJDIR    := build
-OBJS      := $(OBJDIR)/msm.o $(OBJDIR)/msm_bn254.o $(OBJDIR)/msm_secp.o $(OBJDIR)/abi.o $(OBJDIR)/multi.o $(OBJDIR)/abi_secp.o $(OBJDIR)/pint.o $(OBJDIR)/lat.o
+OBJS      := $(OBJDIR)/msm.o $(OBJDIR)/msm_bn254.o $(OBJDIR)/msm_secp.o $(OBJDIR)/abi.o $(OBJDIR)/multi.o $(OBJDIR)/abi_secp.o $(OBJDIR)/pint.o $(OBJDIR)/lat.o $(OBJDIR)/staging.o
 HDRS      := $(wildcard $(CSRC)/*.cuh $(CSRC)/*.h $(CSRC)/*.hpp include/*.h)
 LIB       := porla_b200/libmultiexp.so
 

@@ -56,62 +56,7 @@ struct ClientState {
 ClientState g_client;
 }  // namespace
 
-namespace porla {
-std::mutex g_io_mu;
-Staging g_stage;
-}  // namespace porla
-
 namespace {
-
-// Small calls (Porla's 16..766-term MSMs and 128-term commitments) lease one of a few persistent staging slots (device
-// buffer, pinned buffer, stream, scratch block) and do not take g_io_mu: the pool threads of Server.hpp:1077-1078 /
-// Client.hpp:377-406 then overlap on the device instead of queueing behind one another.  The slots outlive the calling
-// threads (Porla builds a fresh ThreadPool inside align_MAC, Server.hpp:487).  Larger calls, and small ones when every
-// slot is taken, share g_stage under the mutex.
-constexpr int kStageSlots = 16;
-constexpr int64_t kSlotTerms = 4096, kSlotBatch = 4;
-constexpr size_t kSlotScratch = 4u << 20;
-struct StagePool {
-    std::mutex mu;
-    Staging slots[kStageSlots];
-    bool busy[kStageSlots] = {};
-};
-StagePool g_pool;
-struct StageLease {
-    Staging* s = nullptr;
-    std::unique_lock<std::mutex> lk;   // held for the shared staging area only
-    int slot = -1;
-    bool local() const { return slot >= 0; }
-    StageLease() = default;
-    StageLease(StageLease&& o) noexcept : s(o.s), lk(std::move(o.lk)), slot(o.slot) { o.slot = -1; }
-    StageLease(const StageLease&) = delete;
-    ~StageLease() {
-        if (slot >= 0) {
-            std::lock_guard<std::mutex> g(g_pool.mu);
-            g_pool.busy[slot] = false;
-        }
-    }
-};
-StageLease lease_stage(int64_t n, int64_t nbatch) {
-    StageLease l;
-    if (n * nbatch <= kSlotTerms && nbatch <= kSlotBatch && !getenv("PORLA_SERIAL_CALLS")) {
-        std::lock_guard<std::mutex> g(g_pool.mu);
-        for (int i = 0; i < kStageSlots; i++) {
-            if (!g_pool.busy[i]) {
-                g_pool.busy[i] = true;
-                l.slot = i;
-                l.s = &g_pool.slots[i];
-                break;
-            }
-        }
-    }
-    if (l.slot < 0) {
-        l.s = &g_stage;
-        l.lk = std::unique_lock<std::mutex>(g_io_mu);
-    }
-    l.s->init();
-    return l;
-}
 
 // window_bits argument of the device entry points: a plain window size, or a plan code of porla_msm_plan
 void decode_plan(int code, MsmOptions* opt) {
@@ -146,42 +91,6 @@ std::vector<Fr> read_poly(const GoSlice* data_in, int64_t n) {
     const uint8_t* b = (const uint8_t*)data_in->data;
     for (int64_t i = 0; i < n; i++) f[(size_t)i] = elem_from_be<Fr>(b + 32 * i, 32);
     return f;
-}
-
-// Runs nbatch MSMs and brings the nbatch*64-byte results to host memory.  Few MSMs: the device
-// stops at the per-window sums and the serial tail (Horner + normalisation) runs on the host, which
-// is ~15x faster than one GPU thread; many MSMs: the device finaliser runs them in parallel.
-// d_scratch_out must hold max(nbatch*64, nbatch*nwin*128) bytes.  Caller holds g_io_mu.
-constexpr int64_t kHostFinalizeMaxBatch = 4;
-size_t result_scratch_bytes(int curve, int64_t n, int64_t nbatch) {
-    MsmPlan p = msm_plan(curve, (uint32_t)n, (uint32_t)nbatch, 0);  // general plan: an upper bound for fixed-base too
-    const int nwin = p.nwin > 256 ? p.nwin : 256;                   // the bitwise small-MSM plan has one window per scalar bit
-    size_t a = (size_t)nbatch * 64, b = (size_t)nbatch * nwin * 128;
-    return a > b ? a : b;
-}
-void run_and_fetch(int curve, const PointTable& tab, const uint8_t* d_scalars, int64_t n, int64_t nbatch, MsmOptions opt,
-                   uint8_t* d_scratch_out, uint8_t* out, cudaStream_t st, Staging& sg = g_stage) {
-    const char* force_dev = getenv("PORLA_DEVICE_FINALIZE");
-    if (nbatch <= kHostFinalizeMaxBatch && !(force_dev && force_dev[0] == '1')) {
-        MsmPlan p = msm_plan_table(tab, (uint32_t)n, (uint32_t)nbatch, opt);
-        if (p.mode == kPlanPipeline) {   // the device must use exactly the layout the host combines (window size AND split)
-            opt.window_bits = p.c;
-            opt.glv = p.glv;
-        }
-        opt.d_window_sums = d_scratch_out;
-        size_t bytes = (size_t)nbatch * p.nwin * 128;
-        msm_device(curve, tab, d_scalars, (uint32_t)n, (uint32_t)nbatch, opt, nullptr, nullptr, st);
-        uint8_t* h = sg.pinned(bytes);
-        PORLA_CUDA(cudaMemcpyAsync(h, d_scratch_out, bytes, cudaMemcpyDeviceToHost, st));
-        PORLA_CUDA(cudaStreamSynchronize(st));
-        for (int64_t m = 0; m < nbatch; m++) finalize_host(curve, h + (size_t)m * p.nwin * 128, p.nwin, p.c, opt.out_fmt, out + 64 * m);
-        return;
-    }
-    msm_device(curve, tab, d_scalars, (uint32_t)n, (uint32_t)nbatch, opt, d_scratch_out, nullptr, st);
-    uint8_t* h = sg.pinned((size_t)nbatch * 64);
-    PORLA_CUDA(cudaMemcpyAsync(h, d_scratch_out, (size_t)nbatch * 64, cudaMemcpyDeviceToHost, st));
-    PORLA_CUDA(cudaStreamSynchronize(st));
-    memcpy(out, h, (size_t)nbatch * 64);
 }
 
 // Bit length of the largest scalar in a host buffer, or 0 when some scalar may need reduction (or, on
@@ -235,41 +144,32 @@ void msm_host_core(int curve, const uint8_t* scalars, const uint8_t* points, int
             return;
         }
     }
-    StageLease lease = lease_stage(n, nbatch);
-    Staging& sg = *lease.s;
+    StagedCall call(n, nbatch);
     if (nbatch == 1 && n >= (1 << 19) && !getenv("PORLA_NO_SPLIT")) {
         // streamed: the terms cross PCIe in parts that are accumulated into one bucket set as they arrive (multi.cu)
         const MsmPlan plan = msm_plan(curve, (uint32_t)n, 1, 0);
         std::vector<uint8_t> ws((size_t)plan.nwin * 128);
-        msm_host_pipelined(sg, curve, scalars, points, n, scalar_fmt, point_fmt, plan, ws.data());
+        msm_host_pipelined(call.staging(), curve, scalars, points, n, scalar_fmt, point_fmt, plan, ws.data());
         finalize_host(curve, ws.data(), plan.nwin, plan.c, point_fmt, out);
         return;
     }
     const size_t total = (size_t)n * (size_t)nbatch;
-    // staging layout: scalars | raw points | imported table + endomorphism image | infinity flags | result scratch | small-path scratch
-    auto pad = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    size_t sc_bytes = total * 32, pt_bytes = total * 64;
-    size_t sc_off = 0, pt_off = pad(sc_bytes), tab_off = pt_off + pad(pt_bytes), fl_off = tab_off + pad(2 * pt_bytes),
-           out_off = fl_off + pad(total), scr_off = out_off + pad(result_scratch_bytes(curve, n, nbatch));
-    uint8_t* d = sg.dev(scr_off + (lease.local() ? kSlotScratch : 0));
-    cudaStream_t st = sg.stream;
+    // staging layout: scalars | raw points | imported table + endomorphism image | infinity flags | result
+    const size_t sc_bytes = total * 32, pt_bytes = total * 64;
+    const size_t sc_off = call.add(sc_bytes), pt_off = call.add(pt_bytes), tab_off = call.add(2 * pt_bytes), fl_off = call.add(total);
+    call.add_result(curve, n, nbatch);
+    uint8_t* d = call.dev();
+    cudaStream_t st = call.stream();
     h2d_copy(d + sc_off, scalars, sc_bytes, st);
     h2d_copy(d + pt_off, points, pt_bytes, st);
-    MsmOptions opt;
-    opt.scalar_be = scalar_fmt == PORLA_SCALAR_BE32;
-    opt.out_fmt = point_fmt;
-    opt.shared_points = 0;
-    if (lease.local()) {
-        opt.d_scratch = d + scr_off;
-        opt.scratch_bytes = kSlotScratch;
-    }
+    MsmOptions opt = call.msm_options(scalar_fmt, point_fmt, 0);
     if (total <= 4096) opt.max_scalar_bits = host_max_scalar_bits(curve, scalars, total, opt.scalar_be);
     PointTable tab;
     tab.curve = curve;
     // the one-launch tree sum does not use the endomorphism image: skip that launch for Porla-sized calls
     const bool bits_plan = msm_plan_table(tab, (uint32_t)n, (uint32_t)nbatch, opt).mode == kPlanBits;
     table_import_into(curve, d + pt_off, point_fmt, (uint32_t)total, d + tab_off, d + fl_off, &tab, st, !bits_plan);
-    run_and_fetch(curve, tab, d + sc_off, n, nbatch, opt, d + out_off, out, st, sg);
+    call.fetch(curve, tab, d + sc_off, n, nbatch, opt, out);
 }
 
 void upload_srs_locked();
@@ -283,12 +183,14 @@ std::shared_mutex g_srs_mu;
 // Shared lock on the SRS table with the table present and at least `n` bases long; `batch_terms` = n * nbatch of the
 // call (a large batch over a mid-sized SRS, BASELINE config 3, is worth the one-time wide-window look-up table).
 std::shared_lock<std::shared_mutex> srs_reader(int64_t n, uint64_t batch_terms, int64_t nbatch) {
+    auto want_lut = [&] {   // read under g_srs_mu
+        return batch_terms >= (1ull << 22) && g_kzg.srs_table.n > 2048 && g_kzg.srs_table.n <= 8192 && !g_kzg.srs_table.d_lut &&
+               !g_kzg.lut_tried && !getenv("PORLA_NO_LUT");
+    };
     for (;;) {
         {
             std::shared_lock<std::shared_mutex> rd(g_srs_mu);
-            const bool want_lut = batch_terms >= (1ull << 22) && g_kzg.srs_table.n > 2048 && g_kzg.srs_table.n <= 8192 &&
-                                  !g_kzg.srs_table.d_lut && !g_kzg.lut_tried && !getenv("PORLA_NO_LUT");
-            if (g_kzg.have_table && !want_lut) {
+            if (g_kzg.have_table && !want_lut()) {
                 if (n > (int64_t)g_kzg.srs_table.n) die("polynomial longer than the SRS");
                 return rd;
             }
@@ -298,12 +200,10 @@ std::shared_lock<std::shared_mutex> srs_reader(int64_t n, uint64_t batch_terms, 
             if (g_kzg.srs_g1.empty()) die("SRS not initialised (call init_SRS or init_SRS_from_data first)");
             upload_srs_locked();
         }
-        if (batch_terms >= (1ull << 22) && g_kzg.srs_table.n > 2048 && g_kzg.srs_table.n <= 8192 && !g_kzg.srs_table.d_lut &&
-            !g_kzg.lut_tried && !getenv("PORLA_NO_LUT")) {
-            std::lock_guard<std::mutex> io(g_io_mu);
-            g_stage.init();
-            table_precompute(&g_kzg.srs_table, 0, (uint32_t)n, (uint32_t)nbatch, g_stage.stream);
-            PORLA_CUDA(cudaStreamSynchronize(g_stage.stream));
+        if (want_lut()) {
+            StagedCall call;
+            table_precompute(&g_kzg.srs_table, 0, (uint32_t)n, (uint32_t)nbatch, call.stream());
+            PORLA_CUDA(cudaStreamSynchronize(call.stream()));
             g_kzg.lut_tried = true;
         }
     }
@@ -314,23 +214,13 @@ void srs_commit_core(const uint8_t* coeffs_be, int64_t n, int64_t nbatch, uint8_
     check_shape(n, nbatch, "commitment over the SRS");
     device_init();
     std::shared_lock<std::shared_mutex> srs = srs_reader(n, (uint64_t)n * (uint64_t)nbatch, nbatch);
-    StageLease lease = lease_stage(n, nbatch);
-    Staging& sg = *lease.s;
-    auto pad = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    size_t sc_bytes = (size_t)n * nbatch * 32;
-    size_t out_off = pad(sc_bytes), scr_off = out_off + pad(result_scratch_bytes(kCurveBn254, n, nbatch));
-    uint8_t* d = sg.dev(scr_off + (lease.local() ? kSlotScratch : 0));
-    cudaStream_t st = sg.stream;
-    h2d_copy(d, coeffs_be, sc_bytes, st);
-    MsmOptions opt;
-    opt.scalar_be = 1;
-    opt.out_fmt = PORLA_POINT_BE64;
-    opt.shared_points = 1;
-    if (lease.local()) {
-        opt.d_scratch = d + scr_off;
-        opt.scratch_bytes = kSlotScratch;
-    }
-    run_and_fetch(kCurveBn254, g_kzg.srs_table, d, n, nbatch, opt, d + out_off, out, st, sg);   // synchronises `st`
+    StagedCall call(n, nbatch);
+    const size_t sc_bytes = (size_t)n * nbatch * 32;
+    call.add(sc_bytes);
+    call.add_result(kCurveBn254, n, nbatch);
+    uint8_t* d = call.dev();
+    h2d_copy(d, coeffs_be, sc_bytes, call.stream());
+    call.fetch(kCurveBn254, g_kzg.srs_table, d, n, nbatch, call.msm_options(PORLA_SCALAR_BE32, PORLA_POINT_BE64, 1), out);
 }
 
 // SRS bases go to HBM once, at init when a device is present (otherwise on the first commit,
@@ -338,17 +228,16 @@ void srs_commit_core(const uint8_t* coeffs_be, int64_t n, int64_t nbatch, uint8_
 // Caller holds g_srs_mu exclusively.
 void upload_srs_locked() {
     device_init();
-    std::lock_guard<std::mutex> lock(g_io_mu);
-    g_stage.init();
+    StagedCall call;
     if (g_kzg.srs_table.d_points) table_free(&g_kzg.srs_table);
     std::vector<uint8_t> bytes(g_kzg.srs_g1.size() * 64);
     for (size_t i = 0; i < g_kzg.srs_g1.size(); i++) g1_marshal(g_kzg.srs_g1[i], bytes.data() + 64 * i);
     table_import_host(kCurveBn254, bytes.data(), PORLA_POINT_BE64, (uint32_t)g_kzg.srs_g1.size(), &g_kzg.srs_table,
-                      g_stage.stream);
+                      call.stream());
     // the SRS is a fixed base: expand it once so that commitments need no per-window reduction
     if (!getenv("PORLA_NO_FIXED_BASE")) {
-        table_precompute(&g_kzg.srs_table, 0, (uint32_t)g_kzg.srs_g1.size(), 1, g_stage.stream);
-        PORLA_CUDA(cudaStreamSynchronize(g_stage.stream));
+        table_precompute(&g_kzg.srs_table, 0, (uint32_t)g_kzg.srs_g1.size(), 1, call.stream());
+        PORLA_CUDA(cudaStreamSynchronize(call.stream()));
     }
     g_kzg.have_table = true;
     g_kzg.lut_tried = false;
@@ -376,14 +265,13 @@ bool client_base_fresh(const ClientBase& b, int64_t batch) {
 // table_precompute with window_bits = 0 gives a length-1 table the c = 8 look-up table, or the wide one for a large batch.
 void client_base_build(ClientBase* b, const G1A& base, int64_t batch) {
     device_init();
-    std::lock_guard<std::mutex> io(g_io_mu);
-    g_stage.init();
+    StagedCall call;
     if (b->t.t.d_points) table_free(&b->t.t);   // no reader left: each synchronised its stream before dropping g_srs_mu
     uint8_t bytes[64];
     g1_marshal(base, bytes);
-    table_import_host(kCurveBn254, bytes, PORLA_POINT_BE64, 1, &b->t.t, g_stage.stream);
-    table_precompute(&b->t.t, 0, 1, (uint32_t)(batch > 0 ? batch : 1), g_stage.stream);
-    PORLA_CUDA(cudaStreamSynchronize(g_stage.stream));
+    table_import_host(kCurveBn254, bytes, PORLA_POINT_BE64, 1, &b->t.t, call.stream());
+    table_precompute(&b->t.t, 0, 1, (uint32_t)(batch > 0 ? batch : 1), call.stream());
+    PORLA_CUDA(cudaStreamSynchronize(call.stream()));
     b->gen = g_kzg.gen;
     b->wide_tried = batch >= kWideBatch;
 }
@@ -430,14 +318,14 @@ std::shared_lock<std::shared_mutex> client_reader(bool digest, int64_t batch) {
     }
 }
 
-// `batch` fixed-base products over a length-1 table (d_scalars already queued on the lease's stream); returns the lease's
+// `batch` fixed-base products over a length-1 table (d_scalars already queued on the call's stream); returns the call's
 // pinned buffer holding the batch x 64 result bytes (out_fmt).
-const uint8_t* fixed_base_products(const porla_table* base, const uint8_t* d_scalars, int scalar_fmt, int64_t batch, int out_fmt,
-                                   uint8_t* d_out, Staging& sg) {
-    porla_scalar_mul_batch_device(base, d_scalars, batch, scalar_fmt, out_fmt, d_out, sg.stream);
-    uint8_t* h = sg.pinned((size_t)batch * 64);
-    PORLA_CUDA(cudaMemcpyAsync(h, d_out, (size_t)batch * 64, cudaMemcpyDeviceToHost, sg.stream));
-    PORLA_CUDA(cudaStreamSynchronize(sg.stream));
+const uint8_t* fixed_base_products(StagedCall& call, const porla_table* base, const uint8_t* d_scalars, int scalar_fmt,
+                                   int64_t batch, int out_fmt, uint8_t* d_out) {
+    porla_scalar_mul_batch_device(base, d_scalars, batch, scalar_fmt, out_fmt, d_out, call.stream());
+    uint8_t* h = call.pinned((size_t)batch * 64);
+    PORLA_CUDA(cudaMemcpyAsync(h, d_out, (size_t)batch * 64, cudaMemcpyDeviceToHost, call.stream()));
+    PORLA_CUDA(cudaStreamSynchronize(call.stream()));
     return h;
 }
 
@@ -464,40 +352,30 @@ PointTable table_window(const PointTable& t, int64_t first, int64_t n) {
 void align_mac_core(int curve, const PointTable& gens, void* data, int64_t n, int64_t batch, int out_fmt, uint8_t* out) {
     if (batch == 0) return;
     device_init();
-    StageLease lease = lease_stage(n, batch);
-    Staging& sg = *lease.s;
+    StagedCall call(n, batch);
     const size_t total = (size_t)batch * n;
-    auto pad = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    const size_t sc_off = pad(total * 64), out_off = sc_off + pad(total * 32),
-                 scr_off = out_off + pad(result_scratch_bytes(curve, n, batch));
-    uint8_t* d = sg.dev(scr_off + (lease.local() ? kSlotScratch : 0));
-    cudaStream_t st = sg.stream;
+    call.add(total * 64);
+    const size_t sc_off = call.add(total * 32);
+    call.add_result(curve, n, batch);
+    uint8_t* d = call.dev();
+    cudaStream_t st = call.stream();
     h2d_copy(d, data, total * 64, st);
     align_scalars_device(curve, reinterpret_cast<uint32_t*>(d), (uint32_t)total, d + sc_off, st);
     PORLA_CUDA(cudaMemcpyAsync(data, d, total * 64, cudaMemcpyDeviceToHost, st));   // A[i] <- A[i] % PRIME_MODULUS
-    MsmOptions opt;
-    opt.scalar_be = 1;
-    opt.out_fmt = out_fmt;
-    opt.shared_points = 1;
-    if (lease.local()) {
-        opt.d_scratch = d + scr_off;
-        opt.scratch_bytes = kSlotScratch;
-    }
-    run_and_fetch(curve, gens, d + sc_off, n, batch, opt, d + out_off, out, st, sg);
+    call.fetch(curve, gens, d + sc_off, n, batch, call.msm_options(PORLA_SCALAR_BE32, out_fmt, 1), out);
 }
 
 void audit_aggregate_core(int curve, const PointTable& gens, const void* coefs, const void* blocks, int64_t n, int64_t chunks,
                           int out_fmt, uint8_t* b_mod_be, uint8_t* out64) {
     device_init();
     // the blocks are the call's volume: a slot is leased when they are no more than a small MSM's terms
-    StageLease lease = lease_stage((n > 0 ? n : 1) * chunks, 1);
-    Staging& sg = *lease.s;
-    auto pad = [](size_t v) { return (v + 255) & ~(size_t)255; };
+    StagedCall call((n > 0 ? n : 1) * chunks, 1);
     const size_t blk_bytes = (size_t)n * chunks * 64;
-    const size_t cf_off = pad(blk_bytes), b_off = cf_off + pad((size_t)n * 4 + 4), c_off = b_off + pad((size_t)chunks * 32),
-                 out_off = c_off + pad((size_t)chunks * 32), scr_off = out_off + pad(result_scratch_bytes(curve, chunks, 1));
-    uint8_t* d = sg.dev(scr_off + (lease.local() ? kSlotScratch : 0));
-    cudaStream_t st = sg.stream;
+    call.add(blk_bytes);
+    const size_t cf_off = call.add((size_t)n * 4 + 4), b_off = call.add((size_t)chunks * 32), c_off = call.add((size_t)chunks * 32);
+    call.add_result(curve, chunks, 1);
+    uint8_t* d = call.dev();
+    cudaStream_t st = call.stream();
     if (n) {
         h2d_copy(d, blocks, blk_bytes, st);
         PORLA_CUDA(cudaMemcpyAsync(d + cf_off, coefs, (size_t)n * 4, cudaMemcpyHostToDevice, st));
@@ -505,58 +383,40 @@ void audit_aggregate_core(int curve, const PointTable& gens, const void* coefs, 
     audit_aggregate_device(curve, reinterpret_cast<const uint32_t*>(d + cf_off), reinterpret_cast<const uint32_t*>(d), (uint32_t)n,
                            (uint32_t)chunks, d + b_off, d + c_off, st);
     PORLA_CUDA(cudaMemcpyAsync(b_mod_be, d + b_off, (size_t)chunks * 32, cudaMemcpyDeviceToHost, st));
-    MsmOptions opt;
-    opt.scalar_be = 1;
-    opt.out_fmt = out_fmt;
-    opt.shared_points = 1;
-    if (lease.local()) {
-        opt.d_scratch = d + scr_off;
-        opt.scratch_bytes = kSlotScratch;
-    }
-    run_and_fetch(curve, gens, d + c_off, chunks, 1, opt, d + out_off, out64, st, sg);
+    call.fetch(curve, gens, d + c_off, chunks, 1, call.msm_options(PORLA_SCALAR_BE32, out_fmt, 1), out64);
 }
 
 void msm_host_jacobian_secp256k1(const uint32_t* xyz, const uint8_t* inf, const void* scalars, int64_t n, int64_t nbatch,
                                  uint8_t* out) {
     check_shape(n, nbatch, "secp256k1 Jacobian MSM");
     device_init();
-    StageLease lease = lease_stage(n, nbatch);
-    Staging& sg = *lease.s;
+    StagedCall call(n, nbatch);
     const size_t total = (size_t)n * nbatch;
-    // staging layout: scalars | X, Y, Z | infinity flags in | affine table | its flags | result scratch | small-path scratch
-    auto pad = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    const size_t xyz_off = pad(total * 32), inf_off = xyz_off + pad(total * 96), tab_off = inf_off + pad(total),
-                 fl_off = tab_off + pad(total * 64), out_off = fl_off + pad(total),
-                 scr_off = out_off + pad(result_scratch_bytes(kCurveSecp256k1, n, nbatch));
-    uint8_t* d = sg.dev(scr_off + (lease.local() ? kSlotScratch : 0));
-    cudaStream_t st = sg.stream;
+    // staging layout: scalars | X, Y, Z | infinity flags in | affine table | its flags | result
+    call.add(total * 32);
+    const size_t xyz_off = call.add(total * 96), inf_off = call.add(total), tab_off = call.add(total * 64), fl_off = call.add(total);
+    call.add_result(kCurveSecp256k1, n, nbatch);
+    uint8_t* d = call.dev();
+    cudaStream_t st = call.stream();
     h2d_copy(d, scalars, total * 32, st);
     h2d_copy(d + xyz_off, xyz, total * 96, st);
     h2d_copy(d + inf_off, inf, total, st);
-    MsmOptions opt;
-    opt.scalar_be = 0;
-    opt.out_fmt = PORLA_POINT_LE64;
-    opt.shared_points = 0;
-    if (lease.local()) {
-        opt.d_scratch = d + scr_off;
-        opt.scratch_bytes = kSlotScratch;
-    }
+    MsmOptions opt = call.msm_options(PORLA_SCALAR_LE32, PORLA_POINT_LE64, 0);
     if (total <= 4096) opt.max_scalar_bits = host_max_scalar_bits(kCurveSecp256k1, (const uint8_t*)scalars, total, 0);
     PointTable tab;
     table_import_jacobian_secp256k1(reinterpret_cast<const uint32_t*>(d + xyz_off), d + inf_off, (uint32_t)total, d + tab_off,
                                     d + fl_off, &tab, st);
-    run_and_fetch(kCurveSecp256k1, tab, d, n, nbatch, opt, d + out_off, out, st, sg);
+    call.fetch(kCurveSecp256k1, tab, d, n, nbatch, opt, out);
 }
 
-void fixed_base_mul_core(const porla_table* base, const void* scalars, int64_t n, int scalar_fmt, int out_fmt,
-                         const std::function<void(const uint8_t*)>& take) {
-    device_init();
-    StageLease lease = lease_stage(1, n);
-    Staging& sg = *lease.s;
-    const size_t sc_bytes = (size_t)n * 32, out_off = (sc_bytes + 255) & ~(size_t)255;
-    uint8_t* d = sg.dev(out_off + (size_t)n * 64);
-    h2d_copy(d, scalars, sc_bytes, sg.stream);
-    take(fixed_base_products(base, d, scalar_fmt, n, out_fmt, d + out_off, sg));
+const uint8_t* fixed_base_mul_core(StagedCall& call, const porla_table* base, const void* scalars, int64_t n, int scalar_fmt,
+                                   int out_fmt) {
+    const size_t sc_bytes = (size_t)n * 32;
+    call.add(sc_bytes);
+    const size_t out_off = call.add((size_t)n * 64);
+    uint8_t* d = call.dev();
+    h2d_copy(d, scalars, sc_bytes, call.stream());
+    return fixed_base_products(call, base, d, scalar_fmt, n, out_fmt, d + out_off);
 }
 
 }  // namespace porla
@@ -777,15 +637,15 @@ void compute_digest_batch(GoSlice* data_in, GoInt batch, GoSlice* data_out) {
     check_shape(n, batch, "compute_digest_batch");
     device_init();
     std::shared_lock<std::shared_mutex> rd = client_reader(true, batch);
-    StageLease lease = lease_stage(n, batch);
-    Staging& sg = *lease.s;
-    auto pad = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    const size_t co_bytes = (size_t)n * batch * 32, sc_off = pad(co_bytes), out_off = sc_off + pad((size_t)batch * 32);
-    uint8_t* d = sg.dev(out_off + (size_t)batch * 64);
-    if (co_bytes) h2d_copy(d, data_in->data, co_bytes, sg.stream);
+    StagedCall call(n, batch);
+    const size_t co_bytes = (size_t)n * batch * 32;
+    call.add(co_bytes);
+    const size_t sc_off = call.add((size_t)batch * 32), out_off = call.add((size_t)batch * 64);
+    uint8_t* d = call.dev();
+    if (co_bytes) h2d_copy(d, data_in->data, co_bytes, call.stream());
     // alpha * f(tau) per record on the device, then [.]G1 over the resident table of the digest base
-    fr_poly_eval_device(d, g_client.d_powers, (uint32_t)n, (uint32_t)batch, d + sc_off, sg.stream);
-    const uint8_t* h = fixed_base_products(&g_client.digest.t, d + sc_off, PORLA_SCALAR_LE32, batch, PORLA_POINT_BE64, d + out_off, sg);
+    fr_poly_eval_device(d, g_client.d_powers, (uint32_t)n, (uint32_t)batch, d + sc_off, call.stream());
+    const uint8_t* h = fixed_base_products(call, &g_client.digest.t, d + sc_off, PORLA_SCALAR_LE32, batch, PORLA_POINT_BE64, d + out_off);
     go_copy(data_out, h, (size_t)batch * 64);
 }
 
@@ -795,8 +655,9 @@ void compute_digest_complement_batch(GoSlice* data_in, GoInt batch, GoSlice* dat
     check_shape(1, batch, "compute_digest_complement_batch");
     device_init();
     std::shared_lock<std::shared_mutex> rd = client_reader(false, batch);
-    fixed_base_mul_core(&g_client.hmac.t, data_in->data, batch, PORLA_SCALAR_BE32, PORLA_POINT_BE64,
-                        [&](const uint8_t* h) { go_copy(data_out, h, (size_t)batch * 64); });
+    StagedCall call(1, batch);
+    go_copy(data_out, fixed_base_mul_core(call, &g_client.hmac.t, data_in->data, batch, PORLA_SCALAR_BE32, PORLA_POINT_BE64),
+            (size_t)batch * 64);
 }
 
 porla_table* porla_table_create(int curve, const void* points, int64_t n, int point_fmt, int on_device, void* cuda_stream) {
@@ -929,23 +790,13 @@ void porla_msm_table_host_scalars_batch(const porla_table* t, int64_t first, con
         return;
     }
     device_init();
-    StageLease lease = lease_stage(n, nbatch);
-    Staging& sg = *lease.s;
-    auto pad = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    size_t sc_bytes = (size_t)n * nbatch * 32, out_off = pad(sc_bytes), scr_off = out_off + pad(result_scratch_bytes(t->t.curve, n, nbatch));
-    uint8_t* d = sg.dev(scr_off + (lease.local() ? kSlotScratch : 0));
-    cudaStream_t st = sg.stream;
-    h2d_copy(d, scalars, sc_bytes, st);
-    const PointTable view = table_window(t->t, first, n);
-    MsmOptions opt;
-    opt.scalar_be = scalar_fmt == PORLA_SCALAR_BE32;
-    opt.out_fmt = out_fmt;
-    opt.shared_points = 1;
-    if (lease.local()) {
-        opt.d_scratch = d + scr_off;
-        opt.scratch_bytes = kSlotScratch;
-    }
-    run_and_fetch(t->t.curve, view, d, n, nbatch, opt, d + out_off, (uint8_t*)out, st, sg);
+    StagedCall call(n, nbatch);
+    const size_t sc_bytes = (size_t)n * nbatch * 32;
+    call.add(sc_bytes);
+    call.add_result(t->t.curve, n, nbatch);
+    uint8_t* d = call.dev();
+    h2d_copy(d, scalars, sc_bytes, call.stream());
+    call.fetch(t->t.curve, table_window(t->t, first, n), d, n, nbatch, call.msm_options(scalar_fmt, out_fmt, 1), (uint8_t*)out);
 }
 
 void porla_msm_table_host_scalars(const porla_table* t, int64_t first, const void* scalars, int64_t n, int scalar_fmt,
@@ -1051,15 +902,15 @@ void porla_data_butterfly_stage(void* blocks, int64_t n_blocks, int64_t chunks, 
                                 const void* lcm_le64) {
     if (m < 2 || (m & (m - 1)) || n_blocks % m || chunks <= 0) die("porla_data_butterfly_stage: m must be a power of two dividing the block count");
     device_init();
-    std::lock_guard<std::mutex> lock(g_io_mu);
-    g_stage.init();
-    auto pad = [](size_t v) { return (v + 255) & ~(size_t)255; };
+    StagedCall call;
     const size_t bytes = (size_t)n_blocks * chunks * 64, tw_bytes = (size_t)(m / 2) * 32;
-    uint8_t* d = g_stage.dev(pad(bytes) + pad(tw_bytes));
-    cudaStream_t st = g_stage.stream;
+    call.add(bytes);
+    const size_t tw_off = call.add(tw_bytes);
+    uint8_t* d = call.dev();
+    cudaStream_t st = call.stream();
     h2d_copy(d, blocks, bytes, st);
-    PORLA_CUDA(cudaMemcpyAsync(d + pad(bytes), twiddles_le32, tw_bytes, cudaMemcpyHostToDevice, st));
-    data_butterfly_stage_device(reinterpret_cast<uint32_t*>(d), (uint32_t)n_blocks, (uint32_t)chunks, (uint32_t)m, d + pad(bytes),
+    PORLA_CUDA(cudaMemcpyAsync(d + tw_off, twiddles_le32, tw_bytes, cudaMemcpyHostToDevice, st));
+    data_butterfly_stage_device(reinterpret_cast<uint32_t*>(d), (uint32_t)n_blocks, (uint32_t)chunks, (uint32_t)m, d + tw_off,
                                 (const uint8_t*)lcm_le64, st);
     PORLA_CUDA(cudaMemcpyAsync(blocks, d, bytes, cudaMemcpyDeviceToHost, st));
     PORLA_CUDA(cudaStreamSynchronize(st));
@@ -1144,12 +995,11 @@ void bn254_butterfly_stage(GoSlice* points, GoInt n, GoInt m, GoSlice* twiddles)
         return;
     }
     device_init();
-    std::lock_guard<std::mutex> lock(g_io_mu);
-    g_stage.init();
+    StagedCall call;
     porla_table t;
-    table_import_host(kCurveBn254, (const uint8_t*)points->data, PORLA_POINT_BE64, (uint32_t)n, &t.t, g_stage.stream);
-    porla_butterfly_stage_device(&t, m, twiddles->data, PORLA_SCALAR_BE32, 0, g_stage.stream);
-    porla_table_export(&t, PORLA_POINT_BE64, points->data, 0, g_stage.stream);
+    table_import_host(kCurveBn254, (const uint8_t*)points->data, PORLA_POINT_BE64, (uint32_t)n, &t.t, call.stream());
+    porla_butterfly_stage_device(&t, m, twiddles->data, PORLA_SCALAR_BE32, 0, call.stream());
+    porla_table_export(&t, PORLA_POINT_BE64, points->data, 0, call.stream());
     table_free(&t.t);
 }
 
@@ -1210,14 +1060,14 @@ int porla_debug_pairing_selfcheck(int rounds) {
 
 void porla_debug_field_op(int curve, int op, const void* a, const void* b, int64_t n, void* out) {
     device_init();
-    std::lock_guard<std::mutex> lock(g_io_mu);
-    size_t bytes = (size_t)n * 32;
-    uint8_t* d = g_stage.dev(3 * bytes + 1024);
-    cudaStream_t st = g_stage.stream;
-    PORLA_CUDA(cudaMemcpyAsync(d, a, bytes, cudaMemcpyHostToDevice, st));
-    PORLA_CUDA(cudaMemcpyAsync(d + bytes, b, bytes, cudaMemcpyHostToDevice, st));
-    field_mul_device(curve, d, d + bytes, (uint32_t)n, op, d + 2 * bytes, st);
-    PORLA_CUDA(cudaMemcpyAsync(out, d + 2 * bytes, bytes, cudaMemcpyDeviceToHost, st));
+    StagedCall call;
+    const size_t bytes = (size_t)n * 32, a_off = call.add(bytes), b_off = call.add(bytes), out_off = call.add(bytes);
+    uint8_t* d = call.dev();
+    cudaStream_t st = call.stream();
+    PORLA_CUDA(cudaMemcpyAsync(d + a_off, a, bytes, cudaMemcpyHostToDevice, st));
+    PORLA_CUDA(cudaMemcpyAsync(d + b_off, b, bytes, cudaMemcpyHostToDevice, st));
+    field_mul_device(curve, d + a_off, d + b_off, (uint32_t)n, op, d + out_off, st);
+    PORLA_CUDA(cudaMemcpyAsync(out, d + out_off, bytes, cudaMemcpyDeviceToHost, st));
     PORLA_CUDA(cudaStreamSynchronize(st));
 }
 

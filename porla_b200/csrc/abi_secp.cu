@@ -5,7 +5,6 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
-#include <mutex>
 #include <vector>
 
 #include "../../include/porla_multiexp.h"
@@ -115,6 +114,10 @@ void gej_from_le64(const uint8_t* b, porla_secp256k1_gej* r) {
     memset(&r->z, 0, sizeof(r->z));
     r->z.n[0] = 1;
     r->infinity = 0;
+}
+
+void gej_batch_from_le64(const uint8_t* b, size_t n, porla_secp256k1_gej* r) {
+    for (size_t i = 0; i < n; i++) gej_from_le64(b + 64 * i, r + i);
 }
 
 const uint8_t kGenLE[64] = {
@@ -397,13 +400,12 @@ void butterfly_stage_gpu(porla_secp256k1_gej* pts, size_t n, size_t m, const por
     std::vector<uint8_t> inf;
     gej_to_device_form(pts, n, &xyz, &inf);
     device_init();
-    std::lock_guard<std::mutex> lock(g_io_mu);
-    g_stage.init();
-    auto pad = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    const size_t o_inf = pad(96 * n), o_tw = o_inf + pad(n), o_pts = o_tw + pad(32 * (m / 2)), o_flags = o_pts + pad(64 * n),
-                 o_out = o_flags + pad(n);
-    uint8_t* d = g_stage.dev(o_out + 64 * n);
-    cudaStream_t st = g_stage.stream;
+    StagedCall call;
+    call.add(96 * n);
+    const size_t o_inf = call.add(n), o_tw = call.add(32 * (m / 2)), o_pts = call.add(64 * n), o_flags = call.add(n),
+                 o_out = call.add(64 * n);
+    uint8_t* d = call.dev();
+    cudaStream_t st = call.stream();
     h2d_copy(d, xyz.data(), 96 * n, st);
     PORLA_CUDA(cudaMemcpyAsync(d + o_inf, inf.data(), n, cudaMemcpyHostToDevice, st));
     PORLA_CUDA(cudaMemcpyAsync(d + o_tw, tw, 32 * (m / 2), cudaMemcpyHostToDevice, st));
@@ -414,7 +416,7 @@ void butterfly_stage_gpu(porla_secp256k1_gej* pts, size_t n, size_t m, const por
     std::vector<uint8_t> out(64 * n);
     PORLA_CUDA(cudaMemcpyAsync(out.data(), d + o_out, 64 * n, cudaMemcpyDeviceToHost, st));
     PORLA_CUDA(cudaStreamSynchronize(st));
-    for (size_t i = 0; i < n; i++) gej_from_le64(out.data() + 64 * i, pts + i);
+    gej_batch_from_le64(out.data(), n, pts);
 }
 
 // A resident secp256k1 table holding at least n_chunks generators; a staged call indexes terms with 32 bits
@@ -504,7 +506,7 @@ int porla_secp256k1_ecmult_multi_table_batch(const porla_table* t, size_t first,
     std::vector<uint8_t> res(64 * batch);
     porla_msm_table_host_scalars_batch(t, (int64_t)first, scalars, (int64_t)n, (int64_t)batch, PORLA_SCALAR_LE32,
                                        PORLA_POINT_LE64, res.data());
-    for (size_t b = 0; b < batch; b++) gej_from_le64(res.data() + 64 * b, r + b);
+    gej_batch_from_le64(res.data(), batch, r);
     return 1;
 }
 
@@ -522,9 +524,9 @@ int porla_secp256k1_ecmult_const_batch(const porla_table* base, const porla_secp
                                        porla_secp256k1_gej* r) {
     if (!base || base->t.curve != kCurveSecp256k1 || base->t.n != 1 || n >= (1ull << 31)) return 0;
     if (n == 0) return 1;
-    fixed_base_mul_core(base, scalars, (int64_t)n, PORLA_SCALAR_LE32, PORLA_POINT_LE64, [&](const uint8_t* h) {
-        for (size_t i = 0; i < n; i++) gej_from_le64(h + 64 * i, r + i);
-    });
+    device_init();
+    StagedCall call(1, (int64_t)n);
+    gej_batch_from_le64(fixed_base_mul_core(call, base, scalars, (int64_t)n, PORLA_SCALAR_LE32, PORLA_POINT_LE64), n, r);
     return 1;
 }
 
@@ -538,7 +540,7 @@ int porla_secp256k1_align_mac_batch(const porla_table* gens, size_t n_chunks, vo
     std::vector<uint8_t> res(64 * batch);
     align_mac_core(kCurveSecp256k1, table_window(gens->t, 0, (int64_t)n_chunks), data, (int64_t)n_chunks, (int64_t)batch,
                    PORLA_POINT_LE64, res.data());
-    for (size_t b = 0; b < batch; b++) gej_from_le64(res.data() + 64 * b, align_out + b);
+    gej_batch_from_le64(res.data(), batch, align_out);
     return 1;
 }
 
@@ -576,7 +578,7 @@ int porla_secp256k1_ecmult_multi_gej(const porla_secp256k1_gej* points, const po
     gej_to_device_form(points, n * nbatch, &xyz, &inf);
     std::vector<uint8_t> res(64 * nbatch);
     msm_host_jacobian_secp256k1(xyz.data(), inf.data(), scalars, (int64_t)n, (int64_t)nbatch, res.data());
-    for (size_t b = 0; b < nbatch; b++) gej_from_le64(res.data() + 64 * b, r + b);
+    gej_batch_from_le64(res.data(), nbatch, r);
     return 1;
 }
 

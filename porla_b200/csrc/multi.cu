@@ -318,14 +318,13 @@ static MsmOptions window_sums_options(const MsmPlan& plan, int scalar_fmt, int o
 
 void msm_host_pipelined(Staging& sg, int curve, const uint8_t* scalars, const uint8_t* points, int64_t n, int scalar_fmt,
                         int point_fmt, const MsmPlan& plan, uint8_t* h_ws) {
-    auto pad = [](size_t v) { return (v + 255) & ~(size_t)255; };
     const int nparts = stream_parts_for(n, plan);
     const size_t ws_bytes = (size_t)plan.nwin * 128;
-    const size_t bk_bytes = nparts > 1 ? msm_bucket_bytes(plan) : 0;
     // staging layout: scalars | raw points | table + endomorphism image (2 * 64 B per point) | flags | window sums | buckets
-    size_t sc_off = 0, pt_off = pad((size_t)n * 32), tab_off = pt_off + pad((size_t)n * 64), fl_off = tab_off + pad((size_t)n * 128),
-           ws_off = fl_off + pad((size_t)n), bk_off = ws_off + pad(ws_bytes);
-    uint8_t* d = sg.dev(bk_off + pad(bk_bytes));
+    StageLayout lay;
+    const size_t sc_off = lay.add((size_t)n * 32), pt_off = lay.add((size_t)n * 64), tab_off = lay.add((size_t)n * 128),
+                 fl_off = lay.add((size_t)n), ws_off = lay.add(ws_bytes), bk_off = lay.add(nparts > 1 ? msm_bucket_bytes(plan) : 0);
+    uint8_t* d = sg.dev(lay.size);
     cudaStream_t st = sg.stream, cs = sg.copy_stream;
     MsmOptions opt = window_sums_options(plan, scalar_fmt, point_fmt, d + ws_off);
     if (nparts > 1) opt.d_buckets = d + bk_off;
@@ -389,22 +388,6 @@ struct porla_mtable {
     uint8_t* d_scalars[kMaxDevices] = {};     // per-device scratch for host-scalar calls (count * 32 B)
     uint8_t* d_ws[kMaxDevices] = {};          // per-device window sums
 };
-
-// entries [a, a + len) of a resident table (no fixed-base expansion: the parts of a sharded MSM exchange nwin window sums)
-static PointTable table_view(const PointTable& full, size_t a, size_t len) {
-    PointTable view = full;
-    view.d_points = (uint8_t*)full.d_points + a * 64;
-    view.d_flags = full.d_flags ? full.d_flags + a : nullptr;
-    view.n = (uint32_t)len;
-    view.d_fb_points = nullptr;
-    view.d_lut = nullptr;
-    view.fb_c = view.fb_nwin = 0;
-    if (full.d_phi_x) {
-        view.d_phi_x = (uint8_t*)full.d_phi_x + a * 32;
-        view.phi_off = (uint32_t)len;
-    }
-    return view;
-}
 
 extern "C" {
 
@@ -486,7 +469,8 @@ static void mtable_msm(const porla_mtable* mt, const uint8_t* h_scalars, void* c
                 h2d_copy(mt->d_scalars[p] + a * 32, h_scalars + ((size_t)mt->first[p] + a) * 32, len * 32, sg.copy_stream);
                 PORLA_CUDA(cudaEventRecord(sg.ev[h], sg.copy_stream));
                 PORLA_CUDA(cudaStreamWaitEvent(sg.stream, sg.ev[h], 0));
-                const PointTable view = table_view(mt->part[p], a, len);   // entries [a, a + len) of this device's range
+                // entries [a, a + len) of this device's range (a sharded part has no fixed-base expansion)
+                const PointTable view = table_window(mt->part[p], (int64_t)a, (int64_t)len);
                 opt.part_mode = part_mode(h, nparts);
                 msm_device(mt->curve, view, mt->d_scalars[p] + a * 32, (uint32_t)len, 1, opt, nullptr, nullptr, sg.stream);
                 a = last;

@@ -71,6 +71,59 @@ void h2d_copy(void* d_dst, const void* h_src, size_t bytes, cudaStream_t stream)
 extern std::mutex g_io_mu;
 extern Staging g_stage;
 
+// Regions of one staging device buffer, each 256-byte aligned: add() every region, make ONE Staging::dev(size) call (it may
+// reallocate), then form the pointers from the offsets add() returned.
+struct StageLayout {
+    size_t size = 0;
+    size_t add(size_t bytes) {
+        const size_t off = size;
+        size += (bytes + 255) & ~(size_t)255;
+        return off;
+    }
+};
+
+// Runs nbatch MSMs and brings the nbatch*64-byte results to `out`, through sg's pinned buffer.  Few MSMs: the device stops at
+// the per-window sums and the serial tail (Horner + normalisation) runs on the host, which is ~15x faster than one GPU thread;
+// many MSMs: the device finaliser runs them in parallel.  d_scratch_out must hold max(nbatch*64, nbatch*nwin*128) bytes.
+// Returns after `st` has been synchronised.
+void run_and_fetch(int curve, const PointTable& tab, const uint8_t* d_scalars, int64_t n, int64_t nbatch, MsmOptions opt,
+                   uint8_t* d_scratch_out, uint8_t* out, cudaStream_t st, Staging& sg = g_stage);
+
+// The staging of one host-buffer call.  StagedCall(n, nbatch): calls of at most 4096 terms and 4 MSMs lease one of a few
+// persistent slots (device buffer, pinned buffer, stream, scratch block) and take no global lock, so Porla's pool threads
+// (Server.hpp:1077-1078, Client.hpp:377-406) overlap on the device instead of queueing behind one another; larger calls,
+// small ones when every slot is taken, and every call under PORLA_SERIAL_CALLS share g_stage under g_io_mu.  StagedCall():
+// always the shared area.  The staging is held until the frame is destroyed, so results read from pinned() stay valid until then.
+class StagedCall {
+  public:
+    StagedCall();
+    StagedCall(int64_t n, int64_t nbatch);
+    ~StagedCall();
+
+    // Layout phase: add() returns the offset of a region; add_result() reserves what fetch() needs for nbatch MSMs of n terms
+    // (and, in a slot, the scratch block that keeps the one-launch kernels off the engine's arena).  Then ONE dev() call;
+    // pointers are dev() + offset.
+    size_t add(size_t bytes) { return layout_.add(bytes); }
+    void add_result(int curve, int64_t n, int64_t nbatch);
+    uint8_t* dev();
+    // Options of an MSM that fetch() runs (scalar_fmt: PORLA_SCALAR_*, out_fmt: PORLA_POINT_*), with the slot's scratch block.
+    MsmOptions msm_options(int scalar_fmt, int out_fmt, int shared_points) const;
+    // run_and_fetch on the frame's stream, pinned buffer and result region.
+    void fetch(int curve, const PointTable& tab, const uint8_t* d_scalars, int64_t n, int64_t nbatch, const MsmOptions& opt,
+               uint8_t* out);
+    Staging& staging() { return *s_; }
+    cudaStream_t stream() const { return s_->stream; }
+    uint8_t* pinned(size_t bytes) { return s_->pinned(bytes); }
+
+  private:
+    Staging* s_ = nullptr;
+    std::unique_lock<std::mutex> lk_;   // held for the shared staging area only (and makes the frame non-copyable)
+    int slot_ = -1;
+    StageLayout layout_;
+    size_t out_off_ = 0, scr_off_ = 0;   // scr_off_ = 0: no slot scratch block (the result region precedes it)
+    uint8_t* d_ = nullptr;
+};
+
 // A window [first, first + n) of a resident table: the same points, flags, endomorphism image and look-up rows.
 PointTable table_window(const PointTable& t, int64_t first, int64_t n);
 
@@ -107,8 +160,7 @@ struct porla_table {
 namespace porla {
 // n products k_i * B over the ONE point of a length-1 table (compute_digest_complement_batch, porla_secp256k1_ecmult_const_batch):
 // host scalars (n x 32 bytes, scalar_fmt) copied in, porla_scalar_mul_batch_device (k_fixed_base_mul over the table's
-// look-up table), and take() handed the n x 64 result bytes (out_fmt) in the staging's pinned buffer while the staging is
-// still held.  Calls of a few scalars lease a staging slot of their own.
-void fixed_base_mul_core(const porla_table* base, const void* scalars, int64_t n, int scalar_fmt, int out_fmt,
-                         const std::function<void(const uint8_t*)>& take);
+// look-up table); returns call's pinned buffer holding the n x 64 result bytes (out_fmt).  `call` is StagedCall(1, n).
+const uint8_t* fixed_base_mul_core(StagedCall& call, const porla_table* base, const void* scalars, int64_t n, int scalar_fmt,
+                                   int out_fmt);
 }  // namespace porla
